@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- normalize + PCA(k=10) throughput on the BASELINE.json workload.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config c3|c2|c4|c5] [--cells C]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config c3|c2|c4|c5] [--cells C] [--dump-outputs DIR]
 
 One "step" = normalize(CellRanger) + BkSvd::run_pca(k=10) over the whole synthetic
 1.3M-cell x 33,538-gene count matrix (BASELINE.json configs[2]; cells sharded over the N ranks,
@@ -18,6 +18,10 @@ against tests/golden/c3_seed3_k10.json, the CPU oracle's result on the full 1.3M
 `--impl reference` times the CPU restatement of the reference (oracle/, all host threads) on a
 bounded sample of the same workload; the default run also reports a 1-thread `cpu_baseline`.
 `--config` runs the other BASELINE.json configurations through the same code (c2: HVG + k=50; c4: 4M cells, k=100; c5: 60k features, k=30).
+`--dump-outputs DIR` writes what the last timed step of the device-resident arm returned (DIR/sigma.npy, DIR/U.npy, DIR/V.npy, f64;
+U and V each capped at 32 MB by a fixed seeded sample of their rows), so that two builds can be compared output for output:
+the inputs are seeded, identical from run to run for the same arguments.  The f64 reductions do not fix their order, so two
+runs of one build agree at rounding level, not bit for bit (DESIGN.md 4).
 """
 import argparse
 import json
@@ -31,6 +35,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark leaves the tree as the build left it (it may be read-only)
 
 METRIC = "normalize+PCA cells/s, 1.3Mx33.5k, k=10"
 CPU_SAMPLE_CELLS = 40_000      # 1-thread cpu_baseline sample: > n_genes so it takes the same n > m branch of svd_bk
@@ -48,6 +53,15 @@ CONFIGS = {
 }
 N_GENES, K = CONFIGS["c3"]["genes"], CONFIGS["c3"]["k"]
 FIXTURE = os.path.join(ROOT, "tests", "golden", "c3_seed3_k10.json")
+DUMP_BYTES_PER_MATRIX = 32 << 20  # --dump-outputs: U and V each at most 32 MB of f64
+
+
+def dump_rows(n_rows, k, seed):
+    """Rows of an n_rows x k f64 output that --dump-outputs writes: all of them, or a fixed seeded sample that fits the cap."""
+    cap = DUMP_BYTES_PER_MATRIX // (8 * k)
+    if n_rows <= cap:
+        return np.arange(n_rows)
+    return np.sort(np.random.default_rng(seed).choice(n_rows, cap, replace=False))
 
 
 def peaks():
@@ -239,14 +253,18 @@ def main():
     ap.add_argument("--impl", default="b200")
     ap.add_argument("--config", default="c3", choices=sorted(CONFIGS))
     ap.add_argument("--cells", type=int, default=0, help="override the configuration's cell count")
-    ap.add_argument("--e2e-steps", type=int, default=3)
+    ap.add_argument("--e2e-steps", type=int, default=None, help="timed steps of the end-to-end arm (default: --steps)")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--shard", default="nnz", choices=["nnz", "cells"])
     ap.add_argument("--host-form", default="packed", choices=["packed", "compact"],
                     help="host buffers of the end-to-end arm: sb_upload_packed (delta byte + count nibble) or sb_upload_compact (u16 + u8)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write sigma, U and V of the last timed step as DIR/<name>.npy (f64; large outputs as a fixed seeded row sample)")
     args = ap.parse_args()
     args.warmup_ref = min(args.warmup, 1)
+    if args.e2e_steps is None:
+        args.e2e_steps = args.steps
     if args.impl == "reference":
         run_reference(args)
         return
@@ -380,6 +398,17 @@ def main():
             fixture_ok = parity["sigma_rel_vs_cpu_fixture"] < 1e-6 and parity["U_probe_vs_cpu_fixture"] < 2e-5 and parity["V_probe_vs_cpu_fixture"] < 2e-5
             parity["fixture"] = "tests/golden/c3_seed3_k10.json (oracle on the full workload; scripts/make_sigma_fixture.py)"
     sigma_resident = sg.copy()
+    if args.dump_outputs:
+        # U is replicated on every rank; V's rows are sharded, so each rank fills the sampled rows it owns and the sum assembles them
+        vr = dump_rows(n_total, k, seed=1)
+        mine = (vr >= lo) & (vr < hi)
+        v_dump = np.zeros((len(vr), k))
+        v_dump[mine] = v[vr[mine] - lo]
+        v_dump = reduce_ranks(v_dump, "sum")
+        if rank == 0:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, arr in (("sigma", sg), ("U", u[dump_rows(len(u), k, seed=0)]), ("V", v_dump)):
+                np.save(os.path.join(args.dump_outputs, name + ".npy"), np.ascontiguousarray(arr, dtype=np.float64))
     release()
 
     # ---------------- end-to-end arm: pinned host CSC buffers -> results on host
