@@ -308,6 +308,58 @@ SB_API int sb_sum_rows_dual(sb_mat *mat, const uint64_t *cols1, uint64_t n1, con
  * one value per listed cell.  out[n_local]: 0 at unlisted cells. */
 SB_API int sb_size_factors(sb_mat *mat, const uint64_t *cells, uint64_t n_cells, const double *umi_counts, double *out);
 
+/* ---------------------------------------------------------------- differential expression (diff-exp: sSeq, Cell Ranger's published test)
+ * sb_sseq_compute_params replaces compute_sseq_params (diff-exp/src/diff_exp.rs; SURVEY 8f rank 4).  Over all N cells of all ranks:
+ *   sf[c] = cell total / median of the totals (sb_size_factors); mean_g, var_g of the SizeNormalized view v / sf[c] (sb_mean_var_axis);
+ *   use_g = var_g > 0;  S = sum_c 1 / sf[c];  phi_mm_g = max(0, (N var_g - mean_g S) / (mean_g^2 S)) on use_g, 0 elsewhere;
+ *   zeta_hat = percentile of phi_mm_g[use_g] at zeta_quantile (rank q (n - 1), linear interpolation, the rule of the median);
+ *   delta = (sum_use (phi_mm_g - mean(phi_mm[use]))^2 / (G - 1)) / (sum_use (phi_mm_g - zeta_hat)^2 / (G - 2)) with G = m (all genes);
+ *   phi_g = (1 - delta) phi_mm_g + delta zeta_hat on use_g (0 there if no phi_mm_g[use_g] is > 0), NaN elsewhere.
+ * SB_ERR_INVALID_ARG for a cell whose total is 0 and for a matrix without a gene of non-zero variance.
+ * All arrays are caller-allocated; size_factors has n_local entries (this rank's cells), the gene arrays m (replicated). */
+typedef struct sb_sseq_params {
+    uint64_t num_cells;       /* N, over all ranks */
+    uint32_t num_genes;       /* m */
+    uint32_t reserved;
+    double zeta_hat;
+    double delta;
+    double *size_factors;     /* [n_local] */
+    double *gene_means;       /* [m] */
+    double *gene_variances;   /* [m] */
+    double *gene_moment_phi;  /* [m] phi_mm */
+    double *gene_phi;         /* [m] shrunken dispersion */
+    uint8_t *use_genes;       /* [m] 1 where var_g > 0 */
+} sb_sseq_params;
+/* The comparison-dependent results, each [n_comparisons x m] row-major, caller-allocated. */
+typedef struct sb_diff_exp_out {
+    uint64_t *sums_in;
+    uint64_t *sums_out;
+    double *normalized_mean_in;
+    double *normalized_mean_out;
+    double *p_values;
+    double *adjusted_p_values;
+    double *log2_fold_change;
+} sb_diff_exp_out;
+SB_API int sb_sseq_compute_params(sb_mat *mat, double zeta_quantile, sb_sseq_params *out);
+/* sseq_differential_expression (diff_exp.rs): condition lists are strictly ascending LOCAL cell indices, each non-empty over all
+ * ranks; params come from sb_sseq_compute_params (on sharded contexts: this rank's size factors, the replicated gene arrays).
+ *   sums_in / sums_out: exact u64 sums over the listed cells; s_in / s_out = sum of sf over the listed cells (in global cell order);
+ *   normalized_mean = sums / s;  log2_fold_change = log2((1 + sums_in) / (1 + s_in)) - log2((1 + sums_out) / (1 + s_out));
+ *   p = 1 where use_g is 0.  With mu = mean_g, phi = phi_g:
+ *   both sums > big_count (asymptotic): alpha = s_in mu / (1 + phi mu), beta = (s_out / s_in) alpha, T = x_in + x_out, med = median of
+ *     Beta(alpha, beta); p = 2 I_{(x_in + 0.5) / T}(alpha, beta) if (x_in + 0.5) / T < med, else 2 (1 - I_{(x_in - 0.5) / T}(alpha, beta)),
+ *     evaluated as 2 I_{1 - (x_in - 0.5) / T}(beta, alpha) (no cancellation); not clipped;
+ *   otherwise (exact): lp(x, s) = lgamma(r + x) - (lgamma(r) + lgamma(x + 1)) + x log(mu s / (r + mu s)) + r log(r / (r + mu s)),
+ *     r = s / phi (phi = 0: the Poisson limit -lgamma(x + 1) + x log(mu s) - mu s, builder-defined); l(x) = lp(x, s_in) + lp(T - x, s_out);
+ *     p = exp(LSE_{x = 0..T, l(x) <= l(x_in)} l(x) - LSE_{x = 0..T} l(x)); bit-reproducible and independent of the rank count;
+ *   adjusted_p_values: Benjamini-Hochberg over the use_g genes (q = min(1, cummin over descending p of p n / rank)), p elsewhere. */
+SB_API int sb_sseq_diff_exp(sb_mat *mat, const sb_sseq_params *params, const uint64_t *cond_in, uint64_t n_in, const uint64_t *cond_out,
+                     uint64_t n_out, uint64_t big_count, sb_diff_exp_out *out);
+/* Cell Ranger's per-cluster loop, batched: comparison j is "labels == j" against "labels != j" (labels[n_local] of this rank's cells,
+ * each < n_groups; n_groups >= 2; no group may be empty over all ranks).  out arrays are [n_groups x m]. */
+SB_API int sb_sseq_one_vs_rest(sb_mat *mat, const sb_sseq_params *params, const uint32_t *labels, uint32_t n_groups, uint64_t big_count,
+                        sb_diff_exp_out *out);
+
 /* ---------------------------------------------------------------- kNN on the scores (next step of the pipeline)
  * knn / find_nn (scan-rs/src/nn.rs:38-83): for every query row (n_queries x dim, row-major) the indices of its k nearest points
  * (n_points x dim) in Euclidean distance, nearest first, into out[n_queries x k]; rows with fewer than k candidates are padded

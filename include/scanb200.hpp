@@ -12,7 +12,9 @@
 //   scan_rs::normalization::*        scan-rs/src/normalization.rs scanb200::normalization::*
 //   scan_rs::dim_red::{Pca,BkSvd,..} scan-rs/src/dim_red/*.rs     scanb200::dim_red::*
 //   snoop::{CancelProgress,NoOpSnoop} snoop/src/lib.rs            scanb200::snoop::*
+//   diff_exp::{compute_sseq_params,..} diff-exp/src/diff_exp.rs   scanb200::diff_exp::*
 #pragma once
+#include <type_traits>
 #include <algorithm>
 #include <array>
 #include <cmath>
@@ -429,4 +431,84 @@ inline double frobenius(const Array2 &a) {
     return std::sqrt(acc) / (double)(a.rows * a.cols);
 }
 }  // namespace dim_red
+
+// diff-exp: sSeq (compute_sseq_params, sseq_differential_expression; the contract is stated in scanb200.h)
+namespace diff_exp {
+struct SSeqParams {
+    uint64_t num_cells = 0;
+    uint32_t num_genes = 0;
+    std::vector<double> size_factors;  // this rank's cells
+    std::vector<double> gene_means, gene_variances;
+    std::vector<uint8_t> use_genes;
+    std::vector<double> gene_moment_phi;
+    double zeta_hat = 0.0, delta = 0.0;
+    std::vector<double> gene_phi;
+};
+struct DiffExpResult {
+    std::vector<uint8_t> genes_tested;
+    std::vector<uint64_t> sums_in, sums_out;
+    std::vector<double> common_mean, common_dispersion;
+    std::vector<double> normalized_mean_in, normalized_mean_out;
+    std::vector<double> p_values, adjusted_p_values, log2_fold_change;
+};
+
+inline SSeqParams compute_sseq_params(const sqz::AdaptiveMat &mat, double zeta_quantile = 0.995) {
+    const size_t m = mat.rows();
+    SSeqParams p;
+    p.size_factors.resize(mat.cols());
+    p.gene_means.resize(m);
+    p.gene_variances.resize(m);
+    p.use_genes.resize(m);
+    p.gene_moment_phi.resize(m);
+    p.gene_phi.resize(m);
+    sb_sseq_params c{0, 0, 0, 0.0, 0.0, p.size_factors.data(), p.gene_means.data(), p.gene_variances.data(), p.gene_moment_phi.data(),
+                     p.gene_phi.data(), p.use_genes.data()};
+    check(sb_sseq_compute_params(mat.raw(), zeta_quantile, &c));
+    p.num_cells = c.num_cells;
+    p.num_genes = c.num_genes;
+    p.zeta_hat = c.zeta_hat;
+    p.delta = c.delta;
+    return p;
+}
+
+namespace detail {
+// the C view of the params: the library only reads them
+inline sb_sseq_params view(const SSeqParams &p) {
+    return sb_sseq_params{p.num_cells, p.num_genes, 0, p.zeta_hat, p.delta, const_cast<double *>(p.size_factors.data()),
+                          const_cast<double *>(p.gene_means.data()), const_cast<double *>(p.gene_variances.data()),
+                          const_cast<double *>(p.gene_moment_phi.data()), const_cast<double *>(p.gene_phi.data()),
+                          const_cast<uint8_t *>(p.use_genes.data())};
+}
+template <class F>
+std::vector<DiffExpResult> run(const SSeqParams &p, size_t n_comp, size_t m, F call) {
+    std::vector<uint64_t> s_in(n_comp * m), s_out(n_comp * m);
+    std::vector<double> nm_in(n_comp * m), nm_out(n_comp * m), pv(n_comp * m), q(n_comp * m), lfc(n_comp * m);
+    sb_diff_exp_out o{s_in.data(), s_out.data(), nm_in.data(), nm_out.data(), pv.data(), q.data(), lfc.data()};
+    sb_sseq_params c = view(p);
+    check(call(&c, &o));
+    std::vector<DiffExpResult> out(n_comp);
+    for (size_t j = 0; j < n_comp; j++) {
+        auto sl = [&](const auto &v) { return std::vector<typename std::decay_t<decltype(v)>::value_type>(v.begin() + j * m, v.begin() + (j + 1) * m); };
+        out[j] = DiffExpResult{p.use_genes, sl(s_in), sl(s_out), p.gene_means, p.gene_phi, sl(nm_in), sl(nm_out), sl(pv), sl(q), sl(lfc)};
+    }
+    return out;
+}
+}  // namespace detail
+
+// cond_in / cond_out: strictly ascending (local) cell indices
+inline DiffExpResult sseq_differential_expression(const sqz::AdaptiveMat &mat, const std::vector<uint64_t> &cond_in, const std::vector<uint64_t> &cond_out,
+                                                  const SSeqParams &params, uint64_t big_count = 900) {
+    return detail::run(params, 1, mat.rows(), [&](const sb_sseq_params *c, sb_diff_exp_out *o) {
+        return sb_sseq_diff_exp(mat.raw(), c, cond_in.data(), cond_in.size(), cond_out.data(), cond_out.size(), big_count, o);
+    })[0];
+}
+// one result per group j: cells labelled j against all others
+inline std::vector<DiffExpResult> sseq_one_vs_rest(const sqz::AdaptiveMat &mat, const std::vector<uint32_t> &labels, uint32_t n_groups,
+                                                   const SSeqParams &params, uint64_t big_count = 900) {
+    if (labels.size() != mat.cols()) throw Error(SB_ERR_INVALID_ARG, "one label per cell");
+    return detail::run(params, n_groups, mat.rows(), [&](const sb_sseq_params *c, sb_diff_exp_out *o) {
+        return sb_sseq_one_vs_rest(mat.raw(), c, labels.data(), n_groups, big_count, o);
+    });
+}
+}  // namespace diff_exp
 }  // namespace scanb200

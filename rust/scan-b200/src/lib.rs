@@ -310,6 +310,104 @@ impl<'a> Pca<DeviceNormalized<'a>, f64> for GpuIrlba {
     }
 }
 
+/// diff-exp's `SSeqParams` (compute_sseq_params): the per-gene moments of the size-normalized view and the shrunken dispersions.
+/// `size_factors` holds this rank's cells; the gene arrays are replicated.
+#[derive(Clone, Debug)]
+pub struct SSeqParams {
+    pub num_cells: usize,
+    pub num_genes: usize,
+    pub size_factors: Array1<f64>,
+    pub gene_means: Array1<f64>,
+    pub gene_variances: Array1<f64>,
+    pub use_genes: Array1<bool>,
+    pub gene_moment_phi: Array1<f64>,
+    pub zeta_hat: f64,
+    pub delta: f64,
+    pub gene_phi: Array1<f64>,
+}
+
+/// diff-exp's `DiffExpResult` for one comparison.
+#[derive(Clone, Debug)]
+pub struct DiffExpResult {
+    pub genes_tested: Array1<bool>,
+    pub sums_in: Array1<u64>,
+    pub sums_out: Array1<u64>,
+    pub common_mean: Array1<f64>,
+    pub common_dispersion: Array1<f64>,
+    pub normalized_mean_in: Array1<f64>,
+    pub normalized_mean_out: Array1<f64>,
+    pub p_values: Array1<f64>,
+    pub adjusted_p_values: Array1<f64>,
+    pub log2_fold_change: Array1<f64>,
+}
+
+/// compute_sseq_params on the device (the contract is stated beside `sb_sseq_compute_params` in include/scanb200.h)
+pub fn compute_sseq_params(mat: &DeviceCountMatrix<'_>, zeta_quantile: f64) -> Result<SSeqParams, Error> {
+    let [m, n] = mat.shape();
+    let (mut sf, mut mean, mut var) = (Array1::<f64>::zeros(n), Array1::<f64>::zeros(m), Array1::<f64>::zeros(m));
+    let (mut phi_mm, mut phi, mut use_g) = (Array1::<f64>::zeros(m), Array1::<f64>::zeros(m), Array1::<u8>::zeros(m));
+    let mut p = ffi::sb_sseq_params {
+        num_cells: 0, num_genes: 0, reserved: 0, zeta_hat: 0.0, delta: 0.0, size_factors: sf.as_mut_ptr(), gene_means: mean.as_mut_ptr(),
+        gene_variances: var.as_mut_ptr(), gene_moment_phi: phi_mm.as_mut_ptr(), gene_phi: phi.as_mut_ptr(), use_genes: use_g.as_mut_ptr(),
+    };
+    check(unsafe { ffi::sb_sseq_compute_params(mat.h, zeta_quantile, &mut p) })?;
+    Ok(SSeqParams {
+        num_cells: p.num_cells as usize, num_genes: p.num_genes as usize, size_factors: sf, gene_means: mean, gene_variances: var,
+        use_genes: use_g.mapv(|u| u != 0), gene_moment_phi: phi_mm, zeta_hat: p.zeta_hat, delta: p.delta, gene_phi: phi,
+    })
+}
+
+fn sseq_run(mat: &DeviceCountMatrix<'_>, params: &SSeqParams, n_comp: usize,
+            call: impl FnOnce(*const ffi::sb_sseq_params, *mut ffi::sb_diff_exp_out) -> i32) -> Result<Vec<DiffExpResult>, Error> {
+    let m = mat.shape()[0];
+    let (mut s_in, mut s_out) = (Array2::<u64>::zeros((n_comp, m)), Array2::<u64>::zeros((n_comp, m)));
+    let mut f: Vec<Array2<f64>> = (0..5).map(|_| Array2::<f64>::zeros((n_comp, m))).collect();
+    // the library only reads the params; the C struct carries mutable pointers because sb_sseq_compute_params fills the same type
+    let (mut sf, mut mean, mut var, mut phi_mm, mut phi) = (params.size_factors.to_owned(), params.gene_means.to_owned(),
+        params.gene_variances.to_owned(), params.gene_moment_phi.to_owned(), params.gene_phi.to_owned());
+    let mut use_g = params.use_genes.mapv(|b| b as u8);
+    let p = ffi::sb_sseq_params {
+        num_cells: params.num_cells as u64, num_genes: params.num_genes as u32, reserved: 0, zeta_hat: params.zeta_hat, delta: params.delta,
+        size_factors: sf.as_mut_ptr(), gene_means: mean.as_mut_ptr(), gene_variances: var.as_mut_ptr(), gene_moment_phi: phi_mm.as_mut_ptr(),
+        gene_phi: phi.as_mut_ptr(), use_genes: use_g.as_mut_ptr(),
+    };
+    let mut o = ffi::sb_diff_exp_out {
+        sums_in: s_in.as_mut_ptr(), sums_out: s_out.as_mut_ptr(), normalized_mean_in: f[0].as_mut_ptr(), normalized_mean_out: f[1].as_mut_ptr(),
+        p_values: f[2].as_mut_ptr(), adjusted_p_values: f[3].as_mut_ptr(), log2_fold_change: f[4].as_mut_ptr(),
+    };
+    check(call(&p, &mut o))?;
+    Ok((0..n_comp)
+        .map(|j| DiffExpResult {
+            genes_tested: params.use_genes.clone(),
+            sums_in: s_in.row(j).to_owned(),
+            sums_out: s_out.row(j).to_owned(),
+            common_mean: params.gene_means.clone(),
+            common_dispersion: params.gene_phi.clone(),
+            normalized_mean_in: f[0].row(j).to_owned(),
+            normalized_mean_out: f[1].row(j).to_owned(),
+            p_values: f[2].row(j).to_owned(),
+            adjusted_p_values: f[3].row(j).to_owned(),
+            log2_fold_change: f[4].row(j).to_owned(),
+        })
+        .collect())
+}
+
+/// sseq_differential_expression: `cond_in` against `cond_out` (strictly ascending local cell indices)
+pub fn sseq_differential_expression(mat: &DeviceCountMatrix<'_>, cond_in: &[u64], cond_out: &[u64], params: &SSeqParams, big_count: u64)
+                                    -> Result<DiffExpResult, Error> {
+    let mut r = sseq_run(mat, params, 1, |p, o| unsafe {
+        ffi::sb_sseq_diff_exp(mat.h, p, cond_in.as_ptr(), cond_in.len() as u64, cond_out.as_ptr(), cond_out.len() as u64, big_count, o)
+    })?;
+    Ok(r.remove(0))
+}
+
+/// Cell Ranger's cluster-vs-rest loop, batched: result j compares the cells labelled j with all other cells
+pub fn sseq_one_vs_rest(mat: &DeviceCountMatrix<'_>, labels: &[u32], n_groups: u32, params: &SSeqParams, big_count: u64)
+                        -> Result<Vec<DiffExpResult>, Error> {
+    assert_eq!(labels.len(), mat.shape()[1], "one label per cell");
+    sseq_run(mat, params, n_groups as usize, |p, o| unsafe { ffi::sb_sseq_one_vs_rest(mat.h, p, labels.as_ptr(), n_groups, big_count, o) })
+}
+
 /// Every GPU of the box from one caller thread (SURVEY 8b; the reference's only caller is a single process).  `run` executes the
 /// closure once per rank, concurrently, each on its own library worker thread with its own `Context`; inside it a rank uploads
 /// its contiguous cell shard and makes the ordinary calls -- the collectives meet across the workers.

@@ -7,6 +7,7 @@ The package mirrors the reference's module layout for this path only:
   snoop          NoOpSnoop, AtomicSnoop
   mtx            load_mtx (gz MatrixMarket -> device matrix)
   nn             knn, find_nn on the PCA scores
+  diff_exp       sSeq differential expression (compute_sseq_params, sseq_differential_expression, sseq_one_vs_rest)
   synth          synthetic workloads (test / bench utility)
 All compute runs in scan_rs_b200/libscanb200.so (hand-written sm_100a CUDA + cuSOLVER/cuBLAS for the
 small dense steps); there is no CPU fallback."""
@@ -21,3 +22,5 @@ from .snoop import AtomicSnoop, NoOpSnoop  # noqa: F401
 from .mtx import load_mtx  # noqa: F401
 from .nn import find_nn, knn  # noqa: F401
 from .multi import MultiContext  # noqa: F401
+from .diff_exp import (DiffExpResult, SSeqParams, compute_sseq_params, sseq_differential_expression,  # noqa: F401
+                       sseq_one_vs_rest)

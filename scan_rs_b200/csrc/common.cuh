@@ -342,6 +342,10 @@ int comm_allreduce_f64(sb_ctx *ctx, double *buf, size_t count);
 int comm_allreduce_u64(sb_ctx *ctx, u64 *buf, size_t count);
 int comm_allreduce_max_i32(sb_ctx *ctx, int *host_val);
 int comm_allgather_u64_host(sb_ctx *ctx, u64 mine, std::vector<u64> &all);
+// every rank takes the same turn before the next collective: a local rejection becomes every rank's error (matrix.cu)
+int agree_status(sb_ctx *ctx, int rc, const char *what);
+// percentile_of_sorted (stat.rs:140-163) at the fraction q: rank q (n - 1), linear interpolation; sorts v (moments.cu)
+double percentile_of(std::vector<double> &v, double q);
 
 // every API entry: select the device and publish the stream used for stream-ordered allocations
 #define SB_ENTER(ctx_ptr)                         \

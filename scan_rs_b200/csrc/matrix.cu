@@ -808,7 +808,7 @@ static void trace_pool(sb_ctx *ctx, const char *label) {
 
 // Every rank of a sharded context must take the same turn before the collectives of an upload (global shape, hot-gene counts):
 // a rank that rejected its own input would otherwise leave the others waiting inside them.
-static int agree_status(sb_ctx *ctx, int rc, const char *what) {
+int agree_status(sb_ctx *ctx, int rc, const char *what) {
     if (ctx->nranks == 1) return rc;
     int worst = rc;
     const std::string mine = rc != SB_OK ? sb_last_error() : "";

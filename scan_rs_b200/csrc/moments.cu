@@ -255,15 +255,18 @@ extern "C" int sb_sum_cols(sb_mat *mat, const uint64_t *cols, uint64_t n_cols, u
     return SB_OK;
 }
 
-// percentile_of_sorted(.., 50) (stat.rs:140-163)
-static double percentile_median(std::vector<double> &v) {
+// percentile_of_sorted (stat.rs:140-163) at the fraction q in [0, 1]: rank q (n - 1), linear interpolation; sorts v (non-empty).
+// The median of the size factors is q = 0.5; sSeq's zeta_hat (diff_exp.cu) is q = zeta_quantile.
+double percentile_of(std::vector<double> &v, double q) {
     std::sort(v.begin(), v.end());
     if (v.size() == 1) return v[0];
-    const double rank = 0.5 * (double)(v.size() - 1);
+    const double rank = q * (double)(v.size() - 1);
     const double lr = std::floor(rank), d = rank - lr;
     const size_t i = (size_t)lr;
+    if (i + 1 >= v.size()) return v[i];
     return v[i] + (v[i + 1] - v[i]) * d;
 }
+static double percentile_median(std::vector<double> &v) { return percentile_of(v, 0.5); }
 
 // size_factors (diff_exp.rs:314-334).  cells (local indices, may be NULL = all cells) select the cells whose totals define the
 // median; umi_counts (may be NULL) replaces the totals: one value per listed cell (or per local cell when cells is NULL).
