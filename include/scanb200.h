@@ -369,6 +369,54 @@ SB_API int sb_sseq_one_vs_rest(sb_mat *mat, const sb_sseq_params *params, const 
 SB_API int sb_knn(sb_ctx *ctx, const double *points, uint64_t n_points, uint32_t dim, const double *queries, uint64_t n_queries,
            uint32_t k, int include_self, uint64_t self_offset, uint32_t *out);
 
+/* ---------------------------------------------------------------- graph clustering (the step between kNN and diff-exp)
+ * Deterministic Louvain on a shared-nearest-neighbour graph; the base algorithm of the reference's `leiden` crate, made
+ * synchronous so that the result is bit-reproducible and equal to oracle/louvain.py.
+ *
+ * sb_snn_graph: nbr[n x k] as sb_knn returns it (global indices, no self index, 0xFFFFFFFF only at row ends; 1 <= k <= 128,
+ * n k < 2^28, else SB_ERR_UNSUPPORTED).  Edges {i, j} wherever j is in N(i) or i in N(j), stored both ways: indptr[n + 1],
+ * columns ascending, no self loops.  Weight w = (s << 24) / u (integer division), s = |N+(i) n N+(j)|, u = |N+(i)| + |N+(j)| - s,
+ * N+(i) = N(i) u {i}: the Jaccard index of the closed neighbourhoods in 24-bit fixed point.  indices / weights must hold 2 n k
+ * entries; *nnz receives the count.  An index >= n, a self index, a duplicate in a row or padding before a row end is
+ * SB_ERR_INVALID_ARG.
+ *
+ * sb_louvain: a host CSR of n nodes, symmetric (equal weights both ways), no duplicate entry, self loops allowed (checked on the
+ * device: SB_ERR_INVALID_ARG); 2m = sum of all entries must be < 2^53 (SB_ERR_UNSUPPORTED).  K_i = row sum (a self loop once),
+ * S_c = sum of K over c, e_ic = weight from i to the members of c other than i.  Level: every node starts alone; iteration t moves
+ * every node i (community a) to the allowed neighbouring c with the largest
+ *   gain(c) = ((double)e_ic - (double)e_ia) - g2m (double)K_i ((double)S_c - (double)(S_a - K_i)),  g2m = resolution / (double)2m,
+ * evaluated in this order without contraction, if that gain is > 0 (ties: the smallest c).  Allowed: c > a in even iterations,
+ * c < a in odd ones.  The moves are kept only if Q = (double)sum_I / (double)2m - resolution sum_S2 / (2m)^2 strictly increases
+ * (sum_I: intra-community directed weight, self loops included; sum_S2 = sum S_c^2 exact in 128 bits, as (double)hi 2^64 +
+ * (double)lo).  A level ends after two consecutive iterations without a kept move, or max_iterations.  A level that kept a move
+ * is aggregated (communities numbered in ascending id; coarse weights summed per pair, self loops carrying the internal weight)
+ * and the next level runs, up to max_levels.  Labels: clusters numbered by size, descending, ties to the smallest node index
+ * (0..n_clusters-1, none empty).  A graph of total weight 0 leaves every node its own cluster (one level, 0 iterations, Q = 0).
+ *
+ * sb_cluster_knn: sb_snn_graph + sb_louvain with the graph kept on the device.  On a cell-sharded context every rank passes its own
+ * rows (n_local x k, global indices: sb_knn with self_offset = its first cell) and receives its cells' labels; the rows are
+ * gathered in global cell order and every rank runs the same clustering, so labels equal world 1 bit for bit. */
+#define SB_LOUVAIN_MAX_LEVELS 32
+typedef struct sb_louvain_opts {
+    double resolution;        /* gamma > 0 (default 1.0) */
+    uint32_t max_levels;      /* 1..SB_LOUVAIN_MAX_LEVELS (default 32) */
+    uint32_t max_iterations;  /* per level, >= 1 (default 100) */
+} sb_louvain_opts;            /* NULL: the defaults */
+typedef struct sb_louvain_info {
+    uint32_t n_clusters;
+    uint32_t n_levels;
+    double modularity;        /* Q of the final partition */
+    uint64_t level_nodes[SB_LOUVAIN_MAX_LEVELS];
+    uint32_t level_iterations[SB_LOUVAIN_MAX_LEVELS];
+    double level_modularity[SB_LOUVAIN_MAX_LEVELS];
+} sb_louvain_info;
+SB_API int sb_snn_graph(sb_ctx *ctx, const uint32_t *nbr, uint64_t n, uint32_t k, uint64_t *indptr, uint32_t *indices, uint64_t *weights,
+                 uint64_t *nnz);
+SB_API int sb_louvain(sb_ctx *ctx, uint64_t n, const uint64_t *indptr, const uint32_t *indices, const uint64_t *weights,
+               const sb_louvain_opts *opts, uint32_t *labels, sb_louvain_info *info);
+SB_API int sb_cluster_knn(sb_ctx *ctx, const uint32_t *nbr, uint64_t n_local, uint32_t k, const sb_louvain_opts *opts, uint32_t *labels,
+                   sb_louvain_info *info);
+
 /* ---------------------------------------------------------------- measurement
  * Device-side timing on the context's own stream (CUDA events) and per-kernel accounting;
  * bench.py builds its roofline object from these.  Not part of the reference interface. */

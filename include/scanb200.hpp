@@ -13,6 +13,7 @@
 //   scan_rs::dim_red::{Pca,BkSvd,..} scan-rs/src/dim_red/*.rs     scanb200::dim_red::*
 //   snoop::{CancelProgress,NoOpSnoop} snoop/src/lib.rs            scanb200::snoop::*
 //   diff_exp::{compute_sseq_params,..} diff-exp/src/diff_exp.rs   scanb200::diff_exp::*
+//   leiden (Louvain), SNN graph      leiden crate (deterministic)  scanb200::clustering::*
 #pragma once
 #include <type_traits>
 #include <algorithm>
@@ -511,4 +512,69 @@ inline std::vector<DiffExpResult> sseq_one_vs_rest(const sqz::AdaptiveMat &mat, 
     });
 }
 }  // namespace diff_exp
+
+// graph clustering: SNN graph of the kNN lists and deterministic Louvain (the rules are stated in scanb200.h)
+namespace clustering {
+struct Graph {  // symmetric CSR, weights = Jaccard index << 24
+    std::vector<uint64_t> indptr;
+    std::vector<uint32_t> indices;
+    std::vector<uint64_t> weights;
+};
+struct Options {
+    double resolution = 1.0;
+    uint32_t max_levels = SB_LOUVAIN_MAX_LEVELS;
+    uint32_t max_iterations = 100;
+};
+struct Level {
+    uint64_t nodes;
+    uint32_t iterations;
+    double modularity;
+};
+struct Result {
+    std::vector<uint32_t> labels;  // 0..n_clusters-1, by size, descending
+    uint32_t n_clusters = 0;
+    double modularity = 0.0;
+    std::vector<Level> levels;
+};
+
+namespace detail {
+inline Result result(std::vector<uint32_t> labels, const sb_louvain_info &info) {
+    Result r{std::move(labels), info.n_clusters, info.modularity, {}};
+    for (uint32_t l = 0; l < info.n_levels; l++) r.levels.push_back(Level{info.level_nodes[l], info.level_iterations[l], info.level_modularity[l]});
+    return r;
+}
+inline sb_louvain_opts opts(const Options &o) { return sb_louvain_opts{o.resolution, o.max_levels, o.max_iterations}; }
+}  // namespace detail
+
+// nbr: n x k row-major, as knn returns it
+inline Graph snn_graph(const Context &ctx, const std::vector<uint32_t> &nbr, uint32_t k) {
+    if (k == 0 || nbr.size() % k) throw Error(SB_ERR_INVALID_ARG, "nbr must hold n x k entries");
+    const uint64_t n = nbr.size() / k;
+    Graph g{std::vector<uint64_t>(n + 1), std::vector<uint32_t>(2 * n * k), std::vector<uint64_t>(2 * n * k)};
+    uint64_t nnz = 0;
+    check(sb_snn_graph(ctx.raw(), nbr.data(), n, k, g.indptr.data(), g.indices.data(), g.weights.data(), &nnz));
+    g.indices.resize(nnz);
+    g.weights.resize(nnz);
+    return g;
+}
+inline Result louvain(const Context &ctx, const Graph &g, const Options &o = Options()) {
+    if (g.indptr.empty()) throw Error(SB_ERR_INVALID_ARG, "indptr must hold n + 1 entries");
+    const uint64_t n = g.indptr.size() - 1;
+    std::vector<uint32_t> labels(n);
+    sb_louvain_info info;
+    const sb_louvain_opts c = detail::opts(o);
+    check(sb_louvain(ctx.raw(), n, g.indptr.data(), g.indices.data(), g.weights.data(), &c, labels.data(), &info));
+    return detail::result(std::move(labels), info);
+}
+// on a sharded context: this rank's rows (global indices) -> this rank's labels
+inline Result cluster_knn(const Context &ctx, const std::vector<uint32_t> &nbr, uint32_t k, const Options &o = Options()) {
+    if (k == 0 || nbr.size() % k) throw Error(SB_ERR_INVALID_ARG, "nbr must hold n x k entries");
+    const uint64_t n = nbr.size() / k;
+    std::vector<uint32_t> labels(n);
+    sb_louvain_info info;
+    const sb_louvain_opts c = detail::opts(o);
+    check(sb_cluster_knn(ctx.raw(), nbr.data(), n, k, &c, labels.data(), &info));
+    return detail::result(std::move(labels), info);
+}
+}  // namespace clustering
 }  // namespace scanb200

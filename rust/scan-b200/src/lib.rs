@@ -408,6 +408,85 @@ pub fn sseq_one_vs_rest(mat: &DeviceCountMatrix<'_>, labels: &[u32], n_groups: u
     sseq_run(mat, params, n_groups as usize, |p, o| unsafe { ffi::sb_sseq_one_vs_rest(mat.h, p, labels.as_ptr(), n_groups, big_count, o) })
 }
 
+/// Louvain options: resolution (gamma) > 0, max_levels 1..32, max_iterations per level >= 1
+#[derive(Clone, Copy, Debug)]
+pub struct LouvainOptions {
+    pub resolution: f64,
+    pub max_levels: u32,
+    pub max_iterations: u32,
+}
+impl Default for LouvainOptions {
+    fn default() -> Self {
+        LouvainOptions { resolution: 1.0, max_levels: ffi::SB_LOUVAIN_MAX_LEVELS as u32, max_iterations: 100 }
+    }
+}
+
+/// Cluster labels (0..n_clusters-1, by size, descending), the final modularity and (nodes, iterations, Q) per level
+#[derive(Clone, Debug)]
+pub struct Clustering {
+    pub labels: Vec<u32>,
+    pub n_clusters: u32,
+    pub modularity: f64,
+    pub levels: Vec<(u64, u32, f64)>,
+}
+
+/// Shared-nearest-neighbour graph as a symmetric CSR; weights are Jaccard indices in 24-bit fixed point
+#[derive(Clone, Debug)]
+pub struct SnnGraph {
+    pub indptr: Vec<u64>,
+    pub indices: Vec<u32>,
+    pub weights: Vec<u64>,
+}
+
+fn clustering(labels: Vec<u32>, info: &ffi::sb_louvain_info) -> Clustering {
+    let levels = (0..info.n_levels as usize).map(|l| (info.level_nodes[l], info.level_iterations[l], info.level_modularity[l])).collect();
+    Clustering { labels, n_clusters: info.n_clusters, modularity: info.modularity, levels }
+}
+fn louvain_opts(o: &LouvainOptions) -> ffi::sb_louvain_opts {
+    ffi::sb_louvain_opts { resolution: o.resolution, max_levels: o.max_levels, max_iterations: o.max_iterations }
+}
+fn empty_info() -> ffi::sb_louvain_info {
+    ffi::sb_louvain_info { n_clusters: 0, n_levels: 0, modularity: 0.0, level_nodes: [0; ffi::SB_LOUVAIN_MAX_LEVELS],
+                           level_iterations: [0; ffi::SB_LOUVAIN_MAX_LEVELS], level_modularity: [0.0; ffi::SB_LOUVAIN_MAX_LEVELS] }
+}
+
+/// The SNN graph of kNN lists (`nbr` n x k, as `knn` returns them; the rules are stated beside `sb_snn_graph` in include/scanb200.h)
+pub fn snn_graph(ctx: &Context, nbr: &Array2<u32>) -> Result<SnnGraph, Error> {
+    let nbr = nbr.as_standard_layout();
+    let (n, k) = nbr.dim();
+    let mut g = SnnGraph { indptr: vec![0; n + 1], indices: vec![0; 2 * n * k], weights: vec![0; 2 * n * k] };
+    let mut nnz = 0u64;
+    check(unsafe {
+        ffi::sb_snn_graph(ctx.h, nbr.as_ptr(), n as u64, k as u32, g.indptr.as_mut_ptr(), g.indices.as_mut_ptr(), g.weights.as_mut_ptr(), &mut nnz)
+    })?;
+    g.indices.truncate(nnz as usize);
+    g.weights.truncate(nnz as usize);
+    Ok(g)
+}
+
+/// Deterministic Louvain on a symmetric CSR with integer weights
+pub fn louvain(ctx: &Context, g: &SnnGraph, opts: &LouvainOptions) -> Result<Clustering, Error> {
+    assert!(!g.indptr.is_empty(), "indptr must hold n + 1 entries");
+    let n = g.indptr.len() - 1;
+    let mut labels = vec![0u32; n];
+    let mut info = empty_info();
+    let o = louvain_opts(opts);
+    check(unsafe { ffi::sb_louvain(ctx.h, n as u64, g.indptr.as_ptr(), g.indices.as_ptr(), g.weights.as_ptr(), &o, labels.as_mut_ptr(), &mut info) })?;
+    Ok(clustering(labels, &info))
+}
+
+/// kNN lists -> SNN graph -> Louvain with the graph kept on the device; on a sharded context every rank passes its own rows
+/// (global indices) and receives its own cells' labels
+pub fn cluster_knn(ctx: &Context, nbr: &Array2<u32>, opts: &LouvainOptions) -> Result<Clustering, Error> {
+    let nbr = nbr.as_standard_layout();
+    let (n, k) = nbr.dim();
+    let mut labels = vec![0u32; n];
+    let mut info = empty_info();
+    let o = louvain_opts(opts);
+    check(unsafe { ffi::sb_cluster_knn(ctx.h, nbr.as_ptr(), n as u64, k as u32, &o, labels.as_mut_ptr(), &mut info) })?;
+    Ok(clustering(labels, &info))
+}
+
 /// Every GPU of the box from one caller thread (SURVEY 8b; the reference's only caller is a single process).  `run` executes the
 /// closure once per rank, concurrently, each on its own library worker thread with its own `Context`; inside it a rank uploads
 /// its contiguous cell shard and makes the ordinary calls -- the collectives meet across the workers.

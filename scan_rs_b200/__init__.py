@@ -7,6 +7,7 @@ The package mirrors the reference's module layout for this path only:
   snoop          NoOpSnoop, AtomicSnoop
   mtx            load_mtx (gz MatrixMarket -> device matrix)
   nn             knn, find_nn on the PCA scores
+  cluster        SNN graph of the kNN lists and deterministic Louvain (snn_graph, louvain, cluster_knn)
   diff_exp       sSeq differential expression (compute_sseq_params, sseq_differential_expression, sseq_one_vs_rest)
   synth          synthetic workloads (test / bench utility)
 All compute runs in scan_rs_b200/libscanb200.so (hand-written sm_100a CUDA + cuSOLVER/cuBLAS for the
@@ -24,3 +25,4 @@ from .nn import find_nn, knn  # noqa: F401
 from .multi import MultiContext  # noqa: F401
 from .diff_exp import (DiffExpResult, SSeqParams, compute_sseq_params, sseq_differential_expression,  # noqa: F401
                        sseq_one_vs_rest)
+from .cluster import ClusterResult, LouvainOptions, cluster_knn, louvain, snn_graph  # noqa: F401
