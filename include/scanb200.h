@@ -417,6 +417,80 @@ SB_API int sb_louvain(sb_ctx *ctx, uint64_t n, const uint64_t *indptr, const uin
 SB_API int sb_cluster_knn(sb_ctx *ctx, const uint32_t *nbr, uint64_t n_local, uint32_t k, const sb_louvain_opts *opts, uint32_t *labels,
                    sb_louvain_info *info);
 
+/* ---------------------------------------------------------------- UMAP embedding (the reference's `umap-rs`, a port of umap-learn)
+ * The fuzzy kNN graph and umap-learn's layout, made epoch-synchronous so that the result is bit-reproducible at every grid and
+ * world size; restated by oracle/umap.py.
+ *
+ * sb_umap_graph: scores X[n x dim] (f64, row-major; the PCA scores) and nbr[n x k] as sb_knn(..., include_self = 0) returns them
+ * (1 <= k <= 128, n k < 2^28, else SB_ERR_UNSUPPORTED; an index >= n, a self index, a duplicate in a row or padding before a row
+ * end is SB_ERR_INVALID_ARG).  umap-learn's n_neighbors is k + 1 (the point itself at distance 0).
+ *   d_ij  = sqrt(sum_c (x_j,c - x_i,c)^2), summed in coordinate order without contraction (knn.cu's ranking expression);
+ *   rho_i = the smallest non-zero d_ij of the row (0 if none);
+ *   sigma_i by umap-learn's smooth_knn_dist bisection: lo = 0, hi = inf, mid = 1; 64 steps of psum = sum over the listed j, in
+ *           slot order, of (d_ij - rho_i > 0 ? exp(-((d_ij - rho_i) / mid)) : 1); stop when |psum - log2(k + 1)| < 1e-5; psum >
+ *           target: hi = mid, mid = (lo + hi) / 2; else lo = mid, mid = hi == inf ? 2 mid : (lo + hi) / 2.  Floors: sigma_i >=
+ *           1e-3 (s_i / (m_i + 1)) when rho_i > 0, else >= 1e-3 (sum_i s_i / sum_i (m_i + 1)); s_i = the row's distances summed
+ *           in slot order, m_i = its listed count, the rows summed in order;
+ *   w_ij  = exp(-max(0, d_ij - rho_i) / sigma_i);
+ *   union = mix ((a + b) - a b) + (1 - mix) (a b), a = w_ij, b = w_ji (0 when not listed), mix = set_op_mix_ratio; stored both
+ *           ways, columns ascending, no self loops, zero weights dropped.
+ * indices / weights must hold 2 n k entries; *nnz receives the count; rho / sigma (n each) may be NULL.
+ *
+ * sb_umap_layout: a host CSR of n vertices, symmetric (equal weights both ways), no duplicate entry, weights in (0, 1] (checked
+ * on the device: SB_ERR_INVALID_ARG); a row's entries are taken with columns ascending.  Schedule (umap-learn's
+ * optimize_layout_euclidean, arithmetic in f64): n_epochs (0: 500 if n <= 10,000 else 200); entries with w < w_max / n_epochs
+ * dropped; per remaining directed entry e (in CSR order) eps = w_max / w, epn = eps / negative_sample_rate, next = eps,
+ * next_neg = epn.  Epoch t = 0..n_epochs-1, alpha = learning_rate (1 - t / n_epochs), reads one snapshot Y of the positions; every
+ * entry (head j, tail k) with next <= t:
+ *   attractive: d2 = |y_j - y_k|^2 (coordinate order); g = d2 > 0 ? ((-2 a) b) d2^(b - 1) / (a d2^b + 1) : 0; per coordinate
+ *               c = alpha clip(g (y_j - y_k)) goes to j and -c to k;
+ *   next += eps; s = max(0, trunc((t - next_neg) / epn)) negative samples, the p-th one v = mix64(mix64(mix64(mix64(seed) ^ t)
+ *               ^ e) ^ p) % n (mix64: SplitMix64's finaliser; e: the entry's index after pruning); v = j is skipped; d2 > 0:
+ *               c = alpha clip((2 gamma b) / ((0.001 + d2) (a d2^b + 1)) (y_j - y_v)), d2 = 0: c = 4 alpha, to j;
+ *               next_neg += s epn.
+ * clip(x) = max(-4, min(4, x)).  Every contribution is rounded to an integer q = rint(c 2^32), summed per vertex in 64 bits and
+ * added once at the end of the epoch; positions are those integers (y = q 2^-32), so the layout does not depend on the order of
+ * the sums.  A graph whose largest degree could let an epoch's sum pass 2^62 is SB_ERR_UNSUPPORTED.  (a, b): given (both > 0),
+ * or fitted: 1 / (1 + a x^(2b)) to umap-learn's target (1 for x < min_dist, exp(-(x - min_dist) / spread) beyond) on
+ * linspace(0, 3 spread, 300) by Levenberg-Marquardt from (1, 1).  Start (init[n x n_components], f64): SB_UMAP_INIT_PCA scales
+ * every column to [0, 10] as 10 (x - min) / (max - min) (a constant column: 0), SB_UMAP_INIT_USER takes it as given (finite,
+ * |x| < 2^30), SB_UMAP_INIT_RANDOM ignores it: uniform [-10, 10) as -10 + 20 ((h >> 11) 2^-53), h = mix64(mix64(mix64(seed)
+ * ^ (2^64 - 1)) ^ (i n_components + c)).  Either start is rounded to multiples of 2^-32.  out[n x n_components] (f64).
+ *
+ * sb_umap: sb_umap_graph + sb_umap_layout with the graph kept on the device; SB_UMAP_INIT_PCA starts from the first n_components
+ * columns of X, SB_UMAP_INIT_USER from init (this rank's rows).  On a cell-sharded context every rank passes its own rows of X
+ * and nbr (global indices: sb_knn with self_offset = its first cell) and receives its own rows of the embedding; the rows are
+ * gathered in global cell order and every rank runs the same layout, so the embedding equals world 1 bit for bit. */
+#define SB_UMAP_INIT_PCA 0
+#define SB_UMAP_INIT_RANDOM 1
+#define SB_UMAP_INIT_USER 2
+typedef struct sb_umap_opts {
+    uint32_t n_components;          /* 1..8 (default 2) */
+    uint32_t n_epochs;              /* 0: 500 if n <= 10,000, else 200 (default 0) */
+    double min_dist;                /* 0 <= min_dist <= spread (default 0.1) */
+    double spread;                  /* > 0 (default 1.0) */
+    double a, b;                    /* both 0: fitted from min_dist / spread (default); both > 0: used as given */
+    double learning_rate;           /* > 0 (default 1.0) */
+    double repulsion_strength;      /* gamma >= 0 (default 1.0) */
+    double set_op_mix_ratio;        /* 0..1 (default 1.0: fuzzy union; 0: fuzzy intersection) */
+    uint32_t negative_sample_rate;  /* negative samples per positive sample (default 5) */
+    uint32_t init;                  /* SB_UMAP_INIT_PCA (default), SB_UMAP_INIT_RANDOM, SB_UMAP_INIT_USER */
+    uint64_t seed;                  /* negative samples and the random start (default 0) */
+} sb_umap_opts;                     /* NULL: the defaults */
+typedef struct sb_umap_info {
+    double a, b;                    /* as used */
+    double max_weight;              /* w_max of the graph */
+    uint64_t n_edges;               /* directed entries of the graph */
+    uint64_t n_edges_used;          /* after pruning */
+    uint32_t n_epochs;
+} sb_umap_info;
+SB_API int sb_umap_graph(sb_ctx *ctx, const double *scores, const uint32_t *nbr, uint64_t n, uint32_t dim, uint32_t k, const sb_umap_opts *opts,
+                  uint64_t *indptr, uint32_t *indices, double *weights, uint64_t *nnz, double *rho, double *sigma);
+SB_API int sb_umap_layout(sb_ctx *ctx, uint64_t n, const uint64_t *indptr, const uint32_t *indices, const double *weights, const double *init,
+                   const sb_umap_opts *opts, double *out, sb_umap_info *info);
+SB_API int sb_umap(sb_ctx *ctx, const double *scores, const uint32_t *nbr, uint64_t n_local, uint32_t dim, uint32_t k, const sb_umap_opts *opts,
+            const double *init, double *out, sb_umap_info *info);
+
 /* ---------------------------------------------------------------- measurement
  * Device-side timing on the context's own stream (CUDA events) and per-kernel accounting;
  * bench.py builds its roofline object from these.  Not part of the reference interface. */

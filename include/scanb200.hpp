@@ -14,6 +14,7 @@
 //   snoop::{CancelProgress,NoOpSnoop} snoop/src/lib.rs            scanb200::snoop::*
 //   diff_exp::{compute_sseq_params,..} diff-exp/src/diff_exp.rs   scanb200::diff_exp::*
 //   leiden (Louvain), SNN graph      leiden crate (deterministic)  scanb200::clustering::*
+//   umap-rs (UMAP)                   umap-rs crate (deterministic) scanb200::embedding::*
 #pragma once
 #include <type_traits>
 #include <algorithm>
@@ -577,4 +578,82 @@ inline Result cluster_knn(const Context &ctx, const std::vector<uint32_t> &nbr, 
     return detail::result(std::move(labels), info);
 }
 }  // namespace clustering
+
+// UMAP embedding: fuzzy kNN graph and epoch-synchronous layout (the rules are stated in scanb200.h)
+namespace embedding {
+struct Graph {  // symmetric CSR, weights in (0, 1]
+    std::vector<uint64_t> indptr;
+    std::vector<uint32_t> indices;
+    std::vector<double> weights;
+    std::vector<double> rho, sigma;  // per vertex (from umap_graph)
+};
+enum class Init : uint32_t { Pca = SB_UMAP_INIT_PCA, Random = SB_UMAP_INIT_RANDOM, User = SB_UMAP_INIT_USER };
+struct Options {
+    uint32_t n_components = 2;
+    uint32_t n_epochs = 0;  // 0: 500 if n <= 10,000 else 200
+    double min_dist = 0.1, spread = 1.0;
+    double a = 0.0, b = 0.0;  // both 0: fitted
+    double learning_rate = 1.0, repulsion_strength = 1.0, set_op_mix_ratio = 1.0;
+    uint32_t negative_sample_rate = 5;
+    Init init = Init::Pca;
+    uint64_t seed = 0;
+};
+struct Result {
+    std::vector<double> embedding;  // n x n_components, row-major
+    double a = 0.0, b = 0.0, max_weight = 0.0;
+    uint32_t n_epochs = 0;
+    uint64_t n_edges = 0, n_edges_used = 0;
+};
+
+namespace detail {
+inline sb_umap_opts opts(const Options &o) {
+    return sb_umap_opts{o.n_components, o.n_epochs, o.min_dist, o.spread, o.a, o.b, o.learning_rate, o.repulsion_strength, o.set_op_mix_ratio,
+                        o.negative_sample_rate, (uint32_t)o.init, o.seed};
+}
+inline Result result(std::vector<double> emb, const sb_umap_info &info) {
+    return Result{std::move(emb), info.a, info.b, info.max_weight, info.n_epochs, info.n_edges, info.n_edges_used};
+}
+inline uint64_t rows(const std::vector<double> &scores, uint32_t dim, const std::vector<uint32_t> &nbr, uint32_t k) {
+    if (dim == 0 || scores.size() % dim) throw Error(SB_ERR_INVALID_ARG, "scores must hold n x dim entries");
+    if (k == 0 || nbr.size() != scores.size() / dim * k) throw Error(SB_ERR_INVALID_ARG, "nbr must hold n x k entries");
+    return scores.size() / dim;
+}
+}  // namespace detail
+
+// scores: n x dim, nbr: n x k row-major, as knn returns it
+inline Graph umap_graph(const Context &ctx, const std::vector<double> &scores, uint32_t dim, const std::vector<uint32_t> &nbr, uint32_t k,
+                        const Options &o = Options()) {
+    const uint64_t n = detail::rows(scores, dim, nbr, k);
+    Graph g{std::vector<uint64_t>(n + 1), std::vector<uint32_t>(2 * n * k), std::vector<double>(2 * n * k), std::vector<double>(n), std::vector<double>(n)};
+    uint64_t nnz = 0;
+    const sb_umap_opts c = detail::opts(o);
+    check(sb_umap_graph(ctx.raw(), scores.data(), nbr.data(), n, dim, k, &c, g.indptr.data(), g.indices.data(), g.weights.data(), &nnz, g.rho.data(),
+                        g.sigma.data()));
+    g.indices.resize(nnz);
+    g.weights.resize(nnz);
+    return g;
+}
+// init: n x n_components (scaled per column with Init::Pca, as given with Init::User, unused with Init::Random)
+inline Result umap_layout(const Context &ctx, const Graph &g, const std::vector<double> &init, const Options &o = Options()) {
+    if (g.indptr.empty()) throw Error(SB_ERR_INVALID_ARG, "indptr must hold n + 1 entries");
+    const uint64_t n = g.indptr.size() - 1;
+    if (o.init != Init::Random && init.size() != n * o.n_components) throw Error(SB_ERR_INVALID_ARG, "init must hold n x n_components entries");
+    std::vector<double> out(n * o.n_components);
+    sb_umap_info info;
+    const sb_umap_opts c = detail::opts(o);
+    check(sb_umap_layout(ctx.raw(), n, g.indptr.data(), g.indices.data(), g.weights.data(), init.empty() ? nullptr : init.data(), &c, out.data(), &info));
+    return detail::result(std::move(out), info);
+}
+// on a sharded context: this rank's rows (global neighbour indices) -> this rank's rows of the embedding
+inline Result umap(const Context &ctx, const std::vector<double> &scores, uint32_t dim, const std::vector<uint32_t> &nbr, uint32_t k,
+                   const Options &o = Options(), const std::vector<double> &init = {}) {
+    const uint64_t n = detail::rows(scores, dim, nbr, k);
+    if (o.init == Init::User && init.size() != n * o.n_components) throw Error(SB_ERR_INVALID_ARG, "init must hold n x n_components entries");
+    std::vector<double> out(n * o.n_components);
+    sb_umap_info info;
+    const sb_umap_opts c = detail::opts(o);
+    check(sb_umap(ctx.raw(), scores.data(), nbr.data(), n, dim, k, &c, init.empty() ? nullptr : init.data(), out.data(), &info));
+    return detail::result(std::move(out), info);
+}
+}  // namespace embedding
 }  // namespace scanb200

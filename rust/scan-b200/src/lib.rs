@@ -487,6 +487,132 @@ pub fn cluster_knn(ctx: &Context, nbr: &Array2<u32>, opts: &LouvainOptions) -> R
     Ok(clustering(labels, &info))
 }
 
+/// How the UMAP layout starts: the first score columns scaled to [0, 10], the counter hash, or the caller's positions
+#[derive(Clone, Copy, Debug, PartialEq, Eq)]
+pub enum UmapInit {
+    Pca,
+    Random,
+    User,
+}
+
+/// UMAP options (umap-learn's names and defaults; n_epochs 0: 500 up to 10,000 cells, else 200; a = b = 0: fitted)
+#[derive(Clone, Copy, Debug)]
+pub struct UmapOptions {
+    pub n_components: u32,
+    pub n_epochs: u32,
+    pub min_dist: f64,
+    pub spread: f64,
+    pub a: f64,
+    pub b: f64,
+    pub learning_rate: f64,
+    pub repulsion_strength: f64,
+    pub set_op_mix_ratio: f64,
+    pub negative_sample_rate: u32,
+    pub init: UmapInit,
+    pub seed: u64,
+}
+impl Default for UmapOptions {
+    fn default() -> Self {
+        UmapOptions { n_components: 2, n_epochs: 0, min_dist: 0.1, spread: 1.0, a: 0.0, b: 0.0, learning_rate: 1.0, repulsion_strength: 1.0,
+                      set_op_mix_ratio: 1.0, negative_sample_rate: 5, init: UmapInit::Pca, seed: 0 }
+    }
+}
+
+/// The fuzzy kNN graph as a symmetric CSR (weights in (0, 1]) with every vertex's rho and sigma
+#[derive(Clone, Debug)]
+pub struct UmapGraph {
+    pub indptr: Vec<u64>,
+    pub indices: Vec<u32>,
+    pub weights: Vec<f64>,
+    pub rho: Vec<f64>,
+    pub sigma: Vec<f64>,
+}
+
+/// The embedding (n x n_components) and the layout's parameters as used
+#[derive(Clone, Debug)]
+pub struct Umap {
+    pub embedding: Array2<f64>,
+    pub a: f64,
+    pub b: f64,
+    pub n_epochs: u32,
+    pub n_edges: u64,
+    pub n_edges_used: u64,
+    pub max_weight: f64,
+}
+
+fn umap_opts(o: &UmapOptions) -> ffi::sb_umap_opts {
+    let init = match o.init {
+        UmapInit::Pca => ffi::SB_UMAP_INIT_PCA,
+        UmapInit::Random => ffi::SB_UMAP_INIT_RANDOM,
+        UmapInit::User => ffi::SB_UMAP_INIT_USER,
+    };
+    ffi::sb_umap_opts { n_components: o.n_components, n_epochs: o.n_epochs, min_dist: o.min_dist, spread: o.spread, a: o.a, b: o.b,
+                        learning_rate: o.learning_rate, repulsion_strength: o.repulsion_strength, set_op_mix_ratio: o.set_op_mix_ratio,
+                        negative_sample_rate: o.negative_sample_rate, init, seed: o.seed }
+}
+fn umap_result(out: Vec<f64>, n: usize, nc: usize, info: &ffi::sb_umap_info) -> Umap {
+    Umap { embedding: Array2::from_shape_vec((n, nc), out).expect("n x n_components"), a: info.a, b: info.b, n_epochs: info.n_epochs,
+           n_edges: info.n_edges, n_edges_used: info.n_edges_used, max_weight: info.max_weight }
+}
+fn empty_umap_info() -> ffi::sb_umap_info {
+    ffi::sb_umap_info { a: 0.0, b: 0.0, max_weight: 0.0, n_edges: 0, n_edges_used: 0, n_epochs: 0 }
+}
+
+/// The fuzzy kNN graph of the scores (n x dim) and their kNN lists (n x k, as `knn` returns them; the rules are stated beside
+/// `sb_umap_graph` in include/scanb200.h)
+pub fn umap_graph(ctx: &Context, scores: &Array2<f64>, nbr: &Array2<u32>, opts: &UmapOptions) -> Result<UmapGraph, Error> {
+    let scores = scores.as_standard_layout();
+    let nbr = nbr.as_standard_layout();
+    let ((n, dim), k) = (scores.dim(), nbr.dim().1);
+    assert_eq!(nbr.dim().0, n, "scores and nbr must have the same rows");
+    let mut g = UmapGraph { indptr: vec![0; n + 1], indices: vec![0; 2 * n * k], weights: vec![0.0; 2 * n * k], rho: vec![0.0; n], sigma: vec![0.0; n] };
+    let mut nnz = 0u64;
+    let o = umap_opts(opts);
+    check(unsafe {
+        ffi::sb_umap_graph(ctx.h, scores.as_ptr(), nbr.as_ptr(), n as u64, dim as u32, k as u32, &o, g.indptr.as_mut_ptr(), g.indices.as_mut_ptr(),
+                           g.weights.as_mut_ptr(), &mut nnz, g.rho.as_mut_ptr(), g.sigma.as_mut_ptr())
+    })?;
+    g.indices.truncate(nnz as usize);
+    g.weights.truncate(nnz as usize);
+    Ok(g)
+}
+
+/// The layout of a symmetric CSR; `init` (n x n_components) is scaled per column with `UmapInit::Pca`, taken as given with
+/// `UmapInit::User` and not read with `UmapInit::Random`
+pub fn umap_layout(ctx: &Context, g: &UmapGraph, init: Option<&Array2<f64>>, opts: &UmapOptions) -> Result<Umap, Error> {
+    assert!(!g.indptr.is_empty(), "indptr must hold n + 1 entries");
+    let (n, nc) = (g.indptr.len() - 1, opts.n_components as usize);
+    let init = init.map(|a| a.as_standard_layout().into_owned());
+    if let Some(a) = &init {
+        assert_eq!(a.dim(), (n, nc), "init must be n x n_components");
+    }
+    let mut out = vec![0.0; n * nc];
+    let mut info = empty_umap_info();
+    let o = umap_opts(opts);
+    let ip = init.as_ref().map_or(std::ptr::null(), |a| a.as_ptr());
+    check(unsafe { ffi::sb_umap_layout(ctx.h, n as u64, g.indptr.as_ptr(), g.indices.as_ptr(), g.weights.as_ptr(), ip, &o, out.as_mut_ptr(), &mut info) })?;
+    Ok(umap_result(out, n, nc, &info))
+}
+
+/// Scores and kNN lists -> fuzzy graph -> layout with the graph kept on the device; on a sharded context every rank passes its own
+/// rows (global neighbour indices) and receives its own rows of the embedding
+pub fn umap(ctx: &Context, scores: &Array2<f64>, nbr: &Array2<u32>, opts: &UmapOptions, init: Option<&Array2<f64>>) -> Result<Umap, Error> {
+    let scores = scores.as_standard_layout();
+    let nbr = nbr.as_standard_layout();
+    let ((n, dim), k, nc) = (scores.dim(), nbr.dim().1, opts.n_components as usize);
+    assert_eq!(nbr.dim().0, n, "scores and nbr must have the same rows");
+    let init = init.map(|a| a.as_standard_layout().into_owned());
+    if let Some(a) = &init {
+        assert_eq!(a.dim(), (n, nc), "init must be n x n_components");
+    }
+    let mut out = vec![0.0; n * nc];
+    let mut info = empty_umap_info();
+    let o = umap_opts(opts);
+    let ip = init.as_ref().map_or(std::ptr::null(), |a| a.as_ptr());
+    check(unsafe { ffi::sb_umap(ctx.h, scores.as_ptr(), nbr.as_ptr(), n as u64, dim as u32, k as u32, &o, ip, out.as_mut_ptr(), &mut info) })?;
+    Ok(umap_result(out, n, nc, &info))
+}
+
 /// Every GPU of the box from one caller thread (SURVEY 8b; the reference's only caller is a single process).  `run` executes the
 /// closure once per rank, concurrently, each on its own library worker thread with its own `Context`; inside it a rank uploads
 /// its contiguous cell shard and makes the ordinary calls -- the collectives meet across the workers.

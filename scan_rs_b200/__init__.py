@@ -8,6 +8,7 @@ The package mirrors the reference's module layout for this path only:
   mtx            load_mtx (gz MatrixMarket -> device matrix)
   nn             knn, find_nn on the PCA scores
   cluster        SNN graph of the kNN lists and deterministic Louvain (snn_graph, louvain, cluster_knn)
+  embedding      UMAP of the scores and kNN lists: fuzzy graph and deterministic layout (umap_graph, umap_layout, umap)
   diff_exp       sSeq differential expression (compute_sseq_params, sseq_differential_expression, sseq_one_vs_rest)
   synth          synthetic workloads (test / bench utility)
 All compute runs in scan_rs_b200/libscanb200.so (hand-written sm_100a CUDA + cuSOLVER/cuBLAS for the
@@ -26,3 +27,4 @@ from .multi import MultiContext  # noqa: F401
 from .diff_exp import (DiffExpResult, SSeqParams, compute_sseq_params, sseq_differential_expression,  # noqa: F401
                        sseq_one_vs_rest)
 from .cluster import ClusterResult, LouvainOptions, cluster_knn, louvain, snn_graph  # noqa: F401
+from .embedding import UmapOptions, UmapResult, umap, umap_graph, umap_layout  # noqa: F401

@@ -100,7 +100,7 @@ static int sort_keys(sb_ctx *ctx, DevBuf<u64> &keys, u64 count) {
     keys.swap(out);
     return SB_OK;
 }
-static int sort_pairs(sb_ctx *ctx, DevBuf<u64> &keys, DevBuf<u64> &vals, u64 count) {
+int sort_pairs(sb_ctx *ctx, DevBuf<u64> &keys, DevBuf<u64> &vals, u64 count) {
     DevBuf<u64> ko, vo;
     SB_TRY(ko.alloc(count));
     SB_TRY(vo.alloc(count));

@@ -344,6 +344,8 @@ int comm_allreduce_max_i32(sb_ctx *ctx, int *host_val);
 int comm_allgather_u64_host(sb_ctx *ctx, u64 mine, std::vector<u64> &all);
 // every rank takes the same turn before the next collective: a local rejection becomes every rank's error (matrix.cu)
 int agree_status(sb_ctx *ctx, int rc, const char *what);
+// stable radix sort of (keys, vals) by the 64-bit key; the buffers are replaced by the sorted copies (cluster.cu)
+int sort_pairs(sb_ctx *ctx, DevBuf<u64> &keys, DevBuf<u64> &vals, u64 count);
 // percentile_of_sorted (stat.rs:140-163) at the fraction q: rank q (n - 1), linear interpolation; sorts v (moments.cu)
 double percentile_of(std::vector<double> &v, double q);
 
