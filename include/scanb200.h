@@ -359,6 +359,13 @@ SB_API int sb_sseq_diff_exp(sb_mat *mat, const sb_sseq_params *params, const uin
  * each < n_groups; n_groups >= 2; no group may be empty over all ranks).  out arrays are [n_groups x m]. */
 SB_API int sb_sseq_one_vs_rest(sb_mat *mat, const sb_sseq_params *params, const uint32_t *labels, uint32_t n_groups, uint64_t big_count,
                         sb_diff_exp_out *out);
+/* Pairwise comparisons of labelled groups, batched: comparison j is "labels == pairs[2j]" against "labels == pairs[2j + 1]"
+ * (labels[n_local] of this rank's cells, each < n_groups; pairs[n_pairs x 2], n_pairs >= 1, each pair two different groups below
+ * n_groups, neither empty over all ranks; else SB_ERR_INVALID_ARG).  One pass over the matrix for every pair; s of a group is its
+ * cells' size factors summed in global cell order.  Every output row j equals sb_sseq_diff_exp called with the cells of the two
+ * groups, bit for bit.  out arrays are [n_pairs x m]. */
+SB_API int sb_sseq_pairs(sb_mat *mat, const sb_sseq_params *params, const uint32_t *labels, uint32_t n_groups, const uint32_t *pairs,
+                  uint32_t n_pairs, uint64_t big_count, sb_diff_exp_out *out);
 
 /* ---------------------------------------------------------------- kNN on the scores (next step of the pipeline)
  * knn / find_nn (scan-rs/src/nn.rs:38-83): for every query row (n_queries x dim, row-major) the indices of its k nearest points
@@ -416,6 +423,48 @@ SB_API int sb_louvain(sb_ctx *ctx, uint64_t n, const uint64_t *indptr, const uin
                const sb_louvain_opts *opts, uint32_t *labels, sb_louvain_info *info);
 SB_API int sb_cluster_knn(sb_ctx *ctx, const uint32_t *nbr, uint64_t n_local, uint32_t k, const sb_louvain_opts *opts, uint32_t *labels,
                    sb_louvain_info *info);
+
+/* ---------------------------------------------------------------- merging of over-split clusters (Cell Ranger's MERGE_CLUSTERS)
+ * scan-rs's linkage.rs and merge_clusters.rs, restated (neither is pinned here); oracle/merge_clusters.py restates the rule literally.
+ *
+ * sb_linkage_complete: host only, no context.  points[n x dim] (f64, row-major, finite; else SB_ERR_INVALID_ARG), 1 <= n <= 4,096
+ * (SB_ERR_UNSUPPORTED above), dim >= 1 -> Z[(n - 1) x 4] in scipy's layout (scipy.cluster.hierarchy.linkage(method="complete")).
+ *   d(i, j) = sqrt(sum_c (x_j,c - x_i,c)^2), summed in coordinate order without contraction (knn.cu's expression); a non-finite
+ *   distance is SB_ERR_INVALID_ARG.  Between clusters the largest point distance.  NN-chain: the chain starts at the lowest active
+ *   slot; its next element is the active slot nearest to the top -- on a tie the element below the top wins, otherwise the lowest
+ *   slot; two mutual nearest neighbours x < y merge at height d(x, y) into slot y.  The merges are stably sorted by height (equal
+ *   heights keep merge order) and numbered as scipy does: row i = (id_a < id_b, height, size), the new cluster is id n + i.
+ *
+ * sb_merge_clusters: labels[n_local] (each < n_groups, no group empty over all ranks, 1 <= n_groups <= 4,096: SB_ERR_UNSUPPORTED
+ * above), scores[n_local x dim] (the PCA scores, finite, 1 <= dim <= 128), params from sb_sseq_compute_params on the whole matrix.
+ * Each round, with the current clusters numbered 0..K-1 in ascending id:
+ *   1. centroid of a cluster: every score column summed over its cells in ascending global cell order (one rounding per add),
+ *      divided by the cell count;
+ *   2. Z = sb_linkage_complete of the centroids;
+ *   3. candidates: every row of Z whose two children are both leaves (< K); they are disjoint;
+ *   4. one batched pairwise sSeq test (sb_sseq_pairs' path) of every candidate (a, b), a < b, the lower id as the in-group;
+ *   5. a pair merges when fewer than min_de_genes genes have adjusted p < adj_p_threshold; the merged cluster keeps id a;
+ *   6. the survivors are renumbered 0..K'-1 in ascending old id.
+ * Rounds repeat until one merges nothing or one cluster is left (n_rounds counts the rounds that tested pairs).  labels_out[n_local]:
+ * the final clusters numbered by size, descending, ties to the smallest global cell index (sb_cluster_knn's rule, so labels no round
+ * merges come back unchanged).  On a cell-sharded context every rank passes its own labels, score rows and params and receives its
+ * cells' labels; labels, size factors and scores are gathered in global cell order, so the result equals world 1 bit for bit. */
+#define SB_LINKAGE_MAX_POINTS 4096
+typedef struct sb_merge_opts {
+    double adj_p_threshold;  /* 0 < t <= 1 (default 0.05) */
+    uint32_t min_de_genes;   /* a pair with fewer DE genes merges (default 1) */
+    uint32_t reserved;       /* 0 */
+    uint64_t big_count;      /* sSeq's switch to the asymptotic test (default 900) */
+} sb_merge_opts;             /* NULL: the defaults */
+typedef struct sb_merge_info {
+    uint32_t n_clusters;
+    uint32_t n_rounds;
+    uint64_t pairs_tested;
+    uint64_t pairs_merged;
+} sb_merge_info;
+SB_API int sb_linkage_complete(const double *points, uint32_t n, uint32_t dim, double *Z);
+SB_API int sb_merge_clusters(sb_mat *mat, const sb_sseq_params *params, const double *scores, uint32_t dim, const uint32_t *labels,
+                      uint32_t n_groups, const sb_merge_opts *opts, uint32_t *labels_out, sb_merge_info *info);
 
 /* ---------------------------------------------------------------- UMAP embedding (the reference's `umap-rs`, a port of umap-learn)
  * The fuzzy kNN graph and umap-learn's layout, made epoch-synchronous so that the result is bit-reproducible at every grid and

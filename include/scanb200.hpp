@@ -512,6 +512,19 @@ inline std::vector<DiffExpResult> sseq_one_vs_rest(const sqz::AdaptiveMat &mat, 
         return sb_sseq_one_vs_rest(mat.raw(), c, labels.data(), n_groups, big_count, o);
     });
 }
+// one result per pair (a, b): cells labelled a against cells labelled b, one matrix pass for all pairs
+inline std::vector<DiffExpResult> sseq_pairs(const sqz::AdaptiveMat &mat, const std::vector<uint32_t> &labels, uint32_t n_groups,
+                                             const std::vector<std::pair<uint32_t, uint32_t>> &pairs, const SSeqParams &params, uint64_t big_count = 900) {
+    if (labels.size() != mat.cols()) throw Error(SB_ERR_INVALID_ARG, "one label per cell");
+    std::vector<uint32_t> flat;
+    for (const auto &p : pairs) {
+        flat.push_back(p.first);
+        flat.push_back(p.second);
+    }
+    return detail::run(params, pairs.size(), mat.rows(), [&](const sb_sseq_params *c, sb_diff_exp_out *o) {
+        return sb_sseq_pairs(mat.raw(), c, labels.data(), n_groups, flat.data(), (uint32_t)pairs.size(), big_count, o);
+    });
+}
 }  // namespace diff_exp
 
 // graph clustering: SNN graph of the kNN lists and deterministic Louvain (the rules are stated in scanb200.h)
@@ -576,6 +589,41 @@ inline Result cluster_knn(const Context &ctx, const std::vector<uint32_t> &nbr, 
     const sb_louvain_opts c = detail::opts(o);
     check(sb_cluster_knn(ctx.raw(), nbr.data(), n, k, &c, labels.data(), &info));
     return detail::result(std::move(labels), info);
+}
+
+// complete linkage (NN-chain) of points [n x dim] on the host: Z [(n - 1) x 4] in scipy's layout
+inline std::vector<double> linkage_complete(const std::vector<double> &points, uint32_t dim) {
+    if (dim == 0 || points.size() % dim) throw Error(SB_ERR_INVALID_ARG, "points must hold n x dim entries");
+    const uint32_t n = (uint32_t)(points.size() / dim);
+    std::vector<double> Z((n > 1 ? n - 1 : 0) * 4);
+    check(sb_linkage_complete(points.data(), n, dim, Z.data()));
+    return Z;
+}
+struct MergeOptions {
+    double adj_p_threshold = 0.05;
+    uint32_t min_de_genes = 1;
+    uint64_t big_count = 900;
+};
+struct MergeResult {
+    std::vector<uint32_t> labels;  // 0..n_clusters-1, by size, descending
+    uint32_t n_clusters = 0, n_rounds = 0;
+    uint64_t pairs_tested = 0, pairs_merged = 0;
+};
+// Cell Ranger's MERGE_CLUSTERS: scores [n_local x dim] (the PCA scores), labels of this rank's cells
+inline MergeResult merge_clusters(const sqz::AdaptiveMat &mat, const diff_exp::SSeqParams &params, const std::vector<double> &scores, uint32_t dim,
+                                  const std::vector<uint32_t> &labels, uint32_t n_groups, const MergeOptions &o = MergeOptions()) {
+    if (labels.size() != mat.cols() || scores.size() != labels.size() * dim) throw Error(SB_ERR_INVALID_ARG, "one label and one score row per cell");
+    MergeResult r;
+    r.labels.resize(labels.size());
+    const sb_merge_opts c{o.adj_p_threshold, o.min_de_genes, 0, o.big_count};
+    const sb_sseq_params p = diff_exp::detail::view(params);
+    sb_merge_info info;
+    check(sb_merge_clusters(mat.raw(), &p, scores.data(), dim, labels.data(), n_groups, &c, r.labels.data(), &info));
+    r.n_clusters = info.n_clusters;
+    r.n_rounds = info.n_rounds;
+    r.pairs_tested = info.pairs_tested;
+    r.pairs_merged = info.pairs_merged;
+    return r;
 }
 }  // namespace clustering
 

@@ -408,6 +408,17 @@ pub fn sseq_one_vs_rest(mat: &DeviceCountMatrix<'_>, labels: &[u32], n_groups: u
     sseq_run(mat, params, n_groups as usize, |p, o| unsafe { ffi::sb_sseq_one_vs_rest(mat.h, p, labels.as_ptr(), n_groups, big_count, o) })
 }
 
+/// Pairwise comparisons, batched: result j compares the cells labelled `pairs[j].0` with the cells labelled `pairs[j].1`, bit for
+/// bit what `sseq_differential_expression` gives with those cells, in one pass over the matrix
+pub fn sseq_pairs(mat: &DeviceCountMatrix<'_>, labels: &[u32], n_groups: u32, pairs: &[(u32, u32)], params: &SSeqParams, big_count: u64)
+                  -> Result<Vec<DiffExpResult>, Error> {
+    assert_eq!(labels.len(), mat.shape()[1], "one label per cell");
+    let flat: Vec<u32> = pairs.iter().flat_map(|&(a, b)| [a, b]).collect();
+    sseq_run(mat, params, pairs.len(), |p, o| unsafe {
+        ffi::sb_sseq_pairs(mat.h, p, labels.as_ptr(), n_groups, flat.as_ptr(), pairs.len() as u32, big_count, o)
+    })
+}
+
 /// Louvain options: resolution (gamma) > 0, max_levels 1..32, max_iterations per level >= 1
 #[derive(Clone, Copy, Debug)]
 pub struct LouvainOptions {
@@ -485,6 +496,63 @@ pub fn cluster_knn(ctx: &Context, nbr: &Array2<u32>, opts: &LouvainOptions) -> R
     let o = louvain_opts(opts);
     check(unsafe { ffi::sb_cluster_knn(ctx.h, nbr.as_ptr(), n as u64, k as u32, &o, labels.as_mut_ptr(), &mut info) })?;
     Ok(clustering(labels, &info))
+}
+
+/// Complete linkage (NN-chain) of `points` (n x dim) on the host: Z ((n - 1) x 4) in scipy's layout
+pub fn linkage_complete(points: &Array2<f64>) -> Result<Array2<f64>, Error> {
+    let pts = points.as_standard_layout();
+    let (n, dim) = pts.dim();
+    let mut z = Array2::<f64>::zeros((n.saturating_sub(1), 4));
+    check(unsafe { ffi::sb_linkage_complete(pts.as_ptr(), n as u32, dim as u32, z.as_mut_ptr()) })?;
+    Ok(z)
+}
+
+/// Cluster-merge options: a pair merges when fewer than `min_de_genes` genes have adjusted p below `adj_p_threshold`
+#[derive(Clone, Copy, Debug)]
+pub struct MergeOptions {
+    pub adj_p_threshold: f64,
+    pub min_de_genes: u32,
+    pub big_count: u64,
+}
+impl Default for MergeOptions {
+    fn default() -> Self {
+        MergeOptions { adj_p_threshold: 0.05, min_de_genes: 1, big_count: 900 }
+    }
+}
+
+/// Merged labels (0..n_clusters-1, by size, descending), rounds, sibling pairs tested and merged
+#[derive(Clone, Debug)]
+pub struct MergeResult {
+    pub labels: Vec<u32>,
+    pub n_clusters: u32,
+    pub n_rounds: u32,
+    pub pairs_tested: u64,
+    pub pairs_merged: u64,
+}
+
+/// Cell Ranger's MERGE_CLUSTERS (the rule is stated beside `sb_merge_clusters` in include/scanb200.h): `scores` are the PCA scores
+/// of this rank's cells, `labels` their clusters (each < n_groups)
+pub fn merge_clusters(mat: &DeviceCountMatrix<'_>, params: &SSeqParams, scores: &Array2<f64>, labels: &[u32], n_groups: u32, opts: &MergeOptions)
+                      -> Result<MergeResult, Error> {
+    let sc = scores.as_standard_layout();
+    assert_eq!(labels.len(), mat.shape()[1], "one label per cell");
+    assert_eq!(sc.nrows(), labels.len(), "one score row per cell");
+    let mut out = vec![0u32; labels.len()];
+    let mut info = ffi::sb_merge_info { n_clusters: 0, n_rounds: 0, pairs_tested: 0, pairs_merged: 0 };
+    let o = ffi::sb_merge_opts { adj_p_threshold: opts.adj_p_threshold, min_de_genes: opts.min_de_genes, reserved: 0, big_count: opts.big_count };
+    // the library only reads the params (see sseq_run)
+    let (mut sf, mut mean, mut var, mut phi_mm, mut phi) = (params.size_factors.to_owned(), params.gene_means.to_owned(),
+        params.gene_variances.to_owned(), params.gene_moment_phi.to_owned(), params.gene_phi.to_owned());
+    let mut use_g = params.use_genes.mapv(|b| b as u8);
+    let p = ffi::sb_sseq_params {
+        num_cells: params.num_cells as u64, num_genes: params.num_genes as u32, reserved: 0, zeta_hat: params.zeta_hat, delta: params.delta,
+        size_factors: sf.as_mut_ptr(), gene_means: mean.as_mut_ptr(), gene_variances: var.as_mut_ptr(), gene_moment_phi: phi_mm.as_mut_ptr(),
+        gene_phi: phi.as_mut_ptr(), use_genes: use_g.as_mut_ptr(),
+    };
+    check(unsafe {
+        ffi::sb_merge_clusters(mat.h, &p, sc.as_ptr(), sc.ncols() as u32, labels.as_ptr(), n_groups, &o, out.as_mut_ptr(), &mut info)
+    })?;
+    Ok(MergeResult { labels: out, n_clusters: info.n_clusters, n_rounds: info.n_rounds, pairs_tested: info.pairs_tested, pairs_merged: info.pairs_merged })
 }
 
 /// How the UMAP layout starts: the first score columns scaled to [0, 10], the counter hash, or the caller's positions

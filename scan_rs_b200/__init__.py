@@ -7,9 +7,10 @@ The package mirrors the reference's module layout for this path only:
   snoop          NoOpSnoop, AtomicSnoop
   mtx            load_mtx (gz MatrixMarket -> device matrix)
   nn             knn, find_nn on the PCA scores
-  cluster        SNN graph of the kNN lists and deterministic Louvain (snn_graph, louvain, cluster_knn)
+  cluster        SNN graph of the kNN lists and deterministic Louvain (snn_graph, louvain, cluster_knn); merging of over-split
+                 clusters by differential expression (linkage_complete, merge_clusters)
   embedding      UMAP of the scores and kNN lists: fuzzy graph and deterministic layout (umap_graph, umap_layout, umap)
-  diff_exp       sSeq differential expression (compute_sseq_params, sseq_differential_expression, sseq_one_vs_rest)
+  diff_exp       sSeq differential expression (compute_sseq_params, sseq_differential_expression, sseq_one_vs_rest, sseq_pairs)
   synth          synthetic workloads (test / bench utility)
 All compute runs in scan_rs_b200/libscanb200.so (hand-written sm_100a CUDA + cuSOLVER/cuBLAS for the
 small dense steps); there is no CPU fallback."""
@@ -25,6 +26,7 @@ from .mtx import load_mtx  # noqa: F401
 from .nn import find_nn, knn  # noqa: F401
 from .multi import MultiContext  # noqa: F401
 from .diff_exp import (DiffExpResult, SSeqParams, compute_sseq_params, sseq_differential_expression,  # noqa: F401
-                       sseq_one_vs_rest)
-from .cluster import ClusterResult, LouvainOptions, cluster_knn, louvain, snn_graph  # noqa: F401
+                       sseq_one_vs_rest, sseq_pairs)
+from .cluster import (ClusterResult, LouvainOptions, MergeOptions, MergeResult, cluster_knn, linkage_complete, louvain,  # noqa: F401
+                      merge_clusters, snn_graph)
 from .embedding import UmapOptions, UmapResult, umap, umap_graph, umap_layout  # noqa: F401

@@ -346,6 +346,18 @@ int comm_allgather_u64_host(sb_ctx *ctx, u64 mine, std::vector<u64> &all);
 int agree_status(sb_ctx *ctx, int rc, const char *what);
 // stable radix sort of (keys, vals) by the 64-bit key; the buffers are replaced by the sorted copies (cluster.cu)
 int sort_pairs(sb_ctx *ctx, DevBuf<u64> &keys, DevBuf<u64> &vals, u64 count);
+// sSeq pieces shared by diff_exp.cu and merge.cu (diff_exp.cu):
+//   one value per local cell -> the values of all cells in global cell order
+int gather_cells(sb_ctx *ctx, const std::vector<double> &mine, std::vector<double> &all);
+//   params for this matrix and context (sizes, NULL arrays)
+int sseq_check_params(sb_mat *mat, const sb_sseq_params *p, const char *fn);
+//   per-group gene sums of the whole matrix into acc[n_groups x m] (replicated over ranks); d_lab: this rank's labels on the device
+int group_gene_sums(sb_mat *mat, const u32 *d_lab, u32 n_groups, DevBuf<u64> &acc);
+//   the pairwise test stage: comparison j is row rows[2j] of d_sums[. x m] against row rows[2j + 1], with s_in[j] / s_out[j]
+int sseq_pair_tests(sb_mat *mat, const sb_sseq_params *prm, const u64 *d_sums, const std::vector<u32> &rows, const std::vector<double> &s_in,
+                    const std::vector<double> &s_out, u64 big_count, sb_diff_exp_out *out);
+// rows [n_local x width] of every rank, in global cell order, into dst (32-bit words; counts from comm_allgather_u64_host) (umap.cu)
+int um_gather_rows(sb_ctx *ctx, const void *mine_h, u64 n_local, u64 width_words, const std::vector<u64> &counts, u64 maxr, u32 *dst);
 // percentile_of_sorted (stat.rs:140-163) at the fraction q: rank q (n - 1), linear interpolation; sorts v (moments.cu)
 double percentile_of(std::vector<double> &v, double q);
 

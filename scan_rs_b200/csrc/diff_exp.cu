@@ -1,10 +1,10 @@
 // diff_exp.cu -- sSeq differential expression: the statistics of the reference's diff-exp crate (compute_sseq_params,
-// sseq_differential_expression; Cell Ranger's published sSeq, which the crate ports).  The contract is restated beside the three
+// sseq_differential_expression; Cell Ranger's published sSeq, which the crate ports).  The contract is restated beside the four
 // entry points in include/scanb200.h and, literally, in oracle/sseq.py.
 //
 //   params      sb_size_factors + sb_mean_var_axis(axis 1, SizeNormalized view) of moments.cu, then O(m) host work
 //   group sums  k_group_sums: one pass over the cell-major stream, u64 atomics into acc[label * m + gene]; sums_out = total - sums_in
-//               (pairwise: the dual-sum kernel of moments.cu)
+//               (cell lists: the dual-sum kernel of moments.cu; labelled pairs: k_pair_rows picks each pair's two rows of acc)
 //   exact test  the host lists the tests and cuts every sweep x = 0..T into chunks of NB_CHUNK terms; k_nb_sweep evaluates a chunk per
 //               warp with online (max, sum exp) pairs over all terms and over the terms <= l_obs, k_nb_finish folds a test's chunks in
 //               chunk order.  Bit-reproducible and independent of the grid: every term is a fixed function of (test, x), every chunk
@@ -38,6 +38,15 @@ __global__ void k_group_sums(const u64 *__restrict__ ptr, const uint2 *__restric
             const uint2 z = cm[k];
             atomicAdd(&row[z.x], (unsigned long long)z.y);
         }
+    }
+}
+
+// thread per (comparison, gene): in[j] = row rows[2j] of sums, out[j] = row rows[2j + 1]
+__global__ void k_pair_rows(const u64 *__restrict__ sums, u32 m, const u32 *__restrict__ rows, u32 npairs, u64 *__restrict__ in, u64 *__restrict__ out) {
+    for (u64 t = (u64)blockIdx.x * blockDim.x + threadIdx.x; t < (u64)npairs * m; t += (u64)gridDim.x * blockDim.x) {
+        const u64 j = t / m, g = t % m;
+        in[t] = sums[(u64)rows[2 * j] * m + g];
+        out[t] = sums[(u64)rows[2 * j + 1] * m + g];
     }
 }
 
@@ -276,8 +285,22 @@ static int de_grid(sb_ctx *ctx, u64 items, int per_block) {
     return (int)std::max<u64>(1, std::min<u64>((items + per_block - 1) / per_block, (u64)ctx->sm_count * 16));
 }
 
+int group_gene_sums(sb_mat *mat, const u32 *d_lab, u32 n_groups, DevBuf<u64> &acc) {
+    sb_ctx *ctx = mat->ctx;
+    const u64 cells = (u64)n_groups * mat->m;
+    SB_TRY(acc.alloc(cells));
+    SB_CUDA(cudaMemsetAsync(acc.p, 0, cells * sizeof(u64), ctx->stream));
+    if (mat->n && mat->nnz) {
+        ProfScope ps(ctx, PH_REDUCE);
+        k_group_sums<<<de_grid(ctx, mat->n * 32, 256), 256, 0, ctx->stream>>>(mat->cm_ptr.p, mat->cm.p, mat->n, mat->m, d_lab, (unsigned long long *)acc.p);
+        count_launch(ctx);
+        SB_CUDA(cudaGetLastError());
+    }
+    return comm_allreduce_u64(ctx, acc.p, cells);
+}
+
 // one value per local cell -> the values of all cells in global cell order (zero-padded f64 all-reduce: one writer per slot, exact)
-static int gather_cells(sb_ctx *ctx, const std::vector<double> &mine, std::vector<double> &all) {
+int gather_cells(sb_ctx *ctx, const std::vector<double> &mine, std::vector<double> &all) {
     if (ctx->nranks == 1) {
         all = mine;
         return SB_OK;
@@ -300,7 +323,7 @@ static int gather_cells(sb_ctx *ctx, const std::vector<double> &mine, std::vecto
     return SB_OK;
 }
 
-static int check_params(sb_mat *mat, const sb_sseq_params *p, const char *fn) {
+int sseq_check_params(sb_mat *mat, const sb_sseq_params *p, const char *fn) {
     if (!p || !p->size_factors || !p->gene_means || !p->gene_phi || !p->use_genes) return sb_fail(SB_ERR_INVALID_ARG, "%s: NULL params array", fn);
     if (p->num_genes != mat->m || p->num_cells != mat->n_global)
         return sb_fail(SB_ERR_INVALID_ARG, "%s: params are for %u genes x %llu cells, the matrix has %u x %llu", fn, p->num_genes,
@@ -465,6 +488,28 @@ static int sseq_tests(sb_mat *mat, const sb_sseq_params *prm, u32 ncomp, const s
     return SB_OK;
 }
 
+int sseq_pair_tests(sb_mat *mat, const sb_sseq_params *prm, const u64 *d_sums, const std::vector<u32> &rows, const std::vector<double> &s_in,
+                    const std::vector<double> &s_out, u64 big_count, sb_diff_exp_out *out) {
+    sb_ctx *ctx = mat->ctx;
+    const u32 m = mat->m, np = (u32)s_in.size();
+    const u64 total = (u64)np * m;
+    {
+        DevBuf<u32> d_rows;
+        DevBuf<u64> d_in, d_out;
+        SB_TRY(d_rows.alloc(2 * (u64)np));
+        SB_TRY(d_in.alloc(total));
+        SB_TRY(d_out.alloc(total));
+        SB_CUDA(cudaMemcpyAsync(d_rows.p, rows.data(), 2 * (u64)np * sizeof(u32), cudaMemcpyHostToDevice, ctx->stream));
+        k_pair_rows<<<de_grid(ctx, total, 256), 256, 0, ctx->stream>>>(d_sums, m, d_rows.p, np, d_in.p, d_out.p);
+        count_launch(ctx);
+        SB_CUDA(cudaGetLastError());
+        SB_CUDA(cudaMemcpyAsync(out->sums_in, d_in.p, total * sizeof(u64), cudaMemcpyDeviceToHost, ctx->stream));
+        SB_CUDA(cudaMemcpyAsync(out->sums_out, d_out.p, total * sizeof(u64), cudaMemcpyDeviceToHost, ctx->stream));
+        SB_CUDA(cudaStreamSynchronize(ctx->stream));
+    }
+    return sseq_tests(mat, prm, np, s_in, s_out, big_count, out);
+}
+
 static bool de_out_ok(const sb_diff_exp_out *o) {
     return o && o->sums_in && o->sums_out && o->normalized_mean_in && o->normalized_mean_out && o->p_values && o->adjusted_p_values && o->log2_fold_change;
 }
@@ -534,7 +579,7 @@ extern "C" int sb_sseq_diff_exp(sb_mat *mat, const sb_sseq_params *params, const
     if (!mat || !de_out_ok(out) || (!cond_in && n_in) || (!cond_out && n_out)) return sb_fail(SB_ERR_INVALID_ARG, "sb_sseq_diff_exp: bad argument");
     sb_ctx *ctx = mat->ctx;
     SB_ENTER(ctx);
-    int rc = check_params(mat, params, "sb_sseq_diff_exp");
+    int rc = sseq_check_params(mat, params, "sb_sseq_diff_exp");
     const uint64_t *lists[2] = {cond_in, cond_out};
     const uint64_t lens[2] = {n_in, n_out};
     for (int l = 0; l < 2 && rc == SB_OK; l++)
@@ -580,7 +625,7 @@ extern "C" int sb_sseq_one_vs_rest(sb_mat *mat, const sb_sseq_params *params, co
     sb_ctx *ctx = mat->ctx;
     SB_ENTER(ctx);
     const u32 m = mat->m;
-    int rc = check_params(mat, params, "sb_sseq_one_vs_rest");
+    int rc = sseq_check_params(mat, params, "sb_sseq_one_vs_rest");
     for (u64 c = 0; c < mat->n && rc == SB_OK; c++)
         if (labels[c] >= n_groups)
             rc = sb_fail(SB_ERR_INVALID_ARG, "sb_sseq_one_vs_rest: label %u of cell %llu is not below n_groups = %u", labels[c],
@@ -612,15 +657,8 @@ extern "C" int sb_sseq_one_vs_rest(sb_mat *mat, const sb_sseq_params *params, co
         DevBuf<u32> d_lab;
         DevBuf<u64> acc;
         SB_TRY(d_lab.alloc(std::max<u64>(1, mat->n)));
-        SB_TRY(acc.alloc(cells));
         if (mat->n) SB_CUDA(cudaMemcpyAsync(d_lab.p, labels, mat->n * sizeof(u32), cudaMemcpyHostToDevice, ctx->stream));
-        SB_CUDA(cudaMemsetAsync(acc.p, 0, cells * sizeof(u64), ctx->stream));
-        if (mat->n && mat->nnz) {
-            ProfScope ps(ctx, PH_REDUCE);
-            k_group_sums<<<de_grid(ctx, mat->n * 32, 256), 256, 0, ctx->stream>>>(mat->cm_ptr.p, mat->cm.p, mat->n, m, d_lab.p, (unsigned long long *)acc.p);
-            count_launch(ctx);
-        }
-        SB_TRY(comm_allreduce_u64(ctx, acc.p, cells));
+        SB_TRY(group_gene_sums(mat, d_lab.p, n_groups, acc));
         SB_CUDA(cudaMemcpyAsync(out->sums_in, acc.p, cells * sizeof(u64), cudaMemcpyDeviceToHost, ctx->stream));
         SB_CUDA(cudaStreamSynchronize(ctx->stream));
         std::vector<u64> tot(m, 0);
@@ -630,4 +668,52 @@ extern "C" int sb_sseq_one_vs_rest(sb_mat *mat, const sb_sseq_params *params, co
             for (u32 g = 0; g < m; g++) out->sums_out[(u64)j * m + g] = tot[g] - out->sums_in[(u64)j * m + g];
     }
     return sseq_tests(mat, params, n_groups, s_in, s_out, big_count, out);
+}
+
+extern "C" int sb_sseq_pairs(sb_mat *mat, const sb_sseq_params *params, const uint32_t *labels, uint32_t n_groups, const uint32_t *pairs,
+                             uint32_t n_pairs, uint64_t big_count, sb_diff_exp_out *out) {
+    if (!mat || !de_out_ok(out) || (!labels && mat->n) || !pairs || !n_pairs) return sb_fail(SB_ERR_INVALID_ARG, "sb_sseq_pairs: bad argument (n_pairs >= 1)");
+    sb_ctx *ctx = mat->ctx;
+    SB_ENTER(ctx);
+    int rc = sseq_check_params(mat, params, "sb_sseq_pairs");
+    for (u32 j = 0; j < n_pairs && rc == SB_OK; j++)
+        if (pairs[2 * j] == pairs[2 * j + 1] || pairs[2 * j] >= n_groups || pairs[2 * j + 1] >= n_groups)
+            rc = sb_fail(SB_ERR_INVALID_ARG, "sb_sseq_pairs: pair %u = (%u, %u) needs two different groups below n_groups = %u", j, pairs[2 * j],
+                         pairs[2 * j + 1], n_groups);
+    for (u64 c = 0; c < mat->n && rc == SB_OK; c++)
+        if (labels[c] >= n_groups)
+            rc = sb_fail(SB_ERR_INVALID_ARG, "sb_sseq_pairs: label %u of cell %llu is not below n_groups = %u", labels[c],
+                         (unsigned long long)(mat->cell_offset + c), n_groups);
+    SB_TRY(agree_status(ctx, rc, "sb_sseq_pairs"));
+    // s of every group: its size factors summed in global cell order (the bits sb_sseq_diff_exp gets with the group's cell list)
+    std::vector<u64> size(n_groups, 0);
+    std::vector<double> s(n_groups, 0.0);
+    {
+        TraceScope tr(ctx, "sseq: cell gathers");
+        std::vector<double> lab_l(mat->n), lab, sf;
+        for (u64 c = 0; c < mat->n; c++) lab_l[c] = (double)labels[c];
+        SB_TRY(gather_cells(ctx, lab_l, lab));
+        SB_TRY(gather_cells(ctx, std::vector<double>(params->size_factors, params->size_factors + mat->n), sf));
+        for (u64 c = 0; c < lab.size(); c++) {
+            size[(u32)lab[c]]++;
+            s[(u32)lab[c]] += sf[c];
+        }
+    }
+    std::vector<double> s_in(n_pairs), s_out(n_pairs);
+    std::vector<u32> rows(pairs, pairs + 2 * (u64)n_pairs);
+    for (u32 j = 0; j < n_pairs; j++) {
+        for (int h = 0; h < 2; h++)
+            if (!size[pairs[2 * j + h]]) return sb_fail(SB_ERR_INVALID_ARG, "sb_sseq_pairs: group %u (pair %u) is empty", pairs[2 * j + h], j);
+        s_in[j] = s[pairs[2 * j]];
+        s_out[j] = s[pairs[2 * j + 1]];
+    }
+    DevBuf<u64> acc;
+    {
+        TraceScope tr(ctx, "sseq: group sums");
+        DevBuf<u32> d_lab;
+        SB_TRY(d_lab.alloc(std::max<u64>(1, mat->n)));
+        if (mat->n) SB_CUDA(cudaMemcpyAsync(d_lab.p, labels, mat->n * sizeof(u32), cudaMemcpyHostToDevice, ctx->stream));
+        SB_TRY(group_gene_sums(mat, d_lab.p, n_groups, acc));
+    }
+    return sseq_pair_tests(mat, params, acc.p, rows, s_in, s_out, big_count, out);
 }

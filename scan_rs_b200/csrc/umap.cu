@@ -805,8 +805,7 @@ extern "C" int sb_umap_layout(sb_ctx *ctx, uint64_t n, const uint64_t *indptr, c
     return um_copy_out(ctx, Y, 0, n, o.nc, out);
 }
 
-// rows [n_local x width] of every rank, in global cell order, into dst (32-bit words; counts from comm_allgather_u64_host)
-static int um_gather_rows(sb_ctx *ctx, const void *mine_h, u64 n_local, u64 width_words, const std::vector<u64> &counts, u64 maxr, u32 *dst) {
+int um_gather_rows(sb_ctx *ctx, const void *mine_h, u64 n_local, u64 width_words, const std::vector<u64> &counts, u64 maxr, u32 *dst) {
     const u64 slab = maxr * width_words;
     DevBuf<u32> mine, all;
     SB_TRY(mine.alloc(slab));

@@ -4,6 +4,7 @@ published sSeq), on the device through the C ABI (csrc/diff_exp.cu; the contract
     params = compute_sseq_params(mat)                         # size factors, shrunken per-gene dispersions
     res = sseq_differential_expression(mat, cells_a, cells_b, params)
     per_cluster = sseq_one_vs_rest(mat, labels, params)       # Cell Ranger's cluster-vs-rest loop, batched
+    pairwise = sseq_pairs(mat, labels, [(0, 1), (2, 3)], params)  # group a against group b, one matrix pass for all pairs
 
 On a sharded context every rank passes its own cells (local indices / labels) and the params it computed; gene-sized results come
 back replicated."""
@@ -102,3 +103,15 @@ def sseq_one_vs_rest(mat, labels, params: SSeqParams, big_count: int = 900, n_gr
         n_groups = int(lab.max()) + 1 if lab.size else 0
     call = lambda cp, out: L.lib().sb_sseq_one_vs_rest(mat._h, cp, L.vp(lab), C.c_uint32(n_groups), C.c_uint64(big_count), out)
     return _run(mat, params, max(int(n_groups), 1), call)
+
+
+def sseq_pairs(mat, labels, pairs, params: SSeqParams, big_count: int = 900, n_groups: int | None = None) -> List[DiffExpResult]:
+    """One result per pair (a, b): cells labelled a against cells labelled b, each equal bit for bit to
+    sseq_differential_expression with those cells.  n_groups defaults to max(label) + 1 (on a sharded context pass it)."""
+    lab = np.ascontiguousarray(labels, dtype=np.uint32)
+    pr = np.ascontiguousarray(np.asarray(pairs, dtype=np.uint32).reshape(-1, 2))
+    if n_groups is None:
+        n_groups = int(lab.max()) + 1 if lab.size else 0
+    call = lambda cp, out: L.lib().sb_sseq_pairs(mat._h, cp, L.vp(lab), C.c_uint32(n_groups), L.vp(pr), C.c_uint32(pr.shape[0]),
+                                                 C.c_uint64(big_count), out)
+    return _run(mat, params, max(pr.shape[0], 1), call)
