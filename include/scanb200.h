@@ -540,6 +540,91 @@ SB_API int sb_umap_layout(sb_ctx *ctx, uint64_t n, const uint64_t *indptr, const
 SB_API int sb_umap(sb_ctx *ctx, const double *scores, const uint32_t *nbr, uint64_t n_local, uint32_t dim, uint32_t k, const sb_umap_opts *opts,
             const double *init, double *out, sb_umap_info *info);
 
+/* ---------------------------------------------------------------- t-SNE embedding (the reference's `bhtsne`, van der Maaten's
+ * Barnes-Hut t-SNE) with bhtsne's parameter names, defaults and schedule; restated by oracle/tsne.py.
+ *
+ * Ordered sums: a sum over m values is taken in chunks of 1,024 (chunk c: values [1024 c, 1024 (c + 1))), each chunk left to right
+ * from its first value, then the chunk sums left to right.  The order depends on m alone, never on the grid, the SM count or the
+ * world size.
+ *
+ * sb_tsne_affinities: scores X[n x dim] (f64, row-major) and nbr[n x k] as sb_knn(..., include_self = 0) returns them.  bhtsne
+ * lists K = floor(3 perplexity) neighbours: callers pass k = min(n - 1, K).  SB_ERR_INVALID_ARG: perplexity not finite or not > 0,
+ * n - 1 < 3 perplexity, k < min(n - 1, K), an index >= n, a self index, a duplicate in a row, padding before a row end;
+ * SB_ERR_UNSUPPORTED: k > 128, n k >= 2^28.  All listed slots of a row are used.
+ *   scaling  X minus its column means (ordered sums over the cells, / n), then divided by the largest |x| (skipped when 0), as
+ *            bhtsne's run does;
+ *   d_ij     sqrt(sum_c (x_j,c - x_i,c)^2) in coordinate order without contraction (knn.cu's ranking expression); D_ij = d_ij d_ij;
+ *   beta_i   bhtsne's computeGaussianPerplexity: beta = 1, min = -DBL_MAX, max = DBL_MAX; at most 200 steps of p_j = exp(-(beta D_ij)),
+ *            sum_P = DBL_MIN + the p_j in slot order, H = (sum over slots of beta (D_ij p_j)) / sum_P + log(sum_P); stop when
+ *            |H - log(perplexity)| < 1e-5; H above: min = beta, beta = max still +-DBL_MAX ? 2 beta : (beta + max) / 2; below:
+ *            max = beta, beta = min still +-DBL_MAX ? beta / 2 : (beta + min) / 2.  P_j|i = p_j / sum_P of the last step; beta[i]
+ *            is the beta of that step;
+ *   P        P_ij = P_j|i + P_i|j (0 when not listed), zeros dropped, stored both ways with columns ascending, then divided by
+ *            their total (an ordered sum in CSR order).
+ * indices / P must hold 2 n k entries; *nnz receives the count; beta (n) may be NULL.
+ *
+ * sb_tsne_layout: P as a host CSR of n points: symmetric (equal values both ways), no duplicate entry, entries in (0, 1] (checked
+ * on the device: SB_ERR_INVALID_ARG); a row is taken with columns ascending.  n_components must be 2 (else SB_ERR_UNSUPPORTED).
+ * Start (init[n x 2], f64): SB_TSNE_INIT_PCA (default) takes the two columns divided by the population standard deviation of
+ * column 0 (ordered sums: the mean, then the squared deviations; a zero or non-finite deviation is SB_ERR_INVALID_ARG) times 1e-4,
+ * as sklearn and openTSNE do; SB_TSNE_INIT_USER takes them as given (finite); SB_TSNE_INIT_RANDOM ignores them: point i gets
+ * 1e-4 (r cos a, r sin a), r = sqrt(-2 log u1), a = 6.283185307179586 u2, u1 = ((h(2i) >> 11) + 1) 2^-53, u2 = (h(2i + 1) >> 11)
+ * 2^-53, h(x) = mix64(mix64(mix64(seed) ^ (2^64 - 1)) ^ x) (mix64: SplitMix64's finaliser), bhtsne's N(0, 1e-4^2).
+ * Iteration t = 0..max_iter-1 (no host round trip inside the loop; every operation below is one correctly rounded f64 op):
+ *   tree     root box: centre = the mean of Y (ordered sums / n), half-width h_a = max(max_a - mean_a, mean_a - min_a) + 1e-5;
+ *            per point and axis q_a = floor((y_a - (mean_a - h_a)) / (h_a + h_a) 2^32) clamped to [0, 2^32 - 1]; the 64-bit Morton
+ *            code has the bits of q_x at the odd positions (bit 63 the top x bit) and of q_y at the even.  Codes sorted (ties in
+ *            cell order); a run of equal codes is one leaf; the internal nodes are the binary radix tree of the distinct codes
+ *            (Karras 2012).  A leaf's count and sum of y are its run summed in sorted order; an internal node's are left + right.
+ *            An internal node with a common prefix of p bits has half-widths h_x 2^-ceil(p/2), h_y 2^-floor(p/2).
+ *   forces   for every point i: pos_i = sum over its CSR row (columns ascending) of ((e P_ij) / ((1 + b_x b_x) + b_y b_y)) b,
+ *            b = y_i - y_j, e = early_exaggeration for t <= stop_lying_iter, else 1.  neg_i and q_i: a walk from the root, left
+ *            child before right; a node's centre c = sum / count (a leaf holding i: count - 1 points at (sum - y_i) / (count - 1),
+ *            skipped when count = 1), b = y_i - c, D = b_x b_x + b_y b_y; an internal node is opened unless max(half-widths) / sqrt(D)
+ *            < theta; otherwise (and at every leaf) w = 1 / (1 + D), q_i += count w, neg_i += ((count w) w) b.  theta = 0 gives the
+ *            exact gradient.  sum_Q = the ordered sum of q_i over the points in cell order.
+ *   update   dY = pos - neg / sum_Q; gains (from 1): sign(dY) != sign(uY) ? gains + 0.2 : gains 0.8, floor 0.01; uY (from 0) =
+ *            mom uY - (eta gains) dY, mom = 0.5 for t <= mom_switch_iter, else 0.8; Y += uY; then Y minus its mean (ordered sums).
+ * eta = learning_rate, or max(n / (4 early_exaggeration), 50) when it is 0.  info: kl_divergence as bhtsne's evaluateError
+ * estimates it on the final Y (sum_Q from the same walk; sum of P_ij log((P_ij + FLT_MIN) / (Q_ij + FLT_MIN)), Q_ij = (1 / (1 +
+ * |y_i - y_j|^2)) / sum_Q, per row in CSR order, the rows in an ordered sum), the learning rate used, the entries of P and the
+ * iterations.  out[n x 2] (f64).
+ *
+ * sb_tsne: sb_tsne_affinities + sb_tsne_layout with P kept on the device; SB_TSNE_INIT_PCA starts from the first two columns of the
+ * (unscaled) scores, SB_TSNE_INIT_USER from init (this rank's rows).  On a cell-sharded context every rank passes its own rows of X
+ * and nbr (global indices) and receives its own rows of the embedding; the rows are gathered in global cell order and every rank
+ * runs the same layout, so the embedding equals world 1 bit for bit.
+ * Parity with the `bhtsne` crate is not pinned: its source is not part of this project. */
+#define SB_TSNE_INIT_PCA 0
+#define SB_TSNE_INIT_RANDOM 1
+#define SB_TSNE_INIT_USER 2
+typedef struct sb_tsne_opts {
+    double perplexity;          /* > 0 (default 30) */
+    double theta;               /* Barnes-Hut accuracy, >= 0 (default 0.5; 0: exact) */
+    double learning_rate;       /* eta >= 0 (default 200; 0: max(n / (4 early_exaggeration), 50)) */
+    double early_exaggeration;  /* > 0 (default 12) */
+    uint32_t max_iter;          /* iterations (default 1000) */
+    uint32_t stop_lying_iter;   /* last iteration with the exaggeration (default 250) */
+    uint32_t mom_switch_iter;   /* last iteration with momentum 0.5 (default 250) */
+    uint32_t n_components;      /* 2 */
+    uint32_t init;              /* SB_TSNE_INIT_PCA (default), SB_TSNE_INIT_RANDOM, SB_TSNE_INIT_USER */
+    uint32_t reserved;          /* 0 */
+    uint64_t seed;              /* the random start (default 0) */
+} sb_tsne_opts;                 /* NULL: the defaults */
+typedef struct sb_tsne_info {
+    double kl_divergence;       /* bhtsne's estimate on the final embedding */
+    double learning_rate;       /* as used */
+    uint64_t nnz;               /* entries of P */
+    uint32_t n_iter;
+    uint32_t reserved;
+} sb_tsne_info;
+SB_API int sb_tsne_affinities(sb_ctx *ctx, const double *scores, const uint32_t *nbr, uint64_t n, uint32_t dim, uint32_t k, const sb_tsne_opts *opts,
+                       uint64_t *indptr, uint32_t *indices, double *P, uint64_t *nnz, double *beta);
+SB_API int sb_tsne_layout(sb_ctx *ctx, uint64_t n, const uint64_t *indptr, const uint32_t *indices, const double *P, const double *init,
+                   const sb_tsne_opts *opts, double *out, sb_tsne_info *info);
+SB_API int sb_tsne(sb_ctx *ctx, const double *scores, const uint32_t *nbr, uint64_t n_local, uint32_t dim, uint32_t k, const sb_tsne_opts *opts,
+            const double *init, double *out, sb_tsne_info *info);
+
 /* ---------------------------------------------------------------- measurement
  * Device-side timing on the context's own stream (CUDA events) and per-kernel accounting;
  * bench.py builds its roofline object from these.  Not part of the reference interface. */

@@ -15,6 +15,7 @@
 //   diff_exp::{compute_sseq_params,..} diff-exp/src/diff_exp.rs   scanb200::diff_exp::*
 //   leiden (Louvain), SNN graph      leiden crate (deterministic)  scanb200::clustering::*
 //   umap-rs (UMAP)                   umap-rs crate (deterministic) scanb200::embedding::*
+//   bhtsne (t-SNE)                   bhtsne crate (deterministic)  scanb200::embedding::tsne*
 #pragma once
 #include <type_traits>
 #include <algorithm>
@@ -702,6 +703,74 @@ inline Result umap(const Context &ctx, const std::vector<double> &scores, uint32
     const sb_umap_opts c = detail::opts(o);
     check(sb_umap(ctx.raw(), scores.data(), nbr.data(), n, dim, k, &c, init.empty() ? nullptr : init.data(), out.data(), &info));
     return detail::result(std::move(out), info);
+}
+// t-SNE embedding: perplexity-calibrated affinities and a deterministic Barnes-Hut layout (the rules are stated in scanb200.h)
+struct Affinities {  // symmetric P as a CSR, entries in (0, 1] summing to 1
+    std::vector<uint64_t> indptr;
+    std::vector<uint32_t> indices;
+    std::vector<double> P;
+    std::vector<double> beta;  // per point (from tsne_affinities)
+};
+enum class TsneInit : uint32_t { Pca = SB_TSNE_INIT_PCA, Random = SB_TSNE_INIT_RANDOM, User = SB_TSNE_INIT_USER };
+struct TsneOptions {  // bhtsne's names and defaults
+    double perplexity = 30.0;
+    double theta = 0.5;             // 0: the exact gradient
+    double learning_rate = 200.0;   // 0: max(n / (4 early_exaggeration), 50)
+    double early_exaggeration = 12.0;
+    uint32_t max_iter = 1000, stop_lying_iter = 250, mom_switch_iter = 250;
+    TsneInit init = TsneInit::Pca;
+    uint64_t seed = 0;
+};
+struct TsneResult {
+    std::vector<double> embedding;  // n x 2, row-major
+    double kl_divergence = 0.0, learning_rate = 0.0;
+    uint64_t nnz = 0;
+    uint32_t n_iter = 0;
+};
+
+namespace detail {
+inline sb_tsne_opts tsne_opts(const TsneOptions &o) {
+    return sb_tsne_opts{o.perplexity, o.theta, o.learning_rate, o.early_exaggeration, o.max_iter, o.stop_lying_iter, o.mom_switch_iter, 2,
+                        (uint32_t)o.init, 0, o.seed};
+}
+inline TsneResult tsne_result(std::vector<double> emb, const sb_tsne_info &info) {
+    return TsneResult{std::move(emb), info.kl_divergence, info.learning_rate, info.nnz, info.n_iter};
+}
+}  // namespace detail
+
+// scores: n x dim, nbr: n x k row-major, as knn returns it (k = min(n - 1, floor(3 perplexity)))
+inline Affinities tsne_affinities(const Context &ctx, const std::vector<double> &scores, uint32_t dim, const std::vector<uint32_t> &nbr, uint32_t k,
+                                  const TsneOptions &o = TsneOptions()) {
+    const uint64_t n = detail::rows(scores, dim, nbr, k);
+    Affinities a{std::vector<uint64_t>(n + 1), std::vector<uint32_t>(2 * n * k), std::vector<double>(2 * n * k), std::vector<double>(n)};
+    uint64_t nnz = 0;
+    const sb_tsne_opts c = detail::tsne_opts(o);
+    check(sb_tsne_affinities(ctx.raw(), scores.data(), nbr.data(), n, dim, k, &c, a.indptr.data(), a.indices.data(), a.P.data(), &nnz, a.beta.data()));
+    a.indices.resize(nnz);
+    a.P.resize(nnz);
+    return a;
+}
+// init: n x 2 (the first two score columns with TsneInit::Pca, as given with TsneInit::User, unused with TsneInit::Random)
+inline TsneResult tsne_layout(const Context &ctx, const Affinities &a, const std::vector<double> &init, const TsneOptions &o = TsneOptions()) {
+    if (a.indptr.empty()) throw Error(SB_ERR_INVALID_ARG, "indptr must hold n + 1 entries");
+    const uint64_t n = a.indptr.size() - 1;
+    if (o.init != TsneInit::Random && init.size() != n * 2) throw Error(SB_ERR_INVALID_ARG, "init must hold n x 2 entries");
+    std::vector<double> out(n * 2);
+    sb_tsne_info info;
+    const sb_tsne_opts c = detail::tsne_opts(o);
+    check(sb_tsne_layout(ctx.raw(), n, a.indptr.data(), a.indices.data(), a.P.data(), init.empty() ? nullptr : init.data(), &c, out.data(), &info));
+    return detail::tsne_result(std::move(out), info);
+}
+// on a sharded context: this rank's rows (global neighbour indices) -> this rank's rows of the embedding
+inline TsneResult tsne(const Context &ctx, const std::vector<double> &scores, uint32_t dim, const std::vector<uint32_t> &nbr, uint32_t k,
+                       const TsneOptions &o = TsneOptions(), const std::vector<double> &init = {}) {
+    const uint64_t n = detail::rows(scores, dim, nbr, k);
+    if (o.init == TsneInit::User && init.size() != n * 2) throw Error(SB_ERR_INVALID_ARG, "init must hold n x 2 entries");
+    std::vector<double> out(n * 2);
+    sb_tsne_info info;
+    const sb_tsne_opts c = detail::tsne_opts(o);
+    check(sb_tsne(ctx.raw(), scores.data(), nbr.data(), n, dim, k, &c, init.empty() ? nullptr : init.data(), out.data(), &info));
+    return detail::tsne_result(std::move(out), info);
 }
 }  // namespace embedding
 }  // namespace scanb200

@@ -681,6 +681,126 @@ pub fn umap(ctx: &Context, scores: &Array2<f64>, nbr: &Array2<u32>, opts: &UmapO
     Ok(umap_result(out, n, nc, &info))
 }
 
+/// Start of the t-SNE layout
+#[derive(Clone, Copy, Debug, PartialEq, Eq)]
+pub enum TsneInit {
+    Pca,
+    Random,
+    User,
+}
+
+/// t-SNE options (bhtsne's names and defaults; learning_rate 0: max(n / (4 early_exaggeration), 50); 2 components)
+#[derive(Clone, Copy, Debug)]
+pub struct TsneOptions {
+    pub perplexity: f64,
+    pub theta: f64,
+    pub learning_rate: f64,
+    pub early_exaggeration: f64,
+    pub max_iter: u32,
+    pub stop_lying_iter: u32,
+    pub mom_switch_iter: u32,
+    pub init: TsneInit,
+    pub seed: u64,
+}
+impl Default for TsneOptions {
+    fn default() -> Self {
+        TsneOptions { perplexity: 30.0, theta: 0.5, learning_rate: 200.0, early_exaggeration: 12.0, max_iter: 1000, stop_lying_iter: 250,
+                      mom_switch_iter: 250, init: TsneInit::Pca, seed: 0 }
+    }
+}
+
+/// The symmetric affinities P as a CSR (entries in (0, 1], summing to 1) with every point's beta
+#[derive(Clone, Debug)]
+pub struct TsneAffinities {
+    pub indptr: Vec<u64>,
+    pub indices: Vec<u32>,
+    pub p: Vec<f64>,
+    pub beta: Vec<f64>,
+}
+
+/// The embedding (n x 2) and the layout's summary
+#[derive(Clone, Debug)]
+pub struct Tsne {
+    pub embedding: Array2<f64>,
+    pub kl_divergence: f64,
+    pub learning_rate: f64,
+    pub nnz: u64,
+    pub n_iter: u32,
+}
+
+fn tsne_opts(o: &TsneOptions) -> ffi::sb_tsne_opts {
+    let init = match o.init {
+        TsneInit::Pca => ffi::SB_TSNE_INIT_PCA,
+        TsneInit::Random => ffi::SB_TSNE_INIT_RANDOM,
+        TsneInit::User => ffi::SB_TSNE_INIT_USER,
+    };
+    ffi::sb_tsne_opts { perplexity: o.perplexity, theta: o.theta, learning_rate: o.learning_rate, early_exaggeration: o.early_exaggeration,
+                        max_iter: o.max_iter, stop_lying_iter: o.stop_lying_iter, mom_switch_iter: o.mom_switch_iter, n_components: 2, init,
+                        reserved: 0, seed: o.seed }
+}
+fn tsne_result(out: Vec<f64>, n: usize, info: &ffi::sb_tsne_info) -> Tsne {
+    Tsne { embedding: Array2::from_shape_vec((n, 2), out).expect("n x 2"), kl_divergence: info.kl_divergence, learning_rate: info.learning_rate,
+           nnz: info.nnz, n_iter: info.n_iter }
+}
+fn empty_tsne_info() -> ffi::sb_tsne_info {
+    ffi::sb_tsne_info { kl_divergence: 0.0, learning_rate: 0.0, nnz: 0, n_iter: 0, reserved: 0 }
+}
+
+/// The t-SNE affinities of the scores (n x dim) and their kNN lists (n x k with k = min(n - 1, floor(3 perplexity)), as `knn`
+/// returns them; the rules are stated beside `sb_tsne_affinities` in include/scanb200.h)
+pub fn tsne_affinities(ctx: &Context, scores: &Array2<f64>, nbr: &Array2<u32>, opts: &TsneOptions) -> Result<TsneAffinities, Error> {
+    let scores = scores.as_standard_layout();
+    let nbr = nbr.as_standard_layout();
+    let ((n, dim), k) = (scores.dim(), nbr.dim().1);
+    assert_eq!(nbr.dim().0, n, "scores and nbr must have the same rows");
+    let mut a = TsneAffinities { indptr: vec![0; n + 1], indices: vec![0; 2 * n * k], p: vec![0.0; 2 * n * k], beta: vec![0.0; n] };
+    let mut nnz = 0u64;
+    let o = tsne_opts(opts);
+    check(unsafe {
+        ffi::sb_tsne_affinities(ctx.h, scores.as_ptr(), nbr.as_ptr(), n as u64, dim as u32, k as u32, &o, a.indptr.as_mut_ptr(), a.indices.as_mut_ptr(),
+                                a.p.as_mut_ptr(), &mut nnz, a.beta.as_mut_ptr())
+    })?;
+    a.indices.truncate(nnz as usize);
+    a.p.truncate(nnz as usize);
+    Ok(a)
+}
+
+/// The t-SNE layout of P from `init` (n x 2: the first two score columns with TsneInit::Pca, as given with TsneInit::User, unused
+/// with TsneInit::Random)
+pub fn tsne_layout(ctx: &Context, a: &TsneAffinities, init: Option<&Array2<f64>>, opts: &TsneOptions) -> Result<Tsne, Error> {
+    assert!(!a.indptr.is_empty(), "indptr must hold n + 1 entries");
+    let n = a.indptr.len() - 1;
+    let init = init.map(|x| x.as_standard_layout().into_owned());
+    if let Some(x) = &init {
+        assert_eq!(x.dim(), (n, 2), "init must be n x 2");
+    }
+    let mut out = vec![0.0; n * 2];
+    let mut info = empty_tsne_info();
+    let o = tsne_opts(opts);
+    let ip = init.as_ref().map_or(std::ptr::null(), |x| x.as_ptr());
+    check(unsafe { ffi::sb_tsne_layout(ctx.h, n as u64, a.indptr.as_ptr(), a.indices.as_ptr(), a.p.as_ptr(), ip, &o, out.as_mut_ptr(), &mut info) })?;
+    Ok(tsne_result(out, n, &info))
+}
+
+/// Scores and kNN lists -> affinities -> layout with P kept on the device; on a sharded context every rank passes its own rows
+/// (global neighbour indices) and gets its own rows of the embedding
+pub fn tsne(ctx: &Context, scores: &Array2<f64>, nbr: &Array2<u32>, opts: &TsneOptions, init: Option<&Array2<f64>>) -> Result<Tsne, Error> {
+    let scores = scores.as_standard_layout();
+    let nbr = nbr.as_standard_layout();
+    let ((n, dim), k) = (scores.dim(), nbr.dim().1);
+    assert_eq!(nbr.dim().0, n, "scores and nbr must have the same rows");
+    let init = init.map(|x| x.as_standard_layout().into_owned());
+    if let Some(x) = &init {
+        assert_eq!(x.dim(), (n, 2), "init must be n x 2");
+    }
+    let mut out = vec![0.0; n * 2];
+    let mut info = empty_tsne_info();
+    let o = tsne_opts(opts);
+    let ip = init.as_ref().map_or(std::ptr::null(), |x| x.as_ptr());
+    check(unsafe { ffi::sb_tsne(ctx.h, scores.as_ptr(), nbr.as_ptr(), n as u64, dim as u32, k as u32, &o, ip, out.as_mut_ptr(), &mut info) })?;
+    Ok(tsne_result(out, n, &info))
+}
+
 /// Every GPU of the box from one caller thread (SURVEY 8b; the reference's only caller is a single process).  `run` executes the
 /// closure once per rank, concurrently, each on its own library worker thread with its own `Context`; inside it a rank uploads
 /// its contiguous cell shard and makes the ordinary calls -- the collectives meet across the workers.

@@ -9,7 +9,8 @@ The package mirrors the reference's module layout for this path only:
   nn             knn, find_nn on the PCA scores
   cluster        SNN graph of the kNN lists and deterministic Louvain (snn_graph, louvain, cluster_knn); merging of over-split
                  clusters by differential expression (linkage_complete, merge_clusters)
-  embedding      UMAP of the scores and kNN lists: fuzzy graph and deterministic layout (umap_graph, umap_layout, umap)
+  embedding      UMAP of the scores and kNN lists: fuzzy graph and deterministic layout (umap_graph, umap_layout, umap); t-SNE:
+                 perplexity-calibrated affinities and a deterministic Barnes-Hut layout (tsne_affinities, tsne_layout, tsne)
   diff_exp       sSeq differential expression (compute_sseq_params, sseq_differential_expression, sseq_one_vs_rest, sseq_pairs)
   synth          synthetic workloads (test / bench utility)
 All compute runs in scan_rs_b200/libscanb200.so (hand-written sm_100a CUDA + cuSOLVER/cuBLAS for the
@@ -29,4 +30,5 @@ from .diff_exp import (DiffExpResult, SSeqParams, compute_sseq_params, sseq_diff
                        sseq_one_vs_rest, sseq_pairs)
 from .cluster import (ClusterResult, LouvainOptions, MergeOptions, MergeResult, cluster_knn, linkage_complete, louvain,  # noqa: F401
                       merge_clusters, snn_graph)
-from .embedding import UmapOptions, UmapResult, umap, umap_graph, umap_layout  # noqa: F401
+from .embedding import (TsneOptions, TsneResult, UmapOptions, UmapResult, tsne, tsne_affinities, tsne_layout, umap, umap_graph,  # noqa: F401
+                        umap_layout)

@@ -358,6 +358,36 @@ int sseq_pair_tests(sb_mat *mat, const sb_sseq_params *prm, const u64 *d_sums, c
                     const std::vector<double> &s_out, u64 big_count, sb_diff_exp_out *out);
 // rows [n_local x width] of every rank, in global cell order, into dst (32-bit words; counts from comm_allgather_u64_host) (umap.cu)
 int um_gather_rows(sb_ctx *ctx, const void *mine_h, u64 n_local, u64 width_words, const std::vector<u64> &counts, u64 maxr, u32 *dst);
+// kNN-graph pieces shared by umap.cu and tsne.cu (defined in umap.cu):
+//   SplitMix64's finaliser, the counter hash of negative samples and random starts
+__host__ __device__ __forceinline__ u64 um_mix64(u64 z) {
+    z += 0x9E3779B97F4A7C15ull;
+    z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ull;
+    z = (z ^ (z >> 27)) * 0x94D049BB133111EBull;
+    return z ^ (z >> 31);
+}
+//   thread per (row, slot) of nbr [n x k] (0xFFFFFFFF pads a row's end): err bits 1 index >= n, 2 self index, 4 duplicate in the
+//   row, 8 padding before the row end; d = sqrt(sum_c (x_j,c - x_i,c)^2) in coordinate order without contraction (0 at padding)
+__global__ void k_um_dist(const double *__restrict__ X, const u32 *__restrict__ nbr, u64 n, u32 dim, u32 k, double *__restrict__ d,
+                          int *__restrict__ err);
+//   a weighted graph on the device: symmetric CSR, columns ascending, f64 weights in (0, 1]
+struct UmGraph {
+    u64 n = 0, nnz = 0;
+    DevBuf<u64> ptr;     // [n + 1]
+    DevBuf<u32> idx;     // [nnz]
+    DevBuf<double> w;    // [nnz]
+};
+//   the flagged entries of in[count] into out, their number into *d_num (device); T = u32, u64 or double
+template <typename T>
+int um_select(sb_ctx *ctx, const T *in, const char *flags, T *out, u64 count, u64 *d_num);
+//   keys (row << 32 | col, ascending) of g.nnz entries -> g.ptr, g.idx
+int um_rows_from_keys(sb_ctx *ctx, const u64 *keys, UmGraph &g);
+//   a host CSR of n vertices: n < 2^32 - 1, indptr from 0 and non-decreasing, arrays present when there are entries
+int um_csr_host_check(u64 n, const u64 *indptr, const u32 *indices, const double *weights, const char *fn);
+//   the host CSR (checked above) to g, validated on the device: column < n, weights in (0, 1], no duplicate, symmetric with equal
+//   weights both ways (SB_ERR_INVALID_ARG otherwise); columns ascending in g; trace: the name of the validation's trace scope
+int um_csr_upload(sb_ctx *ctx, u64 n, const u64 *indptr, const u32 *indices, const double *weights, UmGraph &g, const char *fn,
+                  const char *trace);
 // percentile_of_sorted (stat.rs:140-163) at the fraction q: rank q (n - 1), linear interpolation; sorts v (moments.cu)
 double percentile_of(std::vector<double> &v, double q);
 

@@ -28,20 +28,11 @@
 typedef unsigned long long ull;
 typedef long long i64;
 
-__host__ __device__ __forceinline__ u64 um_mix64(u64 z) {  // SplitMix64's finaliser
-    z += 0x9E3779B97F4A7C15ull;
-    z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ull;
-    z = (z ^ (z >> 27)) * 0x94D049BB133111EBull;
-    return z ^ (z >> 31);
-}
-
 static int um_grid(sb_ctx *ctx, u64 items, int per_block) {
     return (int)std::max<u64>(1, std::min<u64>((items + per_block - 1) / per_block, (u64)ctx->sm_count * 32));
 }
 
 // ---------------------------------------------------------------- graph
-// thread per (row, slot): err bits 1 index >= n, 2 self index, 4 duplicate in the row, 8 padding before the row end;
-// d = sqrt(sum_c (x_j,c - x_i,c)^2) in coordinate order without contraction (0 at padding)
 __global__ void k_um_dist(const double *__restrict__ X, const u32 *__restrict__ nbr, u64 n, u32 dim, u32 k, double *__restrict__ d,
                           int *__restrict__ err) {
     for (u64 s = (u64)blockIdx.x * blockDim.x + threadIdx.x; s < n * k; s += (u64)gridDim.x * blockDim.x) {
@@ -179,16 +170,8 @@ __global__ void k_um_cols(const u64 *__restrict__ keys, u64 nnz, u32 *__restrict
     for (u64 e = (u64)blockIdx.x * blockDim.x + threadIdx.x; e < nnz; e += (u64)gridDim.x * blockDim.x) idx[e] = (u32)keys[e];
 }
 
-// A fuzzy graph on the device: symmetric CSR, f64 weights in (0, 1].
-struct UmGraph {
-    u64 n = 0, nnz = 0;
-    DevBuf<u64> ptr;     // [n + 1]
-    DevBuf<u32> idx;     // [nnz]
-    DevBuf<double> w;    // [nnz]
-};
-
 template <typename T>
-static int um_select(sb_ctx *ctx, const T *in, const char *flags, T *out, u64 count, u64 *d_num) {
+int um_select(sb_ctx *ctx, const T *in, const char *flags, T *out, u64 count, u64 *d_num) {
     size_t tb = 0;
     SB_CUDA(cub::DeviceSelect::Flagged(nullptr, tb, in, flags, out, d_num, count, ctx->stream));
     DevBuf<char> tmp;
@@ -197,9 +180,12 @@ static int um_select(sb_ctx *ctx, const T *in, const char *flags, T *out, u64 co
     count_launch(ctx, false);
     return SB_OK;
 }
+template int um_select<u32>(sb_ctx *, const u32 *, const char *, u32 *, u64, u64 *);
+template int um_select<u64>(sb_ctx *, const u64 *, const char *, u64 *, u64, u64 *);
+template int um_select<double>(sb_ctx *, const double *, const char *, double *, u64, u64 *);
 
 // keys (row << 32 | col, ascending) of nnz entries -> g.ptr, g.idx
-static int um_rows_from_keys(sb_ctx *ctx, const u64 *keys, UmGraph &g) {
+int um_rows_from_keys(sb_ctx *ctx, const u64 *keys, UmGraph &g) {
     SB_TRY(g.ptr.alloc(g.n + 1));
     SB_TRY(g.idx.alloc(g.nnz));
     k_um_rows<<<um_grid(ctx, g.n + 1, 256), 256, 0, ctx->stream>>>(keys, g.nnz, g.n, g.ptr.p);
@@ -742,60 +728,70 @@ __global__ void k_um_check(const u64 *__restrict__ fk, const u64 *__restrict__ f
     }
 }
 
+int um_csr_host_check(u64 n, const u64 *indptr, const u32 *indices, const double *weights, const char *fn) {
+    if (n >= 0xFFFFFFFFull) return sb_fail(SB_ERR_UNSUPPORTED, "%s: more than 2^32 - 2 vertices", fn);
+    if (indptr[0] != 0) return sb_fail(SB_ERR_INVALID_ARG, "%s: indptr must start at 0", fn);
+    for (u64 i = 0; i < n; i++)
+        if (indptr[i + 1] < indptr[i]) return sb_fail(SB_ERR_INVALID_ARG, "%s: indptr decreases at row %llu", fn, (unsigned long long)i);
+    if (indptr[n] && (!indices || !weights)) return sb_fail(SB_ERR_INVALID_ARG, "%s: NULL argument", fn);
+    return SB_OK;
+}
+
+int um_csr_upload(sb_ctx *ctx, u64 n, const u64 *indptr, const u32 *indices, const double *weights, UmGraph &g, const char *fn,
+                  const char *trace) {
+    const u64 nnz = indptr[n];
+    g.n = n;
+    g.nnz = nnz;
+    SB_TRY(g.ptr.alloc(n + 1));
+    SB_CUDA(cudaMemcpyAsync(g.ptr.p, indptr, (n + 1) * sizeof(u64), cudaMemcpyHostToDevice, ctx->stream));
+    if (!nnz) return SB_OK;
+    // validation: the row-sorted pairs must equal the sorted transposed pairs, weights included, with no repeated pair
+    TraceScope tr(ctx, trace);
+    DevBuf<u32> di;
+    DevBuf<double> dw;
+    DevBuf<u64> fk, fv, tk, tv;
+    DevBuf<int> err;
+    SB_TRY(di.alloc(nnz));
+    SB_TRY(dw.alloc(nnz));
+    SB_TRY(fk.alloc(nnz));
+    SB_TRY(fv.alloc(nnz));
+    SB_TRY(tk.alloc(nnz));
+    SB_TRY(tv.alloc(nnz));
+    SB_TRY(err.alloc(1));
+    SB_CUDA(cudaMemcpyAsync(di.p, indices, nnz * sizeof(u32), cudaMemcpyHostToDevice, ctx->stream));
+    SB_CUDA(cudaMemcpyAsync(dw.p, weights, nnz * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+    SB_CUDA(cudaMemsetAsync(err.p, 0, sizeof(int), ctx->stream));
+    k_um_pairs<<<um_grid(ctx, nnz, 256), 256, 0, ctx->stream>>>(g.ptr.p, di.p, dw.p, n, nnz, fk.p, fv.p, tk.p, tv.p, err.p);
+    count_launch(ctx);
+    SB_TRY(sort_pairs(ctx, fk, fv, nnz));
+    SB_TRY(sort_pairs(ctx, tk, tv, nnz));
+    k_um_check<<<um_grid(ctx, nnz, 256), 256, 0, ctx->stream>>>(fk.p, fv.p, tk.p, tv.p, nnz, err.p);
+    count_launch(ctx);
+    SB_CUDA(cudaGetLastError());
+    int herr = 0;
+    SB_CUDA(cudaMemcpyAsync(&herr, err.p, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
+    SB_CUDA(cudaStreamSynchronize(ctx->stream));
+    if (herr & 1) return sb_fail(SB_ERR_INVALID_ARG, "%s: a column index >= n", fn);
+    if (herr & 8) return sb_fail(SB_ERR_INVALID_ARG, "%s: a weight outside (0, 1]", fn);
+    if (herr & 4) return sb_fail(SB_ERR_INVALID_ARG, "%s: a duplicate entry", fn);
+    if (herr & 2) return sb_fail(SB_ERR_INVALID_ARG, "%s: the CSR is not symmetric (pairs or weights)", fn);
+    // the graph: columns ascending
+    SB_TRY(um_rows_from_keys(ctx, fk.p, g));
+    SB_TRY(g.w.alloc(nnz));
+    SB_CUDA(cudaMemcpyAsync(g.w.p, fv.p, nnz * sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream));
+    return SB_OK;
+}
+
 extern "C" int sb_umap_layout(sb_ctx *ctx, uint64_t n, const uint64_t *indptr, const uint32_t *indices, const double *weights, const double *init,
                               const sb_umap_opts *opts, double *out, sb_umap_info *info) {
     if (!ctx || !indptr || !info || (n && !out)) return sb_fail(SB_ERR_INVALID_ARG, "sb_umap_layout: NULL argument");
     UmOpts o;
     SB_TRY(um_opts(opts, o, "sb_umap_layout"));
-    if (n >= 0xFFFFFFFFull) return sb_fail(SB_ERR_UNSUPPORTED, "sb_umap_layout: more than 2^32 - 2 vertices");
-    if (indptr[0] != 0) return sb_fail(SB_ERR_INVALID_ARG, "sb_umap_layout: indptr must start at 0");
-    for (u64 i = 0; i < n; i++)
-        if (indptr[i + 1] < indptr[i]) return sb_fail(SB_ERR_INVALID_ARG, "sb_umap_layout: indptr decreases at row %llu", (unsigned long long)i);
-    const u64 nnz = indptr[n];
-    if (nnz && (!indices || !weights)) return sb_fail(SB_ERR_INVALID_ARG, "sb_umap_layout: NULL argument");
+    SB_TRY(um_csr_host_check(n, indptr, indices, weights, "sb_umap_layout"));
     if (o.init != SB_UMAP_INIT_RANDOM) SB_TRY(um_user_init(init, n, o.nc, "sb_umap_layout"));
     SB_ENTER(ctx);
     UmGraph g;
-    g.n = n;
-    g.nnz = nnz;
-    SB_TRY(g.ptr.alloc(n + 1));
-    SB_CUDA(cudaMemcpyAsync(g.ptr.p, indptr, (n + 1) * sizeof(u64), cudaMemcpyHostToDevice, ctx->stream));
-    if (nnz) {
-        // validation: the row-sorted pairs must equal the sorted transposed pairs, weights included, with no repeated pair
-        TraceScope tr(ctx, "umap: csr validation");
-        DevBuf<u32> di;
-        DevBuf<double> dw;
-        DevBuf<u64> fk, fv, tk, tv;
-        DevBuf<int> err;
-        SB_TRY(di.alloc(nnz));
-        SB_TRY(dw.alloc(nnz));
-        SB_TRY(fk.alloc(nnz));
-        SB_TRY(fv.alloc(nnz));
-        SB_TRY(tk.alloc(nnz));
-        SB_TRY(tv.alloc(nnz));
-        SB_TRY(err.alloc(1));
-        SB_CUDA(cudaMemcpyAsync(di.p, indices, nnz * sizeof(u32), cudaMemcpyHostToDevice, ctx->stream));
-        SB_CUDA(cudaMemcpyAsync(dw.p, weights, nnz * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
-        SB_CUDA(cudaMemsetAsync(err.p, 0, sizeof(int), ctx->stream));
-        k_um_pairs<<<um_grid(ctx, nnz, 256), 256, 0, ctx->stream>>>(g.ptr.p, di.p, dw.p, n, nnz, fk.p, fv.p, tk.p, tv.p, err.p);
-        count_launch(ctx);
-        SB_TRY(sort_pairs(ctx, fk, fv, nnz));
-        SB_TRY(sort_pairs(ctx, tk, tv, nnz));
-        k_um_check<<<um_grid(ctx, nnz, 256), 256, 0, ctx->stream>>>(fk.p, fv.p, tk.p, tv.p, nnz, err.p);
-        count_launch(ctx);
-        SB_CUDA(cudaGetLastError());
-        int herr = 0;
-        SB_CUDA(cudaMemcpyAsync(&herr, err.p, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
-        SB_CUDA(cudaStreamSynchronize(ctx->stream));
-        if (herr & 1) return sb_fail(SB_ERR_INVALID_ARG, "sb_umap_layout: a column index >= n");
-        if (herr & 8) return sb_fail(SB_ERR_INVALID_ARG, "sb_umap_layout: a weight outside (0, 1]");
-        if (herr & 4) return sb_fail(SB_ERR_INVALID_ARG, "sb_umap_layout: a duplicate entry");
-        if (herr & 2) return sb_fail(SB_ERR_INVALID_ARG, "sb_umap_layout: the CSR is not symmetric (pairs or weights)");
-        // the graph: columns ascending
-        SB_TRY(um_rows_from_keys(ctx, fk.p, g));
-        SB_TRY(g.w.alloc(nnz));
-        SB_CUDA(cudaMemcpyAsync(g.w.p, fv.p, nnz * sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream));
-    }
+    SB_TRY(um_csr_upload(ctx, n, indptr, indices, weights, g, "sb_umap_layout", "umap: csr validation"));
     DevBuf<double> dA;
     SB_TRY(dA.alloc(n * o.nc));
     if (n && o.init != SB_UMAP_INIT_RANDOM) SB_CUDA(cudaMemcpyAsync(dA.p, init, n * o.nc * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
