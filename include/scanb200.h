@@ -242,6 +242,10 @@ SB_API int sb_normalize_fixed_point(sb_mat *mat, int log_base, uint32_t base, ui
 SB_API int sb_nmat_params(const sb_nmat *a, double *col_scale, double *row_scale, double *u, double *v);
 /* LowRankOffset::to_dense (low_rank_offset.rs:55-57): m x n_local row-major; test/debug sizes only */
 SB_API int sb_nmat_to_dense(sb_nmat *a, double *out);
+/* Operand contract of both products (and of the PCA's internal passes): a finite operand entry of any magnitude is used as given.
+ * A NaN or +-inf in operand column j makes out column j non-finite wherever the exact product is; on a log-normalized matrix with a
+ * dense (bit-plane) half it makes the whole of out column j NaN -- for sb_nmat_dot every highly expressed gene's row, for
+ * sb_nmat_rdot every cell -- also where the exact product would be finite (that half scales each operand column as a whole). */
 /* LowRankOffset . Array2 (low_rank_offset.rs:68-81): out[m x w] = A . x[n_local x w], all-reduced over ranks */
 SB_API int sb_nmat_dot(sb_nmat *a, const double *x, uint32_t w, double *out);
 /* Array2 . LowRankOffset (low_rank_offset.rs:83-96): out[w x n_local] = b[w x m] . A */

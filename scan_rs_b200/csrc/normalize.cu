@@ -113,7 +113,8 @@ __global__ void k_finish_moments(const double *__restrict__ S1, const double *__
     }
 }
 
-static int moments(sb_nmat *a, double *S /* 2m */) {
+// S[0, m) = S1, S[m, 2m) = S2, all-reduced over ranks (also reached by tests/cuda/spmm_harness.cu)
+int nmat_moments(sb_nmat *a, double *S /* 2m */) {
     sb_mat *mt = a->mat;
     sb_ctx *ctx = mt->ctx;
     SB_CUDA(cudaMemsetAsync(S, 0, 2 * (size_t)mt->m * sizeof(double), ctx->stream));
@@ -159,7 +160,7 @@ extern "C" int sb_nmat_frobenius_sq(sb_nmat *a, double *out) {
     DevBuf<double> S, acc;
     SB_TRY(S.alloc(2 * (size_t)mt->m + 1));
     SB_TRY(acc.alloc(1));
-    SB_TRY(moments(a, S.p));  // all-reduced over ranks
+    SB_TRY(nmat_moments(a, S.p));  // all-reduced over ranks
     SB_CUDA(cudaMemsetAsync(acc.p, 0, sizeof(double), ctx->stream));
     if (mt->m) {
         k_frob_from_moments<<<cdiv(mt->m, 256), 256, 0, ctx->stream>>>(S.p, S.p + mt->m, a->has_row_scale ? a->row_scale.p : nullptr,
@@ -216,7 +217,7 @@ extern "C" int sb_log_normalize(sb_mat *mat, int has_target, double target, int 
     if (center_scale) {
         DevBuf<double> S, sd;
         SB_TRY(S.alloc(2 * (size_t)mat->m));
-        SB_TRY(moments(a.get(), S.p));
+        SB_TRY(nmat_moments(a.get(), S.p));
         if (center_scale == 2) {
             SB_TRY(sd.alloc(mat->m));
             SB_CUDA(cudaMemcpyAsync(sd.p, sd_override, (size_t)mat->m * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));

@@ -356,7 +356,8 @@ int planes_split_launch(sb_mat *mt, u64 c0, u64 nc, const u64 *new_ptr, u32 *cou
 }
 
 // ---------------------------------------------------------------- digit helpers
-__device__ __forceinline__ double finite_or_zero(double x) { return (x == x && fabs(x) < 1.0e300) ? x : 0.0; }
+// Operand entries are split as they are: a finite entry of any magnitude is exact up to the 54-bit quantum of its column, and a NaN or
+// +-inf makes the column's scale NaN, so that the plane part of that whole output column is NaN (include/scanb200.h, sb_nmat_dot).
 
 // q (|q| <= 2^54) -> 7 balanced base-256 digits in [-128, 127]
 __device__ __forceinline__ void digits7(long long q, signed char (&d)[PL_DIG]) {
@@ -368,17 +369,26 @@ __device__ __forceinline__ void digits7(long long q, signed char (&d)[PL_DIG]) {
     }
 }
 
-__device__ __forceinline__ void atomic_max_abs(unsigned long long *slot, double v) {
-    atomicMax(slot, (unsigned long long)__double_as_longlong(fabs(v)));  // non-negative doubles order like their bits
-}
+// |v| as bits: non-negative doubles order like their bits, +inf above every finite value and NaN above +inf
+__device__ __forceinline__ unsigned long long abs_bits(double v) { return (unsigned long long)__double_as_longlong(v) & 0x7FFFFFFFFFFFFFFFull; }
 
-// scale2[c] = 2^(e_c - PL_FIX) with |x| < 2^e_c for every entry of column c; ex[c] = PL_FIX - e_c
+__device__ __forceinline__ void atomic_max_abs(unsigned long long *slot, double v) { atomicMax(slot, abs_bits(v)); }
+
+// scale2[c] = 2^(e_c - PL_FIX) with |x| < 2^e_c for every entry of column c; ex[c] = PL_FIX - e_c.  e_c >= PL_FIX - 1074 keeps scale2 at
+// least the smallest subnormal (a column below 2^-1020 is quantised to the spacing of doubles at zero).  A non-finite column maximum
+// gives scale2 = NaN.
 __global__ void k_pl_scales(const unsigned long long *__restrict__ colmax_bits, double *__restrict__ scale2, int *__restrict__ ex) {
     const u32 c = threadIdx.x;
     if (c >= PL_COLS) return;
     const double mx = __longlong_as_double((long long)colmax_bits[c]);
+    if (!isfinite(mx)) {
+        scale2[c] = __longlong_as_double(0x7FF8000000000000ll);
+        ex[c] = 0;
+        return;
+    }
     int e = 0;
     if (mx > 0.0) frexp(mx, &e);
+    e = max(e, PL_FIX - 1074);
     scale2[c] = ldexp(1.0, e - PL_FIX);
     ex[c] = PL_FIX - e;
 }
@@ -393,7 +403,7 @@ __global__ void k_pl_colmax_t(const double *__restrict__ Y, u32 ldy, const u32 *
     const u32 g = hot_idx[r];
     double v = Y[(size_t)g * ldy + col0 + c];
     if (rs) v *= rs[g];
-    atomic_max_abs(&colmax_bits[c], finite_or_zero(v));
+    atomic_max_abs(&colmax_bits[c], v);
 }
 
 // Bd[range][k / 16][n / 8][n % 8][k % 16], k = rank % 1024, n = 7 c + s (digit s of column c); with `split` the second ten columns
@@ -406,7 +416,7 @@ __global__ void k_pl_digits_t(const double *__restrict__ Y, u32 ldy, const u32 *
     const u32 g = hot_idx[r];
     double v = c < wt ? Y[(size_t)g * ldy + col0 + c] : 0.0;
     if (rs) v *= rs[g];
-    const long long q = __double2ll_rn(ldexp(finite_or_zero(v), ex[c]));
+    const long long q = __double2ll_rn(ldexp(v, ex[c]));
     signed char d[PL_DIG];
     digits7(q, d);
     const u32 range = r / PT_RANGE, k = r - range * PT_RANGE;
@@ -907,11 +917,11 @@ __global__ void k_pl_reduce_t(const double *__restrict__ part, u32 n_units, u64 
             s.x += v.x;
             s.y += v.y;
         }
-        if (t1) {
+        if (t1) {  // a cell without sparse entries adds nothing: a zero-total cell has L_c(1) = inf, and inf * 0 would be NaN
             const double2 v = *reinterpret_cast<const double2 *>(t1 + c * PL_COLS + j);
             const double f = l1[c];
-            s.x = fma(f, v.x, s.x);
-            s.y = fma(f, v.y, s.y);
+            if (v.x != 0.0) s.x = fma(f, v.x, s.x);
+            if (v.y != 0.0) s.y = fma(f, v.y, s.y);
         }
         double *o = out + c * (size_t)ldo + col0 + j;
         o[0] += s.x;
@@ -923,25 +933,25 @@ __global__ void k_pl_reduce_t(const double *__restrict__ part, u32 n_units, u64 
 // mode 0: value_j = L_c(k) * X[c, col0 + j]; mode 1 (moments): value_0 = L_c(k), value_1 = L_c(k)^2
 __global__ void k_pl_colmax_n(const double *__restrict__ X, u32 ldx, u64 n, const double *__restrict__ lk, u32 Ltop, u32 col0, u32 wt,
                               int mode, unsigned long long *__restrict__ colmax_bits) {
-    double mx[PL_COLS];
+    unsigned long long mx[PL_COLS];  // abs_bits: the maximum keeps a NaN (fmax would drop it)
 #pragma unroll
-    for (u32 j = 0; j < PL_COLS; j++) mx[j] = 0.0;
+    for (u32 j = 0; j < PL_COLS; j++) mx[j] = 0ull;
     for (u64 c = (u64)blockIdx.x * blockDim.x + threadIdx.x; c < n; c += (u64)gridDim.x * blockDim.x) {
         const double l = lk[c * PL_MAX_LEVELS + Ltop - 1];  // L_c(k) grows with k: the top level bounds all
         if (mode == 1) {
-            mx[0] = fmax(mx[0], fabs(l));
-            mx[1] = fmax(mx[1], l * l);
+            mx[0] = max(mx[0], abs_bits(l));
+            mx[1] = max(mx[1], abs_bits(l * l));
         } else {
 #pragma unroll
             for (u32 j = 0; j < PL_COLS; j++)
-                if (j < wt) mx[j] = fmax(mx[j], fabs(finite_or_zero(l * X[c * (size_t)ldx + col0 + j])));
+                if (j < wt) mx[j] = max(mx[j], abs_bits(l * X[c * (size_t)ldx + col0 + j]));
         }
     }
 #pragma unroll
     for (u32 j = 0; j < PL_COLS; j++) {
-        double v = mx[j];
-        for (int o = 16; o > 0; o >>= 1) v = fmax(v, __shfl_xor_sync(0xffffffffu, v, o));
-        if ((threadIdx.x & 31) == 0 && v > 0.0) atomic_max_abs(&colmax_bits[j], v);
+        unsigned long long v = mx[j];
+        for (int o = 16; o > 0; o >>= 1) v = max(v, __shfl_xor_sync(0xffffffffu, v, o));
+        if ((threadIdx.x & 31) == 0 && v != 0ull) atomicMax(&colmax_bits[j], v);
     }
 }
 
@@ -961,7 +971,7 @@ __global__ void k_pl_digits_n(const double *__restrict__ X, u32 ldx, u64 n, u64 
         for (u32 j = 0; j < PL_COLS; j++) {
             double v = 0.0;
             if (mode == 1) v = j == 0 ? l : (j == 1 ? l * l : 0.0);
-            else if (j < wt) v = finite_or_zero(l * X[c * (size_t)ldx + col0 + j]);
+            else if (j < wt) v = l * X[c * (size_t)ldx + col0 + j];
             const long long q = __double2ll_rn(ldexp(v, ex[j]));
             signed char d[PL_DIG];
             digits7(q, d);
@@ -1047,8 +1057,10 @@ k_planes_n(PlDev pl, const PlUnitN *__restrict__ units, const PlItem *__restrict
                 const u32 g = hot_idx[un.g0 + mtile * 128 + row];
                 double *o = out + (size_t)g * row_stride;
 #pragma unroll
-                for (u32 j = 0; j < PL_COLS; j++)
-                    if (j < wt && val[j] != 0.0) atomicAdd(o + (size_t)(col0 + j) * col_stride, val[j] * sh->scale2[j]);
+                for (u32 j = 0; j < PL_COLS; j++) {
+                    const double r = val[j] * sh->scale2[j];  // NaN in every row of a column whose scale is NaN, zero or not
+                    if (j < wt && r != 0.0) atomicAdd(o + (size_t)(col0 + j) * col_stride, r);
+                }
             }
         } else if (warp == PL_EPI_WARPS) {
             // ===== MMA issue: converged warp, uniform values, an elected lane only around the tensor-core instructions (see k_planes_t);
