@@ -428,6 +428,70 @@ SB_API int sb_louvain(sb_ctx *ctx, uint64_t n, const uint64_t *indptr, const uin
 SB_API int sb_cluster_knn(sb_ctx *ctx, const uint32_t *nbr, uint64_t n_local, uint32_t k, const sb_louvain_opts *opts, uint32_t *labels,
                    sb_louvain_info *info);
 
+/* Deterministic Leiden (Traag, Waltman & van Eck 2019): Louvain's synchronous moving plus a refinement that keeps every community
+ * connected, modularity or CPM quality, and passes until the partition is stable.  Restated literally by oracle/leiden.py.
+ *
+ * Weights: W_i and the scaled resolution g' are, for SB_QUALITY_MODULARITY, W_i = K_i and g' = resolution / (double)2m (the gain
+ * below is then sb_louvain's, and Q is sb_louvain's formula); for SB_QUALITY_CPM, W_i = the number of original nodes inside node i
+ * (1 at the first level) and g' = resolution, in the units of the edge weights.  The SNN weights are the Jaccard index x 2^24
+ * (SB_SNN_WEIGHT_SCALE), so a Jaccard-scale CPM resolution is multiplied by SB_SNN_WEIGHT_SCALE.  CPM quality =
+ * ((double)sum_I - g' sum_W2) / (double)2m, sum_W2 = sum of W_c^2 exact in 128 bits, as (double)hi 2^64 + (double)lo.  Every sum
+ * is an integer; every gain a double evaluated in the stated order without contraction.
+ *
+ * Local moving: sb_louvain's iterations with K replaced by W and g2m by g', from a given partition (community ids in [0, 2n)):
+ *   gain(c) = ((double)e_ic - (double)e_ia) - (g' (double)W_i) ((double)W_c - (double)(W_a - W_i)),
+ * best gain > 0, ties to the smallest c, c > a in even iterations and c < a in odd ones, kept only if the quality strictly rises,
+ * two failed iterations in a row end it (or max_iterations).  One more candidate in even iterations only: the empty community
+ * n + i, if a has other members and n + i has none at the start of the iteration; its gain is the formula with e_ic = 0, W_c = 0.
+ * The moved partition P is then compacted: each community takes the id of its smallest member.  If every community of P is a
+ * single node, the pass ends.
+ *
+ * Refinement, inside each community S of P, from singletons R: v is eligible if e(v, S - v) >= (g' (double)W_v) (double)(W_S - W_v)
+ * (e: (double) of the integer weight; this order, no contraction), r is well connected if e(r, S - r) >= (g' (double)W_r)
+ * (double)(W_S - W_r) at the start of the round.  Each round, every eligible v that is still a singleton looks at the refined
+ * communities r of its neighbours in S (a refined community's id is one of its members, never changing); its gain
+ * ((double)e_vr - 0) - (g' (double)W_v) ((double)W_r - 0) must be >= 0 with r well connected, r > v in even rounds and r < v in odd
+ * ones; the best gain wins, ties to the smallest r.  A singleton that some node picks as its target does not move in that round.
+ * Refinement ends after two rounds in a row without a move, or max_iterations rounds.  Every node that joins r is adjacent to a
+ * member of r that stays, so every refined community is connected.
+ *
+ * Aggregation: on R if it has fewer communities than nodes, else on P (aggregate nodes numbered in ascending community id, weights
+ * summed per pair as sb_louvain does, W summed); the next level starts from P: each P community takes the smallest aggregate id
+ * among its members.  A pass ends as above or after max_levels levels; its result is the last partition mapped to the original
+ * nodes.  Passes: the first starts from singletons, each later one from the previous pass's result; they stop when a pass returns
+ * its start partition (stable = 1) or after max_passes passes (0: until stable, at most SB_LEIDEN_MAX_PASSES).  Labels: by size,
+ * as sb_louvain's.  A graph of total weight 0 leaves every node its own cluster (one pass, one level, 0 iterations, quality 0).
+ *
+ * sb_leiden: a host CSR, validated as sb_louvain's (n < 2^31 - 1).  sb_cluster_knn_leiden: sb_snn_graph + sb_leiden with the graph
+ * kept on the device; on a cell-sharded context as sb_cluster_knn (rows gathered in global cell order, labels equal world 1). */
+#define SB_LEIDEN_MAX_LEVELS 32
+#define SB_LEIDEN_MAX_PASSES 32
+#define SB_QUALITY_MODULARITY 0
+#define SB_QUALITY_CPM 1
+#define SB_SNN_WEIGHT_SCALE 16777216.0  /* 2^24: one unit of Jaccard index in sb_snn_graph's weights */
+typedef struct sb_leiden_opts {
+    double resolution;        /* gamma > 0 (default 1.0); CPM: in the units of the edge weights */
+    uint32_t quality;         /* SB_QUALITY_MODULARITY (default) or SB_QUALITY_CPM */
+    uint32_t max_levels;      /* 1..SB_LEIDEN_MAX_LEVELS (default 32) */
+    uint32_t max_iterations;  /* local-moving iterations and refinement rounds per level, >= 1 (default 100) */
+    uint32_t max_passes;      /* 0 (default): until stable, at most SB_LEIDEN_MAX_PASSES; else 1..SB_LEIDEN_MAX_PASSES */
+} sb_leiden_opts;             /* NULL: the defaults */
+typedef struct sb_leiden_info {
+    uint32_t n_clusters;
+    uint32_t n_levels;        /* levels of the last pass */
+    double quality;           /* of the final partition */
+    uint32_t n_passes;
+    uint32_t stable;          /* 1: the last pass returned its start partition */
+    uint64_t level_nodes[SB_LEIDEN_MAX_LEVELS];        /* per level of the last pass */
+    uint32_t level_iterations[SB_LEIDEN_MAX_LEVELS];
+    uint64_t level_refined[SB_LEIDEN_MAX_LEVELS];      /* communities after refinement (the nodes, where the pass ended) */
+    double level_quality[SB_LEIDEN_MAX_LEVELS];        /* after local moving */
+} sb_leiden_info;
+SB_API int sb_leiden(sb_ctx *ctx, uint64_t n, const uint64_t *indptr, const uint32_t *indices, const uint64_t *weights,
+              const sb_leiden_opts *opts, uint32_t *labels, sb_leiden_info *info);
+SB_API int sb_cluster_knn_leiden(sb_ctx *ctx, const uint32_t *nbr, uint64_t n_local, uint32_t k, const sb_leiden_opts *opts,
+                          uint32_t *labels, sb_leiden_info *info);
+
 /* ---------------------------------------------------------------- merging of over-split clusters (Cell Ranger's MERGE_CLUSTERS)
  * scan-rs's linkage.rs and merge_clusters.rs, restated (neither is pinned here); oracle/merge_clusters.py restates the rule literally.
  *

@@ -592,6 +592,57 @@ inline Result cluster_knn(const Context &ctx, const std::vector<uint32_t> &nbr, 
     return detail::result(std::move(labels), info);
 }
 
+// Leiden: connected clusters, modularity or CPM (CPM's resolution in edge-weight units: SNN weights are Jaccard x SB_SNN_WEIGHT_SCALE)
+struct LeidenOptions {
+    double resolution = 1.0;
+    uint32_t quality = SB_QUALITY_MODULARITY;
+    uint32_t max_levels = SB_LEIDEN_MAX_LEVELS;
+    uint32_t max_iterations = 100;
+    uint32_t max_passes = 0;  // 0: until stable
+};
+struct LeidenLevel {
+    uint64_t nodes;
+    uint32_t iterations;
+    uint64_t refined;
+    double quality;
+};
+struct LeidenResult {
+    std::vector<uint32_t> labels;  // 0..n_clusters-1, by size, descending
+    uint32_t n_clusters = 0;
+    double quality = 0.0;
+    uint32_t n_passes = 0;
+    bool stable = true;
+    std::vector<LeidenLevel> levels;  // of the last pass
+};
+namespace detail {
+inline LeidenResult leiden_result(std::vector<uint32_t> labels, const sb_leiden_info &info) {
+    LeidenResult r{std::move(labels), info.n_clusters, info.quality, info.n_passes, info.stable != 0, {}};
+    for (uint32_t l = 0; l < info.n_levels; l++)
+        r.levels.push_back(LeidenLevel{info.level_nodes[l], info.level_iterations[l], info.level_refined[l], info.level_quality[l]});
+    return r;
+}
+inline sb_leiden_opts leiden_opts(const LeidenOptions &o) { return sb_leiden_opts{o.resolution, o.quality, o.max_levels, o.max_iterations, o.max_passes}; }
+}  // namespace detail
+inline LeidenResult leiden(const Context &ctx, const Graph &g, const LeidenOptions &o = LeidenOptions()) {
+    if (g.indptr.empty()) throw Error(SB_ERR_INVALID_ARG, "indptr must hold n + 1 entries");
+    const uint64_t n = g.indptr.size() - 1;
+    std::vector<uint32_t> labels(n);
+    sb_leiden_info info;
+    const sb_leiden_opts c = detail::leiden_opts(o);
+    check(sb_leiden(ctx.raw(), n, g.indptr.data(), g.indices.data(), g.weights.data(), &c, labels.data(), &info));
+    return detail::leiden_result(std::move(labels), info);
+}
+// on a sharded context: this rank's rows (global indices) -> this rank's labels
+inline LeidenResult cluster_knn_leiden(const Context &ctx, const std::vector<uint32_t> &nbr, uint32_t k, const LeidenOptions &o = LeidenOptions()) {
+    if (k == 0 || nbr.size() % k) throw Error(SB_ERR_INVALID_ARG, "nbr must hold n x k entries");
+    const uint64_t n = nbr.size() / k;
+    std::vector<uint32_t> labels(n);
+    sb_leiden_info info;
+    const sb_leiden_opts c = detail::leiden_opts(o);
+    check(sb_cluster_knn_leiden(ctx.raw(), nbr.data(), n, k, &c, labels.data(), &info));
+    return detail::leiden_result(std::move(labels), info);
+}
+
 // complete linkage (NN-chain) of points [n x dim] on the host: Z [(n - 1) x 4] in scipy's layout
 inline std::vector<double> linkage_complete(const std::vector<double> &points, uint32_t dim) {
     if (dim == 0 || points.size() % dim) throw Error(SB_ERR_INVALID_ARG, "points must hold n x dim entries");

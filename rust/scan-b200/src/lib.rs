@@ -498,6 +498,73 @@ pub fn cluster_knn(ctx: &Context, nbr: &Array2<u32>, opts: &LouvainOptions) -> R
     Ok(clustering(labels, &info))
 }
 
+/// Leiden options: resolution (gamma) > 0; quality `ffi::SB_QUALITY_MODULARITY` or `ffi::SB_QUALITY_CPM` (CPM's resolution is in
+/// edge-weight units: the SNN weights are Jaccard x `ffi::SB_SNN_WEIGHT_SCALE`); max_levels 1..32; max_iterations >= 1;
+/// max_passes 0 = until stable
+#[derive(Clone, Copy, Debug)]
+pub struct LeidenOptions {
+    pub resolution: f64,
+    pub quality: u32,
+    pub max_levels: u32,
+    pub max_iterations: u32,
+    pub max_passes: u32,
+}
+impl Default for LeidenOptions {
+    fn default() -> Self {
+        LeidenOptions { resolution: 1.0, quality: ffi::SB_QUALITY_MODULARITY, max_levels: ffi::SB_LEIDEN_MAX_LEVELS as u32, max_iterations: 100, max_passes: 0 }
+    }
+}
+
+/// Leiden labels (0..n_clusters-1, by size, descending), the final quality, passes, whether the last was stable, and per level of
+/// the last pass (nodes, iterations, refined communities, quality)
+#[derive(Clone, Debug)]
+pub struct LeidenClustering {
+    pub labels: Vec<u32>,
+    pub n_clusters: u32,
+    pub quality: f64,
+    pub n_passes: u32,
+    pub stable: bool,
+    pub levels: Vec<(u64, u32, u64, f64)>,
+}
+
+fn leiden_clustering(labels: Vec<u32>, info: &ffi::sb_leiden_info) -> LeidenClustering {
+    let levels = (0..info.n_levels as usize)
+        .map(|l| (info.level_nodes[l], info.level_iterations[l], info.level_refined[l], info.level_quality[l]))
+        .collect();
+    LeidenClustering { labels, n_clusters: info.n_clusters, quality: info.quality, n_passes: info.n_passes, stable: info.stable != 0, levels }
+}
+fn leiden_opts(o: &LeidenOptions) -> ffi::sb_leiden_opts {
+    ffi::sb_leiden_opts { resolution: o.resolution, quality: o.quality, max_levels: o.max_levels, max_iterations: o.max_iterations, max_passes: o.max_passes }
+}
+fn empty_leiden_info() -> ffi::sb_leiden_info {
+    ffi::sb_leiden_info { n_clusters: 0, n_levels: 0, quality: 0.0, n_passes: 0, stable: 0, level_nodes: [0; ffi::SB_LEIDEN_MAX_LEVELS],
+                          level_iterations: [0; ffi::SB_LEIDEN_MAX_LEVELS], level_refined: [0; ffi::SB_LEIDEN_MAX_LEVELS],
+                          level_quality: [0.0; ffi::SB_LEIDEN_MAX_LEVELS] }
+}
+
+/// Deterministic Leiden on a symmetric CSR with integer weights: every cluster connected inside itself
+pub fn leiden(ctx: &Context, g: &SnnGraph, opts: &LeidenOptions) -> Result<LeidenClustering, Error> {
+    assert!(!g.indptr.is_empty(), "indptr must hold n + 1 entries");
+    let n = g.indptr.len() - 1;
+    let mut labels = vec![0u32; n];
+    let mut info = empty_leiden_info();
+    let o = leiden_opts(opts);
+    check(unsafe { ffi::sb_leiden(ctx.h, n as u64, g.indptr.as_ptr(), g.indices.as_ptr(), g.weights.as_ptr(), &o, labels.as_mut_ptr(), &mut info) })?;
+    Ok(leiden_clustering(labels, &info))
+}
+
+/// kNN lists -> SNN graph -> Leiden with the graph kept on the device; on a sharded context every rank passes its own rows
+/// (global indices) and receives its own cells' labels
+pub fn cluster_knn_leiden(ctx: &Context, nbr: &Array2<u32>, opts: &LeidenOptions) -> Result<LeidenClustering, Error> {
+    let nbr = nbr.as_standard_layout();
+    let (n, k) = nbr.dim();
+    let mut labels = vec![0u32; n];
+    let mut info = empty_leiden_info();
+    let o = leiden_opts(opts);
+    check(unsafe { ffi::sb_cluster_knn_leiden(ctx.h, nbr.as_ptr(), n as u64, k as u32, &o, labels.as_mut_ptr(), &mut info) })?;
+    Ok(leiden_clustering(labels, &info))
+}
+
 /// Complete linkage (NN-chain) of `points` (n x dim) on the host: Z ((n - 1) x 4) in scipy's layout
 pub fn linkage_complete(points: &Array2<f64>) -> Result<Array2<f64>, Error> {
     let pts = points.as_standard_layout();

@@ -7,7 +7,8 @@ The package mirrors the reference's module layout for this path only:
   snoop          NoOpSnoop, AtomicSnoop
   mtx            load_mtx (gz MatrixMarket -> device matrix)
   nn             knn, find_nn on the PCA scores
-  cluster        SNN graph of the kNN lists and deterministic Louvain (snn_graph, louvain, cluster_knn); merging of over-split
+  cluster        SNN graph of the kNN lists, deterministic Louvain (snn_graph, louvain, cluster_knn) and Leiden (leiden,
+                 cluster_knn_leiden: connected clusters, modularity or CPM); merging of over-split
                  clusters by differential expression (linkage_complete, merge_clusters)
   embedding      UMAP of the scores and kNN lists: fuzzy graph and deterministic layout (umap_graph, umap_layout, umap); t-SNE:
                  perplexity-calibrated affinities and a deterministic Barnes-Hut layout (tsne_affinities, tsne_layout, tsne)
@@ -28,7 +29,8 @@ from .nn import find_nn, knn  # noqa: F401
 from .multi import MultiContext  # noqa: F401
 from .diff_exp import (DiffExpResult, SSeqParams, compute_sseq_params, sseq_differential_expression,  # noqa: F401
                        sseq_one_vs_rest, sseq_pairs)
-from .cluster import (ClusterResult, LouvainOptions, MergeOptions, MergeResult, cluster_knn, linkage_complete, louvain,  # noqa: F401
+from .cluster import (QUALITY_CPM, QUALITY_MODULARITY, SNN_WEIGHT_SCALE, ClusterResult, LeidenOptions, LeidenResult,  # noqa: F401
+                      LouvainOptions, MergeOptions, MergeResult, cluster_knn, cluster_knn_leiden, leiden, linkage_complete, louvain,
                       merge_clusters, snn_graph)
 from .embedding import (TsneOptions, TsneResult, UmapOptions, UmapResult, tsne, tsne_affinities, tsne_layout, umap, umap_graph,  # noqa: F401
                         umap_layout)

@@ -50,7 +50,7 @@ SYMBOLS = [
     "sb_timer_end", "sb_flush_l2", "sb_synth_generate", "sb_knn",
     "sb_irlba", "sb_irlba_start", "sb_mean_var_axis", "sb_mean_var_rows", "sb_sum_rows", "sb_sum_cols", "sb_sum_rows_dual", "sb_size_factors", "sb_upload_unsorted", "sb_filter_genes", "sb_multi_init", "sb_multi_size", "sb_multi_ctx", "sb_multi_run", "sb_multi_shutdown",
     "sb_sseq_compute_params", "sb_sseq_diff_exp", "sb_sseq_one_vs_rest", "sb_sseq_pairs",
-    "sb_snn_graph", "sb_louvain", "sb_cluster_knn", "sb_linkage_complete", "sb_merge_clusters",
+    "sb_snn_graph", "sb_louvain", "sb_cluster_knn", "sb_leiden", "sb_cluster_knn_leiden", "sb_linkage_complete", "sb_merge_clusters",
     "sb_umap_graph", "sb_umap_layout", "sb_umap", "sb_tsne_affinities", "sb_tsne_layout", "sb_tsne",
 ]
 

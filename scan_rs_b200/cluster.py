@@ -1,9 +1,10 @@
 """Graph clustering of the kNN lists on the device (csrc/cluster.cu; the rules are stated in include/scanb200.h): the
-shared-nearest-neighbour graph and deterministic Louvain, the step that turns neighbour lists into the labels sseq_one_vs_rest
+shared-nearest-neighbour graph and deterministic Louvain or Leiden, the step that turns neighbour lists into the labels sseq_one_vs_rest
 takes; and the merge of over-split clusters by differential expression (csrc/merge.cu, Cell Ranger's MERGE_CLUSTERS).
 
     nbr = knn(ctx, scores, 15)
     res = cluster_knn(ctx, nbr)                # res.labels: 0..n_clusters-1, by size, descending
+    res = cluster_knn_leiden(ctx, nbr)         # or Leiden: every cluster connected inside itself
     merged = merge_clusters(mat, scores, res.labels, params)  # join clusters no gene separates
     de = sseq_one_vs_rest(mat, merged.labels, params)
 
@@ -19,6 +20,10 @@ import numpy as np
 from . import _lib as L
 
 MAX_LEVELS = 32
+LEIDEN_MAX_LEVELS = 32
+LEIDEN_MAX_PASSES = 32
+QUALITY_MODULARITY, QUALITY_CPM = 0, 1
+SNN_WEIGHT_SCALE = float(1 << 24)  # the SNN weights: Jaccard index x 2^24
 LINKAGE_MAX_POINTS = 4096
 
 
@@ -64,6 +69,52 @@ def _rows(nbr) -> np.ndarray:
     return nbr
 
 
+class SbLeidenOpts(C.Structure):  # include/scanb200.h: sb_leiden_opts
+    _fields_ = [("resolution", C.c_double), ("quality", C.c_uint32), ("max_levels", C.c_uint32), ("max_iterations", C.c_uint32),
+                ("max_passes", C.c_uint32)]
+
+
+class SbLeidenInfo(C.Structure):  # include/scanb200.h: sb_leiden_info
+    _fields_ = [("n_clusters", C.c_uint32), ("n_levels", C.c_uint32), ("quality", C.c_double), ("n_passes", C.c_uint32),
+                ("stable", C.c_uint32), ("level_nodes", C.c_uint64 * LEIDEN_MAX_LEVELS),
+                ("level_iterations", C.c_uint32 * LEIDEN_MAX_LEVELS), ("level_refined", C.c_uint64 * LEIDEN_MAX_LEVELS),
+                ("level_quality", C.c_double * LEIDEN_MAX_LEVELS)]
+
+
+@dataclass
+class LeidenOptions:
+    """resolution: gamma.  quality: QUALITY_MODULARITY or QUALITY_CPM.  For CPM the resolution is in the units of the edge weights;
+    the SNN weights are the Jaccard index x 2^24, so a Jaccard-scale resolution is multiplied by SNN_WEIGHT_SCALE.
+    max_passes = 0: passes until the partition is stable (at most LEIDEN_MAX_PASSES)."""
+    resolution: float = 1.0
+    quality: int = QUALITY_MODULARITY
+    max_levels: int = LEIDEN_MAX_LEVELS
+    max_iterations: int = 100
+    max_passes: int = 0
+
+
+@dataclass
+class LeidenResult(ClusterResult):
+    """ClusterResult plus Leiden's passes.  modularity holds the final quality (CPM's when quality is CPM); levels are those of
+    the last pass as (nodes, iterations, Q), and refined the refined community count of each."""
+    quality: int = QUALITY_MODULARITY
+    n_passes: int = 0
+    stable: bool = True
+    refined: List[int] = field(default_factory=list)
+
+
+def _leiden_opts(o: LeidenOptions | None):
+    o = o or LeidenOptions()
+    return SbLeidenOpts(float(o.resolution), int(o.quality), int(o.max_levels), int(o.max_iterations), int(o.max_passes))
+
+
+def _leiden_result(labels, info: SbLeidenInfo, quality: int) -> LeidenResult:
+    r = range(info.n_levels)
+    lv = [(int(info.level_nodes[i]), int(info.level_iterations[i]), float(info.level_quality[i])) for i in r]
+    return LeidenResult(labels, int(info.n_clusters), float(info.quality), lv, int(quality), int(info.n_passes), bool(info.stable),
+                        [int(info.level_refined[i]) for i in r])
+
+
 def snn_graph(ctx, nbr):
     """kNN lists [n x k] -> symmetric CSR (indptr u64, indices u32, weights u64 = Jaccard index << 24)."""
     nbr = _rows(nbr)
@@ -98,6 +149,30 @@ def cluster_knn(ctx, nbr, options: LouvainOptions | None = None) -> ClusterResul
     o = _opts(options)
     L.check(L.lib().sb_cluster_knn(ctx._h, L.vp(nbr), C.c_uint64(n), C.c_uint32(k), C.byref(o), L.vp(labels), C.byref(info)))
     return _result(labels[:n], info)
+
+
+def leiden(ctx, indptr, indices, weights, options: LeidenOptions | None = None) -> LeidenResult:
+    """Deterministic Leiden on a symmetric CSR with integer (u64) weights: every cluster is connected inside itself."""
+    indptr = np.ascontiguousarray(indptr, dtype=np.uint64)
+    indices = np.ascontiguousarray(indices, dtype=np.uint32)
+    weights = np.ascontiguousarray(weights, dtype=np.uint64)
+    n = indptr.shape[0] - 1
+    labels = np.zeros(max(n, 1), dtype=np.uint32)
+    info = SbLeidenInfo()
+    o = _leiden_opts(options)
+    L.check(L.lib().sb_leiden(ctx._h, C.c_uint64(n), L.vp(indptr), L.vp(indices), L.vp(weights), C.byref(o), L.vp(labels), C.byref(info)))
+    return _leiden_result(labels[:n], info, o.quality)
+
+
+def cluster_knn_leiden(ctx, nbr, options: LeidenOptions | None = None) -> LeidenResult:
+    """kNN lists -> SNN graph -> Leiden, the graph kept on the device."""
+    nbr = _rows(nbr)
+    n, k = nbr.shape
+    labels = np.zeros(max(n, 1), dtype=np.uint32)
+    info = SbLeidenInfo()
+    o = _leiden_opts(options)
+    L.check(L.lib().sb_cluster_knn_leiden(ctx._h, L.vp(nbr), C.c_uint64(n), C.c_uint32(k), C.byref(o), L.vp(labels), C.byref(info)))
+    return _leiden_result(labels[:n], info, o.quality)
 
 
 class SbMergeOpts(C.Structure):  # include/scanb200.h: sb_merge_opts

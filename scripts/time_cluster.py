@@ -1,13 +1,15 @@
 """Timing of the graph clustering (csrc/cluster.cu) on the device.
 
 Workload: synthetic cells x 2,000 genes with the generator's 16 planted clusters -> CellRanger normalization -> BkSvd PCA (k = 10)
--> exhaustive kNN (k = 15) -> sb_cluster_knn.  Reported: the kNN time (separately: it is O(n^2) and dominates at large n), the
+-> exhaustive kNN (k = 15) -> sb_cluster_knn (--algorithm louvain) or sb_cluster_knn_leiden (--algorithm leiden).  Reported: the kNN time (separately: it is O(n^2) and dominates at large n), the
 clustering's device time (best and median of --reps after a warm-up), its stage split from the library's SCANB200_TRACE scopes
 (each ends in a stream synchronise; a level's time includes its aggregation), per level the node count, iterations and Q, the
 final Q, the ARI against the planted clusters, and the card name and power limit read in the same run.  With --compare the CPU
-oracle and networkx's Louvain run on the same graph (time, Q, ARI).
+oracle and networkx's Louvain run on the same graph (time, Q, ARI).  For Leiden the split is per pass (its levels, refinements and
+aggregations), and the labels of both algorithms are checked for clusters that are not connected inside themselves.
 
-usage: python scripts/time_cluster.py --cells 100000 --out profiles/cluster_100k.json [--compare]"""
+usage: python scripts/time_cluster.py --cells 100000 --out profiles/cluster_100k.json [--compare]
+       python scripts/time_cluster.py --algorithm leiden --cells 100000 --out profiles/leiden_100k.json"""
 import argparse
 import json
 import os
@@ -24,6 +26,7 @@ sys.path.insert(0, ROOT)
 import numpy as np  # noqa: E402
 
 import scan_rs_b200 as sb  # noqa: E402
+from oracle import leiden as ld  # noqa: E402
 from oracle import louvain as ol  # noqa: E402
 from scan_rs_b200.synth import SynthConfig, generate_device, tables  # noqa: E402
 
@@ -60,6 +63,45 @@ def stages(text):
     return {"snn_graph_ms": sum(snn), "level_ms": lev, "aggregation_ms": agg}
 
 
+def leiden_stages(text):
+    """per pass: the times of its levels, refinements and aggregations (every scope prints when it ends)"""
+    passes, cur = [], {"level_ms": [], "refinement_ms": [], "aggregation_ms": []}
+    snn = 0.0
+    for name, ms in re.findall(r"\[scanb200\] cluster: (snn graph|leiden level|refinement|aggregation|leiden pass)\s+([\d.]+) ms", text):
+        ms = float(ms)
+        if name == "snn graph":
+            snn += ms
+        elif name == "leiden pass":
+            passes.append({"pass_ms": ms, **cur})
+            cur = {"level_ms": [], "refinement_ms": [], "aggregation_ms": []}
+        else:
+            cur[{"leiden level": "level_ms", "refinement": "refinement_ms", "aggregation": "aggregation_ms"}[name]].append(ms)
+    return {"snn_graph_ms": snn, "passes": passes}
+
+
+def main_leiden(a, rec, ctx, nbr, truth):
+    o = sb.LeidenOptions(a.resolution)
+    res = sb.cluster_knn_leiden(ctx, nbr, o)  # warm-up
+    times = []
+    for _ in range(a.reps):
+        ctx.timer_begin()
+        sb.cluster_knn_leiden(ctx, nbr, o)
+        times.append(ctx.timer_end())
+    with Stderr() as err:
+        traced = sb.cluster_knn_leiden(ctx, nbr, o)
+    assert (traced.labels == res.labels).all()
+    ctx.timer_begin()
+    lv = sb.cluster_knn(ctx, nbr, sb.LouvainOptions(a.resolution))
+    louvain_ms = ctx.timer_end()
+    ip, ix, w = sb.snn_graph(ctx, nbr)
+    rec.update(resolution=a.resolution, cluster_ms_best=min(times), cluster_ms_median=float(np.median(times)), stages=leiden_stages(err.text),
+               n_passes=res.n_passes, stable=res.stable, levels_last_pass=res.levels, refined_last_pass=res.refined,
+               n_clusters=res.n_clusters, modularity=res.modularity, ari_planted=ol.adjusted_rand_index(truth, res.labels),
+               disconnected_labels=ld.disconnected_labels(ip, ix, res.labels),
+               louvain={"cluster_ms": louvain_ms, "n_clusters": lv.n_clusters, "modularity": lv.modularity,
+                        "ari_planted": ol.adjusted_rand_index(truth, lv.labels), "disconnected_labels": ld.disconnected_labels(ip, ix, lv.labels)})
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--cells", type=int, default=100000)
@@ -67,6 +109,8 @@ def main():
     ap.add_argument("--seed", type=int, default=3)
     ap.add_argument("--reps", type=int, default=3)
     ap.add_argument("--compare", action="store_true")
+    ap.add_argument("--algorithm", choices=["louvain", "leiden"], default="louvain")
+    ap.add_argument("--resolution", type=float, default=1.0)
     ap.add_argument("--out", default=None)
     a = ap.parse_args()
     rec = {"workload": f"synthetic {a.cells} cells x {a.genes} genes, 16 planted clusters, PCA k = 10, kNN k = 15", **gpu_info()}
@@ -80,6 +124,9 @@ def main():
         t0 = time.perf_counter()
         nbr = sb.knn(ctx, scores, 15)
         rec["knn_s"] = time.perf_counter() - t0
+        if a.algorithm == "leiden":
+            main_leiden(a, rec, ctx, nbr, truth)
+            return finish(a, rec)
         res = sb.cluster_knn(ctx, nbr)  # warm-up
         times = []
         for _ in range(a.reps):
@@ -112,6 +159,10 @@ def main():
                 nxl[list(cs)] = j
             rec["networkx"] = {"s": dt, "modularity": nx.community.modularity(G, comms, weight="weight"), "n_clusters": len(comms),
                                "ari_planted": ol.adjusted_rand_index(truth, nxl)}
+    finish(a, rec)
+
+
+def finish(a, rec):
     line = json.dumps(rec)
     print(line)
     if a.out:
