@@ -236,6 +236,17 @@ SB_API int sb_normalize(sb_mat *mat, int norm, const uint32_t *size_factors, sb_
  * 2 = scale_and_center(Axis(1), Some(sd_override[m])). */
 SB_API int sb_log_normalize(sb_mat *mat, int has_target, double target, int log_base, const uint32_t *size_factors,
                      int center_scale, const double *sd_override, sb_nmat **out);
+/* The reference's map applied to other cells (a second sample, late cells, a query mapped onto an atlas): out borrows `query`
+ * (not the reference: the reference may be freed first).  The reference must be a log-chain map whose column scale is
+ * target / total_c: sb_normalize with SB_NORM_CELLRANGER, _CELLRANGER8 or _SEURATLOG, or sb_log_normalize without size factors
+ * (any center_scale); any other (the binomial kinds, WITH_SIZE_FACTORS, LOG_TRANSFORM, fixed point, a map built with size
+ * factors) is SB_ERR_UNSUPPORTED.  The query gets col_scale = target / total_c from its own cell totals (the same rule, zero
+ * totals included) and its own L_c tables; the log base, row_scale (1/sd), u (-mean/sd) and the offset flags are the reference's,
+ * copied on the device.  The query must have the reference's m genes in the same order (select them with sb_select_rows) and its
+ * context (else SB_ERR_INVALID_ARG).  Sharded contexts: the query's cells are sharded; the m-vectors are the same on every rank.
+ * Scores in the reference's PCA space: sb_nmat_rdot(out, U^T, k) gives (A_q^T U)^T; for sb_bksvd's U, S, V of the reference
+ * A^T U = V diag(S), so the query's scores share the space of V diag(S). */
+SB_API int sb_normalize_like(sb_mat *query, const sb_nmat *reference, sb_nmat **out);
 /* log1p_normalize_fixed_point (normalization.rs:191-213) */
 SB_API int sb_normalize_fixed_point(sb_mat *mat, int log_base, uint32_t base, uint32_t exponent, sb_nmat **out);
 /* The derived tables: col_scale[n_local], row_scale[m] (1/sd), u[m], v[n_local]; any pointer may be NULL */
@@ -607,6 +618,59 @@ SB_API int sb_umap_layout(sb_ctx *ctx, uint64_t n, const uint64_t *indptr, const
                    const sb_umap_opts *opts, double *out, sb_umap_info *info);
 SB_API int sb_umap(sb_ctx *ctx, const double *scores, const uint32_t *nbr, uint64_t n_local, uint32_t dim, uint32_t k, const sb_umap_opts *opts,
             const double *init, double *out, sb_umap_info *info);
+
+/* UMAP transform: new points placed into a fixed reference embedding (umap-learn's transform: the reference never moves,
+ * move_other = False); restated by oracle/umap.py (transform_graph, transform_start, transform_layout).  opts as in the fit:
+ * n_components must equal the reference embedding's width (1..8); a, b (or min_dist / spread), learning_rate,
+ * repulsion_strength, negative_sample_rate and seed are used as in the fit; init and set_op_mix_ratio are ignored.
+ *
+ * Input: ref_scores[n_ref x dim] (the scores the reference embedding was fitted on), the query's scores[n x dim] and nbr[n x k],
+ * reference indices as sb_knn(points = ref_scores, queries = scores, k, include_self = 1) returns them; k is umap-learn's
+ * n_neighbors (the fit's k + 1).  2 <= k <= 128 and k <= n_ref (else SB_ERR_INVALID_ARG; k > 128: SB_ERR_UNSUPPORTED), n k < 2^28
+ * and n_ref < 2^32 - 1 (SB_ERR_UNSUPPORTED).  Rows must be full: padding, an index >= n_ref or a duplicate in a row is
+ * SB_ERR_INVALID_ARG.
+ *
+ * sb_umap_transform_graph: umap-learn's transform graph with local_connectivity - 1 = 0, bipartite, no fuzzy union.
+ *   d_ij    = sqrt(sum_c (r_j,c - x_i,c)^2), reference minus query, summed in coordinate order without contraction;
+ *   rho_i   = 0;
+ *   sigma_i by the fit's 64-step bisection with rho = 0 and target log2(k) (no self slot: k, not k + 1); every rho is 0, so every
+ *           row gets the global floor sigma_i >= 1e-3 (sum_i s_i / sum_i m_i), s_i = the row's distances summed in slot order, the
+ *           rows summed left to right in global query order, m_i = k (no + 1: umap-learn takes mean(dists) over the n x k array);
+ *   w_ij    = exp(-d_ij / sigma_i) (1 at d_ij = 0).
+ * weights[n x k] (slot order); sigma[n] may be NULL.
+ *
+ * sb_umap_transform_layout: the reference embedding ref_embedding[n_ref x n_components] (f64, finite, |e| < 2^30, else
+ * SB_ERR_INVALID_ARG; sb_umap's output is) and the query's nbr[n x k] with weights[n x k] in [0, 1] (a weight outside it, or a row
+ * whose weights are all 0, is SB_ERR_INVALID_ARG).  Positions are integers in units of 2^-32, the reference converted as
+ * rint(e 2^32).
+ *   start   umap-learn's init_graph_transform, slots in order: the reference position of the first slot with w = 1 if there is
+ *           one, else sum_slots (w / row_sum) e_j (row_sum = sum of the row's w in slot order), rounded to the 2^-32 grid;
+ *   epochs  n_epochs = 0: 100 if the global query count is <= 10,000, else 30; otherwise floor(n_epochs / 3); 0 returns the start;
+ *   prune   entries with w < w_max / n_epochs are dropped (w_max over all query entries, globally); per remaining entry eps =
+ *           w_max / w, epn = eps / negative_sample_rate, next = eps, next_neg = epn (the fit's schedule);
+ *   layout  alpha_t = (learning_rate / 4) (1 - t / n_epochs) (umap-learn's initial_alpha / 4).  For query row i (global index)
+ *           and epoch t = 0..n_epochs-1, the row's kept entries in slot order, each one with next <= t: attraction to the
+ *           reference point j with the fit's expression, c = alpha clip(g (y_i - e_j)) per coordinate; next += eps;
+ *           s = max(0, trunc((t - next_neg) / epn)) negative samples, the p-th one v = mix64(mix64(mix64(mix64(seed) ^ t) ^ e) ^ p)
+ *           % n_ref with e = i k + slot (none is skipped: the head is not a reference vertex); d2 > 0: c = alpha clip((2 gamma b) /
+ *           ((0.001 + d2) (a d2^b + 1)) (y_i - e_v)), d2 = 0: c = 4 alpha; next_neg += s epn.  Every contribution is rounded to
+ *           rint(c 2^32) and added to y_i at once; the reference is never written.  Only the head moves and a head's entries are
+ *           its own, so taking every epoch of one row before the next row equals umap-learn's loop (epochs outside, entries
+ *           inside) bit for bit.  A run whose epochs could move a point by 2^62 units is SB_ERR_UNSUPPORTED.
+ * out[n x n_components] (f64).  info: a, b, max_weight = w_max, n_epochs, n_edges = entries with w > 0, n_edges_used = entries
+ * left after pruning (both over all ranks).
+ *
+ * sb_umap_transform: sb_umap_transform_graph + sb_umap_transform_layout with the weights kept on the device.
+ * All three are collective on a cell-sharded context: every rank passes the whole reference (scores and embedding) and its own
+ * query rows and nbr, and gets its own rows back.  The global quantities use exact collectives (the row distance sums
+ * all-gathered and summed in order, sum m by the integer all-reduce, w_max as a max over the ranks, the query count and the
+ * rank's first row all-gathered); the query rows are not gathered.  The embedding equals world 1 bit for bit. */
+SB_API int sb_umap_transform_graph(sb_ctx *ctx, const double *ref_scores, uint64_t n_ref, const double *scores, const uint32_t *nbr, uint64_t n,
+                            uint32_t dim, uint32_t k, const sb_umap_opts *opts, double *weights, double *sigma);
+SB_API int sb_umap_transform_layout(sb_ctx *ctx, const double *ref_embedding, uint64_t n_ref, const uint32_t *nbr, const double *weights, uint64_t n,
+                             uint32_t k, const sb_umap_opts *opts, double *out, sb_umap_info *info);
+SB_API int sb_umap_transform(sb_ctx *ctx, const double *ref_scores, const double *ref_embedding, uint64_t n_ref, const double *scores,
+                      const uint32_t *nbr, uint64_t n_local, uint32_t dim, uint32_t k, const sb_umap_opts *opts, double *out, sb_umap_info *info);
 
 /* ---------------------------------------------------------------- t-SNE embedding (the reference's `bhtsne`, van der Maaten's
  * Barnes-Hut t-SNE) with bhtsne's parameter names, defaults and schedule; restated by oracle/tsne.py.

@@ -353,6 +353,13 @@ inline sqz::LowRankOffset log1p_normalize_fixed_point(const sqz::AdaptiveMat &ma
     check(sb_normalize_fixed_point(mat.raw(), (int)base, fp.base, fp.exponent, &h));
     return sqz::LowRankOffset(h, mat);
 }
+// the reference's map on the query's cells (sb_normalize_like): borrows `query`, so the reference may be freed first.  Query scores
+// in the reference's PCA space: normalize_like(query, reference).dot_left(U^T), transposed
+inline sqz::LowRankOffset normalize_like(const sqz::AdaptiveMat &query, const sqz::LowRankOffset &reference) {
+    sb_nmat *h = nullptr;
+    check(sb_normalize_like(query.raw(), reference.raw(), &h));
+    return sqz::LowRankOffset(h, query);
+}
 inline sqz::LowRankOffset binom_deviance_resid(const sqz::AdaptiveMat &mat) {  // :233-260
     sb_nmat *h = nullptr;
     check(sb_normalize(mat.raw(), SB_NORM_BINOMIAL_DEVIANCE, nullptr, &h));
@@ -753,6 +760,47 @@ inline Result umap(const Context &ctx, const std::vector<double> &scores, uint32
     sb_umap_info info;
     const sb_umap_opts c = detail::opts(o);
     check(sb_umap(ctx.raw(), scores.data(), nbr.data(), n, dim, k, &c, init.empty() ? nullptr : init.data(), out.data(), &info));
+    return detail::result(std::move(out), info);
+}
+// UMAP transform: new points placed into a fixed reference embedding (the rules are stated in scanb200.h).  ref_scores: n_ref x dim;
+// scores: n x dim; nbr: n x k reference indices (knn of the query against the reference, include_self = 1; k = n_neighbors)
+struct TransformGraph {
+    std::vector<double> weights;  // n x k, slot order
+    std::vector<double> sigma;    // n
+};
+inline TransformGraph umap_transform_graph(const Context &ctx, const std::vector<double> &ref_scores, const std::vector<double> &scores, uint32_t dim,
+                                           const std::vector<uint32_t> &nbr, uint32_t k, const Options &o = Options()) {
+    const uint64_t n = detail::rows(scores, dim, nbr, k);
+    if (ref_scores.size() % dim) throw Error(SB_ERR_INVALID_ARG, "ref_scores must hold n_ref x dim entries");
+    TransformGraph g{std::vector<double>(n * k), std::vector<double>(n)};
+    const sb_umap_opts c = detail::opts(o);
+    check(sb_umap_transform_graph(ctx.raw(), ref_scores.data(), ref_scores.size() / dim, scores.data(), nbr.data(), n, dim, k, &c, g.weights.data(),
+                                  g.sigma.data()));
+    return g;
+}
+// ref_embedding: n_ref x n_components
+inline Result umap_transform_layout(const Context &ctx, const std::vector<double> &ref_embedding, const std::vector<uint32_t> &nbr,
+                                    const std::vector<double> &weights, uint32_t k, const Options &o = Options()) {
+    if (k == 0 || nbr.size() % k || weights.size() != nbr.size()) throw Error(SB_ERR_INVALID_ARG, "nbr and weights must hold n x k entries");
+    if (o.n_components == 0 || ref_embedding.size() % o.n_components) throw Error(SB_ERR_INVALID_ARG, "ref_embedding must hold n_ref x n_components entries");
+    const uint64_t n = nbr.size() / k;
+    std::vector<double> out(n * o.n_components);
+    sb_umap_info info;
+    const sb_umap_opts c = detail::opts(o);
+    check(sb_umap_transform_layout(ctx.raw(), ref_embedding.data(), ref_embedding.size() / o.n_components, nbr.data(), weights.data(), n, k, &c,
+                                   out.data(), &info));
+    return detail::result(std::move(out), info);
+}
+// on a sharded context: the whole reference and this rank's query rows -> this rank's rows
+inline Result umap_transform(const Context &ctx, const std::vector<double> &ref_scores, const std::vector<double> &ref_embedding,
+                             const std::vector<double> &scores, uint32_t dim, const std::vector<uint32_t> &nbr, uint32_t k, const Options &o = Options()) {
+    const uint64_t n = detail::rows(scores, dim, nbr, k), n_ref = ref_scores.size() / dim;
+    if (ref_scores.size() % dim || ref_embedding.size() != n_ref * o.n_components)
+        throw Error(SB_ERR_INVALID_ARG, "ref_scores and ref_embedding must hold n_ref x dim and n_ref x n_components entries");
+    std::vector<double> out(n * o.n_components);
+    sb_umap_info info;
+    const sb_umap_opts c = detail::opts(o);
+    check(sb_umap_transform(ctx.raw(), ref_scores.data(), ref_embedding.data(), n_ref, scores.data(), nbr.data(), n, dim, k, &c, out.data(), &info));
     return detail::result(std::move(out), info);
 }
 // t-SNE embedding: perplexity-calibrated affinities and a deterministic Barnes-Hut layout (the rules are stated in scanb200.h)

@@ -204,6 +204,17 @@ impl<'c> DeviceCountMatrix<'c> {
         Ok(DeviceNormalized { h, mat: self })
     }
 
+    /// The reference's normalization applied to this matrix's cells (`sb_normalize_like`): column scales target / total_c from these
+    /// cells' own totals, the reference's log base, 1/sd row scales and offset.  The reference must be CellRanger, CellRanger8,
+    /// SeuratLog or a log normalization without size factors; this matrix must have its genes in the same order.  The result
+    /// borrows this matrix only.  Query scores in the reference's PCA space: (U^T . A_q)^T, i.e. A_q^T U, which for BkSvd's output
+    /// shares the space of V diag(S).
+    pub fn normalize_like(&self, reference: &DeviceNormalized<'_>) -> Result<DeviceNormalized<'_>, Error> {
+        let mut h = std::ptr::null_mut();
+        check(unsafe { ffi::sb_normalize_like(self.h, reference.h, &mut h) })?;
+        Ok(DeviceNormalized { h, mat: self })
+    }
+
     /// mean_var_axis(Axis(1)) of the SizeNormalized view (diff-exp/src/diff_exp.rs:458-472)
     pub fn mean_var_genes(&self, size_factors: Option<&[f64]>) -> Result<(Array1<f64>, Array1<f64>), Error> {
         let (mut mean, mut var) = (Array1::<f64>::zeros(self.rows), Array1::<f64>::zeros(self.rows));
@@ -745,6 +756,67 @@ pub fn umap(ctx: &Context, scores: &Array2<f64>, nbr: &Array2<u32>, opts: &UmapO
     let o = umap_opts(opts);
     let ip = init.as_ref().map_or(std::ptr::null(), |a| a.as_ptr());
     check(unsafe { ffi::sb_umap(ctx.h, scores.as_ptr(), nbr.as_ptr(), n as u64, dim as u32, k as u32, &o, ip, out.as_mut_ptr(), &mut info) })?;
+    Ok(umap_result(out, n, nc, &info))
+}
+
+/// The query rows' graph against the reference (`sb_umap_transform_graph`): ref_scores (n_ref x dim), the query's scores (n x dim)
+/// and nbr (n x k reference indices, `find_nn` of the query against the reference with include_self; k = umap-learn's
+/// n_neighbors) -> weights (n x k, slot order) and sigma (n)
+pub fn umap_transform_graph(ctx: &Context, ref_scores: &Array2<f64>, scores: &Array2<f64>, nbr: &Array2<u32>, opts: &UmapOptions)
+                            -> Result<(Array2<f64>, Vec<f64>), Error> {
+    let ref_scores = ref_scores.as_standard_layout();
+    let scores = scores.as_standard_layout();
+    let nbr = nbr.as_standard_layout();
+    let ((n, dim), k) = (scores.dim(), nbr.dim().1);
+    assert_eq!(nbr.dim().0, n, "scores and nbr must have the same rows");
+    assert_eq!(ref_scores.dim().1, dim, "ref_scores and scores must have the same columns");
+    let (mut w, mut sigma) = (vec![0.0; n * k], vec![0.0; n]);
+    let o = umap_opts(opts);
+    check(unsafe {
+        ffi::sb_umap_transform_graph(ctx.h, ref_scores.as_ptr(), ref_scores.dim().0 as u64, scores.as_ptr(), nbr.as_ptr(), n as u64, dim as u32,
+                                     k as u32, &o, w.as_mut_ptr(), sigma.as_mut_ptr())
+    })?;
+    Ok((Array2::from_shape_vec((n, k), w).expect("n x k"), sigma))
+}
+
+/// The start and the epochs of the query rows against the fixed reference embedding (n_ref x n_components)
+pub fn umap_transform_layout(ctx: &Context, ref_embedding: &Array2<f64>, nbr: &Array2<u32>, weights: &Array2<f64>, opts: &UmapOptions)
+                             -> Result<Umap, Error> {
+    let e = ref_embedding.as_standard_layout();
+    let nbr = nbr.as_standard_layout();
+    let weights = weights.as_standard_layout();
+    let ((n, k), nc) = (nbr.dim(), opts.n_components as usize);
+    assert_eq!(weights.dim(), (n, k), "nbr and weights must both be n x k");
+    assert_eq!(e.dim().1, nc, "ref_embedding must be n_ref x n_components");
+    let mut out = vec![0.0; n * nc];
+    let mut info = empty_umap_info();
+    let o = umap_opts(opts);
+    check(unsafe {
+        ffi::sb_umap_transform_layout(ctx.h, e.as_ptr(), e.dim().0 as u64, nbr.as_ptr(), weights.as_ptr(), n as u64, k as u32, &o, out.as_mut_ptr(),
+                                      &mut info)
+    })?;
+    Ok(umap_result(out, n, nc, &info))
+}
+
+/// New points placed into a fitted embedding (umap-learn's transform; the reference does not move), the weights kept on the
+/// device; on a sharded context every rank passes the whole reference and its own query rows, and receives its own rows
+pub fn umap_transform(ctx: &Context, ref_scores: &Array2<f64>, ref_embedding: &Array2<f64>, scores: &Array2<f64>, nbr: &Array2<u32>,
+                      opts: &UmapOptions) -> Result<Umap, Error> {
+    let ref_scores = ref_scores.as_standard_layout();
+    let e = ref_embedding.as_standard_layout();
+    let scores = scores.as_standard_layout();
+    let nbr = nbr.as_standard_layout();
+    let ((n, dim), k, nc) = (scores.dim(), nbr.dim().1, opts.n_components as usize);
+    assert_eq!(nbr.dim().0, n, "scores and nbr must have the same rows");
+    assert_eq!(ref_scores.dim().1, dim, "ref_scores and scores must have the same columns");
+    assert_eq!(e.dim(), (ref_scores.dim().0, nc), "ref_embedding must be n_ref x n_components");
+    let mut out = vec![0.0; n * nc];
+    let mut info = empty_umap_info();
+    let o = umap_opts(opts);
+    check(unsafe {
+        ffi::sb_umap_transform(ctx.h, ref_scores.as_ptr(), e.as_ptr(), e.dim().0 as u64, scores.as_ptr(), nbr.as_ptr(), n as u64, dim as u32, k as u32,
+                               &o, out.as_mut_ptr(), &mut info)
+    })?;
     Ok(umap_result(out, n, nc, &info))
 }
 

@@ -44,14 +44,14 @@ SYMBOLS = [
     "sb_version", "sb_last_error", "sb_init", "sb_shutdown", "sb_comm_unique_id", "sb_comm_init", "sb_sync", "sb_set_option", "sb_host_alloc", "sb_host_free",
     "sb_upload", "sb_upload_compact", "sb_pack_csc_count", "sb_pack_csc_fill", "sb_upload_packed", "sb_adaptive_decode_vec", "sb_upload_adaptive", "sb_mat_shape", "sb_download", "sb_free_mat", "sb_cell_totals", "sb_gene_totals", "sb_gene_nnz",
     "sb_median_cell_total", "sb_partition", "sb_select_rows", "sb_select_cols", "sb_hvg_select",
-    "sb_normalize", "sb_log_normalize", "sb_normalize_fixed_point", "sb_nmat_params", "sb_nmat_to_dense",
+    "sb_normalize", "sb_log_normalize", "sb_normalize_like", "sb_normalize_fixed_point", "sb_nmat_params", "sb_nmat_to_dense",
     "sb_nmat_dot", "sb_nmat_rdot", "sb_nmat_frobenius_sq", "sb_free_nmat", "sb_omega", "sb_bksvd", "sb_bksvd_run_pca", "sb_pca_diagnostics", "sb_randsvd",
     "sb_randsvd_run_pca", "sb_profile_enable", "sb_profile_reset", "sb_profile_get", "sb_timer_begin",
     "sb_timer_end", "sb_flush_l2", "sb_synth_generate", "sb_knn",
     "sb_irlba", "sb_irlba_start", "sb_mean_var_axis", "sb_mean_var_rows", "sb_sum_rows", "sb_sum_cols", "sb_sum_rows_dual", "sb_size_factors", "sb_upload_unsorted", "sb_filter_genes", "sb_multi_init", "sb_multi_size", "sb_multi_ctx", "sb_multi_run", "sb_multi_shutdown",
     "sb_sseq_compute_params", "sb_sseq_diff_exp", "sb_sseq_one_vs_rest", "sb_sseq_pairs",
     "sb_snn_graph", "sb_louvain", "sb_cluster_knn", "sb_leiden", "sb_cluster_knn_leiden", "sb_linkage_complete", "sb_merge_clusters",
-    "sb_umap_graph", "sb_umap_layout", "sb_umap", "sb_tsne_affinities", "sb_tsne_layout", "sb_tsne",
+    "sb_umap_graph", "sb_umap_layout", "sb_umap", "sb_umap_transform_graph", "sb_umap_transform_layout", "sb_umap_transform", "sb_tsne_affinities", "sb_tsne_layout", "sb_tsne",
 ]
 
 _lib = None

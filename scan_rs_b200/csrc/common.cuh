@@ -320,6 +320,9 @@ struct sb_nmat {
     bool v_ones = true;
     DevBuf<double> u;  // [m]
     DevBuf<double> v;  // [n] (only when !v_ones)
+    // a log-chain map whose column scale is target / total_c (no size factors): sb_normalize_like can apply it to other cells
+    bool like_ok = false;
+    double target = 0.0;
 };
 
 // ---------------------------------------------------------------- profiling helpers (ctx.cu)
@@ -366,10 +369,11 @@ __host__ __device__ __forceinline__ u64 um_mix64(u64 z) {
     z = (z ^ (z >> 27)) * 0x94D049BB133111EBull;
     return z ^ (z >> 31);
 }
-//   thread per (row, slot) of nbr [n x k] (0xFFFFFFFF pads a row's end): err bits 1 index >= n, 2 self index, 4 duplicate in the
-//   row, 8 padding before the row end; d = sqrt(sum_c (x_j,c - x_i,c)^2) in coordinate order without contraction (0 at padding)
-__global__ void k_um_dist(const double *__restrict__ X, const u32 *__restrict__ nbr, u64 n, u32 dim, u32 k, double *__restrict__ d,
-                          int *__restrict__ err);
+//   thread per (row i, slot) of nbr [n x k], the neighbours j rows of P [np x dim] (0xFFFFFFFF pads a row's end): err bits 1
+//   index >= np, 2 self index (P = X only), 4 duplicate in the row, 8 padding before the row end, 16 padding where full rows are
+//   required (full = 1); d = sqrt(sum_c (p_j,c - x_i,c)^2) in coordinate order without contraction (0 at padding)
+__global__ void k_um_dist(const double *__restrict__ X, const double *__restrict__ P, u64 np, const u32 *__restrict__ nbr, u64 n, u32 dim,
+                          u32 k, int full, double *__restrict__ d, int *__restrict__ err);
 //   a weighted graph on the device: symmetric CSR, columns ascending, f64 weights in (0, 1]
 struct UmGraph {
     u64 n = 0, nnz = 0;

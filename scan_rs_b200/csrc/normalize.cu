@@ -172,6 +172,34 @@ extern "C" int sb_nmat_frobenius_sq(sb_nmat *a, double *out) {
     return SB_OK;
 }
 
+// col_scale = target / (size factor or cell total) per local cell (normalization.rs:169), and the L_c(1) and level tables of it
+static int log_col_tables(sb_nmat *a, double target, const uint32_t *size_factors) {
+    sb_mat *mat = a->mat;
+    sb_ctx *ctx = mat->ctx;
+    a->target = target;
+    a->like_ok = size_factors == nullptr;
+    SB_TRY(a->col_scale.alloc(mat->n));
+    if (mat->n) {
+        const u32 *counts = mat->cell_tot.p;
+        DevBuf<u32> d_sf;
+        if (size_factors) {
+            SB_TRY(d_sf.alloc(mat->n));
+            SB_CUDA(cudaMemcpyAsync(d_sf.p, size_factors, mat->n * sizeof(u32), cudaMemcpyHostToDevice, ctx->stream));
+            counts = d_sf.p;
+        }
+        k_col_scale<<<cdiv(mat->n, 256), 256, 0, ctx->stream>>>(counts, mat->n, target, a->col_scale.p);
+        SB_TRY(a->l1c.alloc(mat->n));
+        SB_TRY(a->inv_l1c.alloc(mat->n));
+        k_l1_tables<<<cdiv(mat->n, 256), 256, 0, ctx->stream>>>(a->col_scale.p, mat->n, a->log_base, a->l1c.p, a->inv_l1c.p);
+        SB_TRY(a->lk.alloc(mat->n * PL_MAX_LEVELS));
+        k_level_table<<<cdiv(mat->n * PL_MAX_LEVELS, 256), 256, 0, ctx->stream>>>(a->col_scale.p, mat->n, a->log_base, a->lk.p);
+        count_launch(ctx);
+        count_launch(ctx); count_launch(ctx);
+        SB_CUDA(cudaStreamSynchronize(ctx->stream));
+    }
+    return SB_OK;
+}
+
 extern "C" int sb_log_normalize(sb_mat *mat, int has_target, double target, int log_base, const uint32_t *size_factors,
                                 int center_scale, const double *sd_override, sb_nmat **out) {
     if (!mat || !out) return sb_fail(SB_ERR_INVALID_ARG, "sb_log_normalize: NULL argument");
@@ -195,25 +223,7 @@ extern "C" int sb_log_normalize(sb_mat *mat, int has_target, double target, int 
         SB_TRY(mat_median_total(mat, &med, &nonempty));
         target = nonempty ? ((double)med > 1.0 ? (double)med : 1.0) : 1.0;  // .max(1.0), map_or(1.0)
     }
-    SB_TRY(a->col_scale.alloc(mat->n));
-    if (mat->n) {
-        const u32 *counts = mat->cell_tot.p;
-        DevBuf<u32> d_sf;
-        if (size_factors) {
-            SB_TRY(d_sf.alloc(mat->n));
-            SB_CUDA(cudaMemcpyAsync(d_sf.p, size_factors, mat->n * sizeof(u32), cudaMemcpyHostToDevice, ctx->stream));
-            counts = d_sf.p;
-        }
-        k_col_scale<<<cdiv(mat->n, 256), 256, 0, ctx->stream>>>(counts, mat->n, target, a->col_scale.p);
-        SB_TRY(a->l1c.alloc(mat->n));
-        SB_TRY(a->inv_l1c.alloc(mat->n));
-        k_l1_tables<<<cdiv(mat->n, 256), 256, 0, ctx->stream>>>(a->col_scale.p, mat->n, log_base, a->l1c.p, a->inv_l1c.p);
-        SB_TRY(a->lk.alloc(mat->n * PL_MAX_LEVELS));
-        k_level_table<<<cdiv(mat->n * PL_MAX_LEVELS, 256), 256, 0, ctx->stream>>>(a->col_scale.p, mat->n, log_base, a->lk.p);
-        count_launch(ctx);
-        count_launch(ctx); count_launch(ctx);
-        SB_CUDA(cudaStreamSynchronize(ctx->stream));
-    }
+    SB_TRY(log_col_tables(a.get(), target, size_factors));
     if (center_scale) {
         DevBuf<double> S, sd;
         SB_TRY(S.alloc(2 * (size_t)mat->m));
@@ -308,8 +318,11 @@ extern "C" int sb_normalize(sb_mat *mat, int norm, const uint32_t *size_factors,
     }
     case SB_NORM_SEURATLOG:  // :59, :90-92
         return sb_log_normalize(mat, 1, 10000.0, SB_LOG_E, nullptr, 1, nullptr, out);
-    case SB_NORM_WITH_SIZE_FACTORS:  // :93-95 (size_factors == None falls back to the cell totals, :148-160)
-        return sb_log_normalize(mat, 0, 0.0, SB_LOG_TWO, size_factors, 1, nullptr, out);
+    case SB_NORM_WITH_SIZE_FACTORS: {  // :93-95 (size_factors == None falls back to the cell totals, :148-160)
+        const int rc = sb_log_normalize(mat, 0, 0.0, SB_LOG_TWO, size_factors, 1, nullptr, out);
+        if (rc == SB_OK) (*out)->like_ok = false;  // a size-factor map: sb_normalize_like does not apply it
+        return rc;
+    }
     case SB_NORM_LOG_TRANSFORM: {  // :96-100
         std::vector<u32> ones(mat->n, 1u);
         return sb_log_normalize(mat, 1, 1.0, SB_LOG_TWO, ones.data(), 1, nullptr, out);
@@ -321,6 +334,43 @@ extern "C" int sb_normalize(sb_mat *mat, int norm, const uint32_t *size_factors,
     default:
         return sb_fail(SB_ERR_INVALID_ARG, "sb_normalize: not implemented (normalization %d)", norm);
     }
+}
+
+// the reference's map applied to the query's cells: col_scale = target / total_c from the query's own totals and its own L_c tables;
+// log base, 1/sd row scales, the -mean/sd offset and the flags copied device to device (the m-vectors are the same on every rank)
+extern "C" int sb_normalize_like(sb_mat *query, const sb_nmat *reference, sb_nmat **out) {
+    if (!query || !reference || !out) return sb_fail(SB_ERR_INVALID_ARG, "sb_normalize_like: NULL argument");
+    *out = nullptr;
+    if (query->ctx != reference->ctx) return sb_fail(SB_ERR_INVALID_ARG, "sb_normalize_like: the query and the reference have different contexts");
+    if (!reference->like_ok)
+        return sb_fail(SB_ERR_UNSUPPORTED, "sb_normalize_like: the reference must be a log-chain normalization without size factors "
+                                           "(CellRanger, CellRanger8, SeuratLog or sb_log_normalize without size factors)");
+    if (query->m != reference->mat->m)
+        return sb_fail(SB_ERR_INVALID_ARG, "sb_normalize_like: the query has %u genes, the reference %u", query->m, reference->mat->m);
+    sb_ctx *ctx = query->ctx;
+    SB_ENTER(ctx);
+    std::unique_ptr<sb_nmat> a(new sb_nmat());
+    a->mat = query;
+    a->ctx = ctx;
+    a->kind = 1;
+    a->log_base = reference->log_base;
+    SB_TRY(mat_cell_totals_dev(query));
+    SB_TRY(log_col_tables(a.get(), reference->target, nullptr));
+    a->has_row_scale = reference->has_row_scale;
+    a->has_offset = reference->has_offset;
+    a->v_ones = reference->v_ones;
+    const size_t mb = (size_t)query->m * sizeof(double);
+    if (a->has_row_scale) {
+        SB_TRY(a->row_scale.alloc(query->m));
+        if (mb) SB_CUDA(cudaMemcpyAsync(a->row_scale.p, reference->row_scale.p, mb, cudaMemcpyDeviceToDevice, ctx->stream));
+    }
+    if (a->has_offset) {
+        SB_TRY(a->u.alloc(query->m));
+        if (mb) SB_CUDA(cudaMemcpyAsync(a->u.p, reference->u.p, mb, cudaMemcpyDeviceToDevice, ctx->stream));
+    }
+    SB_CUDA(cudaStreamSynchronize(ctx->stream));
+    *out = a.release();
+    return SB_OK;
 }
 
 extern "C" int sb_normalize_fixed_point(sb_mat *mat, int log_base, uint32_t base, uint32_t exponent, sb_nmat **out) {

@@ -212,7 +212,7 @@ static int ts_affinities(sb_ctx *ctx, double *X, const u32 *nbr, u64 n, u32 dim,
     ts.run(ctx, X, dim, dim, n, nullptr, 1, st.p);
     k_ts_center_cols<<<ts_grid(ctx, n * dim, 256), 256, 0, ctx->stream>>>(X, n, dim, st.p, amax.p);
     k_ts_scale<<<ts_grid(ctx, n * dim, 256), 256, 0, ctx->stream>>>(X, n * dim, amax.p);
-    k_um_dist<<<ts_grid(ctx, nk, 256), 256, 0, ctx->stream>>>(X, nbr, n, dim, k, d.p, err.p);
+    k_um_dist<<<ts_grid(ctx, nk, 256), 256, 0, ctx->stream>>>(X, X, n, nbr, n, dim, k, 0, d.p, err.p);
     k_ts_beta<<<ts_grid(ctx, n, 128), 128, 0, ctx->stream>>>(d.p, nbr, n, k, log(perplexity), pc.p, beta.p, keys.p, vals.p);
     for (int q = 0; q < 4; q++) count_launch(ctx);
     SB_CUDA(cudaGetLastError());

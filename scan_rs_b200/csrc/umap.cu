@@ -11,6 +11,8 @@
 //            contribution alpha grad is rounded to an integer multiple of 2^-32 and summed per vertex with 64-bit atomics, so the
 //            sums do not depend on the order the atomics land in, and the positions are kept as those integers.  No host round
 //            trip inside the epoch loop.
+//   transform  new points into a fixed embedding (umap-learn's transform): the graph from the fit's kernels against a second
+//            point set with rho = 0, then k_ut_start and k_ut_layout, a thread per query row running every epoch in one launch.
 #include <cmath>
 
 #include <cub/cub.cuh>
@@ -33,8 +35,8 @@ static int um_grid(sb_ctx *ctx, u64 items, int per_block) {
 }
 
 // ---------------------------------------------------------------- graph
-__global__ void k_um_dist(const double *__restrict__ X, const u32 *__restrict__ nbr, u64 n, u32 dim, u32 k, double *__restrict__ d,
-                          int *__restrict__ err) {
+__global__ void k_um_dist(const double *__restrict__ X, const double *__restrict__ P, u64 np, const u32 *__restrict__ nbr, u64 n, u32 dim,
+                          u32 k, int full, double *__restrict__ d, int *__restrict__ err) {
     for (u64 s = (u64)blockIdx.x * blockDim.x + threadIdx.x; s < n * k; s += (u64)gridDim.x * blockDim.x) {
         const u64 i = s / k;
         const u32 t = (u32)(s - i * k), j = nbr[s];
@@ -42,18 +44,20 @@ __global__ void k_um_dist(const double *__restrict__ X, const u32 *__restrict__ 
         int e = 0;
         if (j != UM_PAD) {
             if (t && nbr[s - 1] == UM_PAD) e |= 8;
-            if (j >= n) e |= 1;
-            else if (j == i) e |= 2;
+            if (j >= np) e |= 1;
+            else if (!full && j == i) e |= 2;
             for (u32 q = 0; q < t; q++)
                 if (nbr[i * k + q] == j) e |= 4;
             if (!e) {
-                const double *xi = X + i * dim, *xj = X + (u64)j * dim;
+                const double *xi = X + i * dim, *xj = P + (u64)j * dim;
                 for (u32 c = 0; c < dim; c++) {
                     const double df = __dsub_rn(xj[c], xi[c]);
                     r = __dadd_rn(r, __dmul_rn(df, df));
                 }
                 r = sqrt(r);
             }
+        } else if (full) {
+            e |= 16;
         }
         d[s] = r;
         if (e) atomicOr(err, e);
@@ -61,9 +65,11 @@ __global__ void k_um_dist(const double *__restrict__ X, const u32 *__restrict__ 
 }
 
 // thread per row: rho, the row sum of the distances, sigma by umap-learn's bisection with the row-mean floor (rows with rho = 0
-// get the global floor later: flag[0] = 1), cnt[0] += listed entries + 1
-__global__ void k_um_smooth(const double *__restrict__ d, const u32 *__restrict__ nbr, u64 n, u32 k, double target, double *__restrict__ rho,
-                            double *__restrict__ sigma, double *__restrict__ rowsum, int *__restrict__ flag, ull *__restrict__ cnt) {
+// get the global floor later: flag[0] = 1), cnt[0] += listed entries + 1.  rho0 = 1 (the transform's local connectivity 0): rho = 0
+// on every row and cnt[0] += listed entries
+__global__ void k_um_smooth(const double *__restrict__ d, const u32 *__restrict__ nbr, u64 n, u32 k, double target, int rho0,
+                            double *__restrict__ rho, double *__restrict__ sigma, double *__restrict__ rowsum, int *__restrict__ flag,
+                            ull *__restrict__ cnt) {
     for (u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (u64)gridDim.x * blockDim.x) {
         const double *di = d + i * k;
         const u32 *ri = nbr + i * k;
@@ -73,7 +79,7 @@ __global__ void k_um_smooth(const double *__restrict__ d, const u32 *__restrict_
             if (ri[t] == UM_PAD) continue;
             m++;
             s = __dadd_rn(s, di[t]);
-            if (di[t] > 0.0 && di[t] < r) r = di[t];
+            if (!rho0 && di[t] > 0.0 && di[t] < r) r = di[t];
         }
         if (r == INFINITY) r = 0.0;
         double lo = 0.0, hi = INFINITY, mid = 1.0;
@@ -102,7 +108,7 @@ __global__ void k_um_smooth(const double *__restrict__ d, const u32 *__restrict_
         rho[i] = r;
         sigma[i] = mid;
         rowsum[i] = s;
-        atomicAdd(cnt, (ull)(m + 1));
+        atomicAdd(cnt, (ull)(rho0 ? m : m + 1));
     }
 }
 
@@ -112,7 +118,7 @@ __global__ void k_um_global_floor(const double *__restrict__ rho, double *__rest
 }
 
 // thread per (row, slot): w = exp(-max(0, d - rho) / sigma); the forward key (i << 32 | j, value: the slot) and the transposed key
-// (j << 32 | i, value: the slot | UM_TAG); all-ones keys at padding
+// (j << 32 | i, value: the slot | UM_TAG); all-ones keys at padding.  keys = NULL: the weights only
 __global__ void k_um_member(const double *__restrict__ d, const u32 *__restrict__ nbr, u64 n, u32 k, const double *__restrict__ rho,
                             const double *__restrict__ sigma, double *__restrict__ w, u64 *__restrict__ keys, u64 *__restrict__ vals) {
     for (u64 s = (u64)blockIdx.x * blockDim.x + threadIdx.x; s < n * k; s += (u64)gridDim.x * blockDim.x) {
@@ -120,12 +126,14 @@ __global__ void k_um_member(const double *__restrict__ d, const u32 *__restrict_
         const u32 j = nbr[s];
         if (j == UM_PAD) {
             w[s] = 0.0;
+            if (!keys) continue;
             keys[2 * s] = keys[2 * s + 1] = ~0ull;
             vals[2 * s] = vals[2 * s + 1] = 0;
             continue;
         }
         const double x = __dsub_rn(d[s], rho[i]);
         w[s] = x > 0.0 ? exp(-__ddiv_rn(x, sigma[i])) : 1.0;
+        if (!keys) continue;
         keys[2 * s] = (i << 32) | j;
         vals[2 * s] = s;
         keys[2 * s + 1] = ((u64)j << 32) | i;
@@ -217,8 +225,9 @@ static int um_graph_build(sb_ctx *ctx, const double *X, const u32 *nbr, u64 n, u
     SB_CUDA(cudaMemsetAsync(cnt.p, 0, sizeof(ull), ctx->stream));
     g.n = n;
     if (n) {
-        k_um_dist<<<um_grid(ctx, nk, 256), 256, 0, ctx->stream>>>(X, nbr, n, dim, k, d.p, flags.p);
-        k_um_smooth<<<um_grid(ctx, n, 128), 128, 0, ctx->stream>>>(d.p, nbr, n, k, std::log2((double)k + 1.0), rho.p, sigma.p, rs.p, flags.p + 1, cnt.p);
+        k_um_dist<<<um_grid(ctx, nk, 256), 256, 0, ctx->stream>>>(X, X, n, nbr, n, dim, k, 0, d.p, flags.p);
+        k_um_smooth<<<um_grid(ctx, n, 128), 128, 0, ctx->stream>>>(d.p, nbr, n, k, std::log2((double)k + 1.0), 0, rho.p, sigma.p, rs.p, flags.p + 1,
+                                                                   cnt.p);
         count_launch(ctx);
         count_launch(ctx);
         SB_CUDA(cudaGetLastError());
@@ -875,4 +884,422 @@ extern "C" int sb_umap(sb_ctx *ctx, const double *X, const uint32_t *nbr, uint64
     dU.release();
     SB_TRY(um_layout(ctx, g, Y, o, info, "sb_umap"));
     return um_copy_out(ctx, Y, off, n_local, o.nc, out);
+}
+
+// ---------------------------------------------------------------- transform: new points into a fixed reference embedding
+// umap-learn's transform with move_other = False: only the query point (the head) moves, and a head's entries are its own, so one
+// thread per query row runs every epoch with its entries in slot order and adds every contribution at once.  That is umap-learn's
+// loop (epochs outside, entries inside) bit for bit, in one launch, without atomics.
+
+// thread per row of the n x k weights: the start (umap-learn's init_graph_transform, slots in order) into Y; the largest weight
+// (positive doubles order as their bits) and the entries with w > 0 into mx[0], mx[1]; err bits 32 a weight outside [0, 1], 64 a
+// row whose weights are all 0
+__global__ void k_ut_start(const u32 *__restrict__ nbr, const double *__restrict__ w, u64 n, u32 k, u32 nc, const i64 *__restrict__ E,
+                           i64 *__restrict__ Y, ull *__restrict__ mx, int *__restrict__ err) {
+    for (u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (u64)gridDim.x * blockDim.x) {
+        const double *wi = w + i * k;
+        const u32 *ri = nbr + i * k;
+        double rs = 0.0;
+        ull m = 0, pos = 0;
+        u32 one = k;
+        int e = 0;
+        for (u32 t = 0; t < k; t++) {
+            const double v = wi[t];
+            if (!(v >= 0.0 && v <= 1.0)) e |= 32;
+            rs = __dadd_rn(rs, v);
+            if (v > 0.0) pos++;
+            if (v == 1.0 && one == k) one = t;
+            const ull b = (ull)__double_as_longlong(v);
+            m = v > 0.0 && b > m ? b : m;
+        }
+        if (!e && !(rs > 0.0)) e |= 64;
+        if (e) {
+            atomicOr(err, e);
+            continue;
+        }
+        for (u32 c = 0; c < nc; c++) {
+            if (one < k) {
+                Y[i * nc + c] = E[(u64)ri[one] * nc + c];
+                continue;
+            }
+            double acc = 0.0;
+            for (u32 t = 0; t < k; t++)
+                acc = __dadd_rn(acc, __dmul_rn(__ddiv_rn(wi[t], rs), __dmul_rn((double)E[(u64)ri[t] * nc + c], UM_IFIX)));
+            Y[i * nc + c] = __double2ll_rn(__dmul_rn(acc, UM_FIX));
+        }
+        if (m) atomicMax(&mx[0], m);
+        atomicAdd(&mx[1], pos);
+    }
+}
+
+struct UtArgs {
+    const u32 *nbr;      // [n x k] reference indices
+    const double *w;     // [n x k]
+    const i64 *E;        // [n_ref x NC] the reference, units of 2^-32 (never written)
+    i64 *Y;              // [n x NC] the start in, the result out
+    double *ens, *enn;   // [k x n] next epoch of each entry and of its negative samples
+    ull *used;           // entries left after pruning
+    u64 n, n_ref, row0;  // row0: the global index of local row 0
+    u32 k, n_epochs;
+    double wmax, thr, rate, a, b, bm1, m2ab, two_gb, alpha0;
+    u64 key0;            // mix64(seed)
+    int negatives;
+};
+
+// thread per query row, every epoch
+template <int NC>
+__global__ void __launch_bounds__(128) k_ut_layout(UtArgs p) {
+    for (u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x; i < p.n; i += (u64)gridDim.x * blockDim.x) {
+        i64 y[NC];
+#pragma unroll
+        for (int c = 0; c < NC; c++) y[c] = p.Y[i * NC + c];
+        const double *wi = p.w + i * p.k;
+        const u32 *ri = p.nbr + i * p.k;
+        ull used = 0;
+        for (u32 t = 0; t < p.k; t++) {  // prune and schedule: eps = w_max / w, epn = eps / rate; next = eps, next_neg = epn
+            const double v = wi[t];
+            const bool keep = v >= p.thr;
+            const double eps = keep ? __ddiv_rn(p.wmax, v) : INFINITY;
+            p.ens[(u64)t * p.n + i] = eps;
+            p.enn[(u64)t * p.n + i] = p.negatives ? __ddiv_rn(eps, p.rate) : INFINITY;
+            used += keep;
+        }
+        if (used) atomicAdd(p.used, used);
+        for (u32 ep = 0; ep < p.n_epochs; ep++) {
+            const double epoch = (double)ep;
+            const double alpha = __dmul_rn(p.alpha0, __dsub_rn(1.0, __ddiv_rn(epoch, (double)p.n_epochs)));
+            const u64 key = um_mix64(p.key0 ^ (u64)ep);
+            for (u32 t = 0; t < p.k; t++) {
+                double *ens = p.ens + (u64)t * p.n + i;
+                const double ns = *ens;
+                if (ns > epoch) continue;
+                const u64 j = ri[t];
+                double yi[NC], yk[NC];
+                double d2 = 0.0;
+#pragma unroll
+                for (int c = 0; c < NC; c++) {
+                    yi[c] = __dmul_rn((double)y[c], UM_IFIX);
+                    yk[c] = __dmul_rn((double)p.E[j * NC + c], UM_IFIX);
+                    const double df = __dsub_rn(yi[c], yk[c]);
+                    d2 = __dadd_rn(d2, __dmul_rn(df, df));
+                }
+                const double gc = d2 > 0.0 ? __ddiv_rn(__dmul_rn(p.m2ab, pow(d2, p.bm1)), __dadd_rn(__dmul_rn(p.a, pow(d2, p.b)), 1.0)) : 0.0;
+#pragma unroll
+                for (int c = 0; c < NC; c++) y[c] += um_fix(um_clip(__dmul_rn(gc, __dsub_rn(yi[c], yk[c]))), alpha);
+                const double eps = __ddiv_rn(p.wmax, wi[t]);
+                *ens = __dadd_rn(ns, eps);
+                if (!p.negatives) continue;
+                double *enn = p.enn + (u64)t * p.n + i;
+                const double epn = __ddiv_rn(eps, p.rate), nn_f = *enn;
+                i64 nn = (i64)__ddiv_rn(__dsub_rn(epoch, nn_f), epn);
+                if (nn < 0) nn = 0;
+                const u64 k2 = um_mix64(key ^ ((p.row0 + i) * p.k + t));
+                for (i64 s = 0; s < nn; s++) {
+                    const u64 v = um_mix64(k2 ^ (u64)s) % p.n_ref;
+                    double dd = 0.0;
+#pragma unroll
+                    for (int c = 0; c < NC; c++) {
+                        yi[c] = __dmul_rn((double)y[c], UM_IFIX);
+                        yk[c] = __dmul_rn((double)p.E[v * NC + c], UM_IFIX);
+                        const double df = __dsub_rn(yi[c], yk[c]);
+                        dd = __dadd_rn(dd, __dmul_rn(df, df));
+                    }
+                    if (dd > 0.0) {
+                        const double g = __ddiv_rn(p.two_gb, __dmul_rn(__dadd_rn(0.001, dd), __dadd_rn(__dmul_rn(p.a, pow(dd, p.b)), 1.0)));
+#pragma unroll
+                        for (int c = 0; c < NC; c++) y[c] += um_fix(um_clip(__dmul_rn(g, __dsub_rn(yi[c], yk[c]))), alpha);
+                    } else {
+                        const i64 f = um_fix(4.0, alpha);
+#pragma unroll
+                        for (int c = 0; c < NC; c++) y[c] += f;
+                    }
+                }
+                *enn = __dadd_rn(nn_f, __dmul_rn((double)nn, epn));
+            }
+        }
+#pragma unroll
+        for (int c = 0; c < NC; c++) p.Y[i * NC + c] = y[c];
+    }
+}
+
+template <int NC>
+static void ut_launch_layout(sb_ctx *ctx, const UtArgs &a) {
+    k_ut_layout<NC><<<um_grid(ctx, a.n, 128), 128, 0, ctx->stream>>>(a);
+}
+
+// the entry points' host checks (k, n_ref, sizes; opts with init and set_op_mix_ratio ignored); NULL pointers are the caller's
+static int ut_args(const sb_umap_opts *opts, u64 n_ref, u64 n, u32 k, UmOpts &o, const char *fn) {
+    sb_umap_opts c = opts ? *opts : sb_umap_opts{2, 0, 0.1, 1.0, 0.0, 0.0, 1.0, 1.0, 1.0, 5, SB_UMAP_INIT_PCA, 0};
+    c.init = SB_UMAP_INIT_PCA;
+    c.set_op_mix_ratio = 1.0;
+    SB_TRY(um_opts(&c, o, fn));
+    if (k < 2) return sb_fail(SB_ERR_INVALID_ARG, "%s: k must be >= 2", fn);
+    if (k > UM_MAX_K) return sb_fail(SB_ERR_UNSUPPORTED, "%s: k must be <= %d", fn, UM_MAX_K);
+    if (n_ref >= 0xFFFFFFFFull) return sb_fail(SB_ERR_UNSUPPORTED, "%s: n_ref must be below 2^32 - 1", fn);
+    if (k > n_ref) return sb_fail(SB_ERR_INVALID_ARG, "%s: k must be <= n_ref", fn);
+    if (n * k >= ((u64)1 << 28)) return sb_fail(SB_ERR_UNSUPPORTED, "%s: n x k must be below 2^28", fn);
+    return SB_OK;
+}
+
+// the reference embedding [n_ref x nc]: finite and |e| < 2^30
+static int ut_ref_embedding(const double *e, u64 n_ref, u32 nc, const char *fn) {
+    if (!e) return sb_fail(SB_ERR_INVALID_ARG, "%s: NULL argument", fn);
+    for (u64 x = 0; x < n_ref * nc; x++)
+        if (!(std::fabs(e[x]) < UM_INIT_LIMIT)) return sb_fail(SB_ERR_INVALID_ARG, "%s: ref_embedding values must be finite and below 2^30 in magnitude", fn);
+    return SB_OK;
+}
+
+// the device error bits of k_um_dist / k_ut_start -> a status (agreed over the ranks by the caller)
+static int ut_err(int e, const char *fn) {
+    if (!e) return SB_OK;
+    return sb_fail(SB_ERR_INVALID_ARG, "%s: invalid neighbour lists or weights:%s%s%s%s%s", fn, e & 1 ? " an index >= n_ref" : "",
+                   e & 4 ? " a duplicate in a row" : "", e & 24 ? " padding (rows must be full)" : "", e & 32 ? " a weight outside [0, 1]" : "",
+                   e & 64 ? " a row whose weights are all 0" : "");
+}
+
+// every rank's row count -> the global query count and this rank's first row; k must agree
+static int ut_rows(sb_ctx *ctx, u64 n, u32 k, u64 &n_global, u64 &row0, const char *fn) {
+    std::vector<u64> counts, ks;
+    SB_TRY(comm_allgather_u64_host(ctx, n, counts));
+    SB_TRY(comm_allgather_u64_host(ctx, k, ks));
+    n_global = row0 = 0;
+    for (int r = 0; r < ctx->nranks; r++) {
+        if (ks[r] != k) return sb_fail(SB_ERR_INVALID_ARG, "%s: k differs between ranks (rank %d)", fn, r);
+        if (r < ctx->rank) row0 += counts[r];
+        n_global += counts[r];
+    }
+    return SB_OK;
+}
+
+// the query rows' graph: X [n x dim] against the reference R [n_ref x dim], nbr [n x k] on the device -> w [n x k], sigma [n]
+static int ut_graph(sb_ctx *ctx, const double *R, u64 n_ref, const double *X, const u32 *nbr, u64 n, u32 dim, u32 k, DevBuf<double> &w,
+                    DevBuf<double> &sigma, const char *fn) {
+    TraceScope tr(ctx, "umap transform: graph");
+    const u64 nk = n * k;
+    DevBuf<double> d, rho, rs;
+    DevBuf<int> flags;  // [0] error bits, [1] unused (every rho is 0)
+    DevBuf<ull> cnt;
+    SB_TRY(d.alloc(nk));
+    SB_TRY(w.alloc(nk));
+    SB_TRY(rho.alloc(n));
+    SB_TRY(rs.alloc(n));
+    SB_TRY(sigma.alloc(n));
+    SB_TRY(flags.alloc(2));
+    SB_TRY(cnt.alloc(1));
+    SB_CUDA(cudaMemsetAsync(flags.p, 0, 2 * sizeof(int), ctx->stream));
+    SB_CUDA(cudaMemsetAsync(cnt.p, 0, sizeof(ull), ctx->stream));
+    if (n) {
+        k_um_dist<<<um_grid(ctx, nk, 256), 256, 0, ctx->stream>>>(X, R, n_ref, nbr, n, dim, k, 1, d.p, flags.p);
+        k_um_smooth<<<um_grid(ctx, n, 128), 128, 0, ctx->stream>>>(d.p, nbr, n, k, std::log2((double)k), 1, rho.p, sigma.p, rs.p, flags.p + 1, cnt.p);
+        count_launch(ctx);
+        count_launch(ctx);
+        SB_CUDA(cudaGetLastError());
+    }
+    int hf[2];
+    SB_CUDA(cudaMemcpyAsync(hf, flags.p, 2 * sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
+    SB_CUDA(cudaStreamSynchronize(ctx->stream));
+    SB_TRY(agree_status(ctx, ut_err(hf[0], fn), fn));
+    // the global floor: the row sums of all ranks in global row order, summed left to right; sum m by the integer all-reduce
+    std::vector<double> mine(n), all;
+    if (n) SB_CUDA(cudaMemcpyAsync(mine.data(), rs.p, n * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+    SB_CUDA(cudaStreamSynchronize(ctx->stream));
+    SB_TRY(gather_cells(ctx, mine, all));
+    SB_TRY(comm_allreduce_u64(ctx, (u64 *)cnt.p, 1));
+    ull hc = 0;
+    SB_CUDA(cudaMemcpyAsync(&hc, cnt.p, sizeof(ull), cudaMemcpyDeviceToHost, ctx->stream));
+    SB_CUDA(cudaStreamSynchronize(ctx->stream));
+    double tot = 0.0;
+    for (double v : all) tot += v;
+    if (n) {
+        k_um_global_floor<<<um_grid(ctx, n, 256), 256, 0, ctx->stream>>>(rho.p, sigma.p, n, 1e-3 * (tot / (double)hc));
+        k_um_member<<<um_grid(ctx, nk, 256), 256, 0, ctx->stream>>>(d.p, nbr, n, k, rho.p, sigma.p, w.p, nullptr, nullptr);
+        count_launch(ctx);
+        count_launch(ctx);
+        SB_CUDA(cudaGetLastError());
+    }
+    SB_CUDA(cudaStreamSynchronize(ctx->stream));
+    return SB_OK;
+}
+
+// the start and the epochs from the reference embedding (host, checked) and the query rows' nbr and w on the device -> host out
+static int ut_layout(sb_ctx *ctx, const double *ref_embedding, u64 n_ref, const u32 *nbr, const double *w, u64 n, u32 k, const UmOpts &o,
+                     double *out, sb_umap_info *info, const char *fn) {
+    TraceScope tr(ctx, "umap transform: start");
+    const u32 nc = o.nc;
+    DevBuf<double> dA;
+    DevBuf<i64> E, Y;
+    DevBuf<ull> mx;
+    DevBuf<int> err;
+    SB_TRY(dA.alloc(n_ref * nc));
+    SB_TRY(E.alloc(n_ref * nc));
+    SB_TRY(Y.alloc(n * nc));
+    SB_TRY(mx.alloc(3));
+    SB_TRY(err.alloc(1));
+    SB_CUDA(cudaMemsetAsync(mx.p, 0, 3 * sizeof(ull), ctx->stream));
+    SB_CUDA(cudaMemsetAsync(err.p, 0, sizeof(int), ctx->stream));
+    SB_CUDA(cudaMemcpyAsync(dA.p, ref_embedding, n_ref * nc * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+    k_um_init<<<um_grid(ctx, n_ref * nc, 256), 256, 0, ctx->stream>>>(dA.p, n_ref, nc, nc, 2, nullptr, nullptr, 0, E.p);
+    count_launch(ctx);
+    if (n) {
+        k_ut_start<<<um_grid(ctx, n, 128), 128, 0, ctx->stream>>>(nbr, w, n, k, nc, E.p, Y.p, mx.p, err.p);
+        count_launch(ctx);
+    }
+    SB_CUDA(cudaGetLastError());
+    ull hm[2];
+    int herr = 0;
+    SB_CUDA(cudaMemcpyAsync(hm, mx.p, 2 * sizeof(ull), cudaMemcpyDeviceToHost, ctx->stream));
+    SB_CUDA(cudaMemcpyAsync(&herr, err.p, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
+    SB_CUDA(cudaStreamSynchronize(ctx->stream));
+    dA.release();
+    SB_TRY(agree_status(ctx, ut_err(herr, fn), fn));
+    // the global quantities: the query count and this rank's first row, w_max (max over the ranks) and the entries with w > 0
+    u64 n_global = 0, row0 = 0;
+    SB_TRY(ut_rows(ctx, n, k, n_global, row0, fn));
+    std::vector<u64> wm, pos;
+    SB_TRY(comm_allgather_u64_host(ctx, hm[0], wm));
+    SB_TRY(comm_allgather_u64_host(ctx, hm[1], pos));
+    u64 wbits = 0, n_pos = 0;
+    for (int r = 0; r < ctx->nranks; r++) {
+        wbits = std::max(wbits, wm[r]);
+        n_pos += pos[r];
+    }
+    double wmax;
+    memcpy(&wmax, &wbits, sizeof(double));
+    double a = o.a, b = o.b;
+    if (!(a > 0.0 && b > 0.0)) um_fit_ab(o.spread, o.min_dist, a, b);
+    const u32 n_epochs = o.n_epochs ? o.n_epochs / 3 : (n_global <= 10000 ? 100 : 30);
+    info->a = a;
+    info->b = b;
+    info->max_weight = wmax;
+    info->n_edges = n_pos;
+    info->n_edges_used = 0;
+    info->n_epochs = n_epochs;
+    if (n_epochs && n_global) {
+        // the most a point can move over all epochs: per epoch and entry one attractive and at most 2 rate + 2 negative
+        // contributions, each at most 4 alpha <= learning_rate, rounded
+        const double bound = (double)n_epochs * k * (2.0 * o.rate + 4.0) * (o.lr * UM_FIX + 1.0);
+        if (!(bound < 4611686018427387904.0))
+            return sb_fail(SB_ERR_UNSUPPORTED, "%s: the epochs could move a point by 2^62 units of 2^-32 (k %u, %u epochs, learning_rate %g)", fn, k,
+                           n_epochs, o.lr);
+        TraceScope te(ctx, "umap transform: epochs");
+        DevBuf<double> ens, enn;
+        SB_TRY(ens.alloc(n * k));
+        SB_TRY(enn.alloc(n * k));
+        UtArgs p{nbr, w, E.p, Y.p, ens.p, enn.p, mx.p + 2, n, n_ref, row0, k, n_epochs, wmax, wmax / (double)n_epochs, (double)o.rate, a, b,
+                 b - 1.0, -2.0 * a * b, 2.0 * o.gamma * b, o.lr / 4.0, um_mix64(o.seed), o.rate > 0};
+        if (n) {
+            switch (nc) {
+                case 1: ut_launch_layout<1>(ctx, p); break;
+                case 2: ut_launch_layout<2>(ctx, p); break;
+                case 3: ut_launch_layout<3>(ctx, p); break;
+                case 4: ut_launch_layout<4>(ctx, p); break;
+                case 5: ut_launch_layout<5>(ctx, p); break;
+                case 6: ut_launch_layout<6>(ctx, p); break;
+                case 7: ut_launch_layout<7>(ctx, p); break;
+                default: ut_launch_layout<8>(ctx, p); break;
+            }
+            count_launch(ctx);
+            SB_CUDA(cudaGetLastError());
+        }
+        ull used = 0;
+        SB_CUDA(cudaMemcpyAsync(&used, mx.p + 2, sizeof(ull), cudaMemcpyDeviceToHost, ctx->stream));
+        SB_CUDA(cudaStreamSynchronize(ctx->stream));
+        std::vector<u64> us;
+        SB_TRY(comm_allgather_u64_host(ctx, used, us));
+        for (u64 v : us) info->n_edges_used += v;
+    }
+    return um_copy_out(ctx, Y, 0, n, nc, out);
+}
+
+extern "C" int sb_umap_transform_graph(sb_ctx *ctx, const double *ref_scores, uint64_t n_ref, const double *scores, const uint32_t *nbr, uint64_t n,
+                                       uint32_t dim, uint32_t k, const sb_umap_opts *opts, double *weights, double *sigma) {
+    const char *fn = "sb_umap_transform_graph";
+    if (!ctx) return sb_fail(SB_ERR_INVALID_ARG, "%s: NULL argument", fn);
+    UmOpts o;
+    int rc = (!ref_scores || (n && (!scores || !nbr || !weights))) ? sb_fail(SB_ERR_INVALID_ARG, "%s: NULL argument", fn) : SB_OK;
+    if (rc == SB_OK && dim == 0) rc = sb_fail(SB_ERR_INVALID_ARG, "%s: dim must be >= 1", fn);
+    if (rc == SB_OK) rc = ut_args(opts, n_ref, n, k, o, fn);
+    SB_ENTER(ctx);
+    SB_TRY(agree_status(ctx, rc, fn));
+    DevBuf<double> dR, dX, w, s;
+    DevBuf<u32> dn;
+    SB_TRY(dR.alloc(n_ref * dim));
+    SB_TRY(dX.alloc(n * dim));
+    SB_TRY(dn.alloc(n * k));
+    SB_CUDA(cudaMemcpyAsync(dR.p, ref_scores, n_ref * dim * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+    if (n) {
+        SB_CUDA(cudaMemcpyAsync(dX.p, scores, n * dim * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+        SB_CUDA(cudaMemcpyAsync(dn.p, nbr, n * k * sizeof(u32), cudaMemcpyHostToDevice, ctx->stream));
+    }
+    SB_TRY(ut_graph(ctx, dR.p, n_ref, dX.p, dn.p, n, dim, k, w, s, fn));
+    if (n) {
+        SB_CUDA(cudaMemcpyAsync(weights, w.p, n * k * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+        if (sigma) SB_CUDA(cudaMemcpyAsync(sigma, s.p, n * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+    }
+    SB_CUDA(cudaStreamSynchronize(ctx->stream));
+    return SB_OK;
+}
+
+extern "C" int sb_umap_transform_layout(sb_ctx *ctx, const double *ref_embedding, uint64_t n_ref, const uint32_t *nbr, const double *weights, uint64_t n,
+                                        uint32_t k, const sb_umap_opts *opts, double *out, sb_umap_info *info) {
+    const char *fn = "sb_umap_transform_layout";
+    if (!ctx) return sb_fail(SB_ERR_INVALID_ARG, "%s: NULL argument", fn);
+    UmOpts o;
+    int rc = (!info || (n && (!nbr || !weights || !out))) ? sb_fail(SB_ERR_INVALID_ARG, "%s: NULL argument", fn) : SB_OK;
+    if (rc == SB_OK) rc = ut_args(opts, n_ref, n, k, o, fn);
+    if (rc == SB_OK) rc = ut_ref_embedding(ref_embedding, n_ref, o.nc, fn);
+    SB_ENTER(ctx);
+    SB_TRY(agree_status(ctx, rc, fn));
+    DevBuf<double> dw, d;
+    DevBuf<u32> dn;
+    DevBuf<int> err;
+    SB_TRY(dw.alloc(n * k));
+    SB_TRY(dn.alloc(n * k));
+    SB_TRY(d.alloc(n * k));
+    SB_TRY(err.alloc(1));
+    SB_CUDA(cudaMemsetAsync(err.p, 0, sizeof(int), ctx->stream));
+    if (n) {
+        SB_CUDA(cudaMemcpyAsync(dn.p, nbr, n * k * sizeof(u32), cudaMemcpyHostToDevice, ctx->stream));
+        SB_CUDA(cudaMemcpyAsync(dw.p, weights, n * k * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+        // the neighbour lists' checks of the graph step (dim 0: no distance is computed)
+        k_um_dist<<<um_grid(ctx, n * k, 256), 256, 0, ctx->stream>>>(nullptr, nullptr, n_ref, dn.p, n, 0, k, 1, d.p, err.p);
+        count_launch(ctx);
+        SB_CUDA(cudaGetLastError());
+    }
+    int herr = 0;
+    SB_CUDA(cudaMemcpyAsync(&herr, err.p, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
+    SB_CUDA(cudaStreamSynchronize(ctx->stream));
+    d.release();
+    SB_TRY(agree_status(ctx, ut_err(herr, fn), fn));
+    return ut_layout(ctx, ref_embedding, n_ref, dn.p, dw.p, n, k, o, out, info, fn);
+}
+
+extern "C" int sb_umap_transform(sb_ctx *ctx, const double *ref_scores, const double *ref_embedding, uint64_t n_ref, const double *scores,
+                                 const uint32_t *nbr, uint64_t n_local, uint32_t dim, uint32_t k, const sb_umap_opts *opts, double *out,
+                                 sb_umap_info *info) {
+    const char *fn = "sb_umap_transform";
+    if (!ctx) return sb_fail(SB_ERR_INVALID_ARG, "%s: NULL argument", fn);
+    UmOpts o;
+    int rc = (!ref_scores || !info || (n_local && (!scores || !nbr || !out))) ? sb_fail(SB_ERR_INVALID_ARG, "%s: NULL argument", fn) : SB_OK;
+    if (rc == SB_OK && dim == 0) rc = sb_fail(SB_ERR_INVALID_ARG, "%s: dim must be >= 1", fn);
+    if (rc == SB_OK) rc = ut_args(opts, n_ref, n_local, k, o, fn);
+    if (rc == SB_OK) rc = ut_ref_embedding(ref_embedding, n_ref, o.nc, fn);
+    SB_ENTER(ctx);
+    SB_TRY(agree_status(ctx, rc, fn));
+    const u64 n = n_local;
+    DevBuf<double> dR, dX, w, s;
+    DevBuf<u32> dn;
+    SB_TRY(dR.alloc(n_ref * dim));
+    SB_TRY(dX.alloc(n * dim));
+    SB_TRY(dn.alloc(n * k));
+    SB_CUDA(cudaMemcpyAsync(dR.p, ref_scores, n_ref * dim * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+    if (n) {
+        SB_CUDA(cudaMemcpyAsync(dX.p, scores, n * dim * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+        SB_CUDA(cudaMemcpyAsync(dn.p, nbr, n * k * sizeof(u32), cudaMemcpyHostToDevice, ctx->stream));
+    }
+    SB_TRY(ut_graph(ctx, dR.p, n_ref, dX.p, dn.p, n, dim, k, w, s, fn));
+    dR.release();
+    dX.release();
+    s.release();
+    return ut_layout(ctx, ref_embedding, n_ref, dn.p, w.p, n, k, o, out, info, fn);
 }

@@ -7,6 +7,12 @@ layout, made epoch-synchronous so that the embedding is bit-reproducible at ever
     nn = knn(ctx, scores, 90)                  # floor(3 perplexity) neighbours
     emb = tsne(ctx, scores, nn).embedding      # n x 2, f64
 
+New cells are placed into a fitted embedding without moving it (umap-learn's transform):
+
+    q = normalize_like(query_mat, reference_nmat).rdot(u.T).T   # query scores in the reference's PCA space (ref: v * d)
+    nn = find_nn(ctx, q, 16, ref_scores, include_self=True)    # k = umap-learn's n_neighbors (the fit's 15 + 1)
+    emb_q = umap_transform(ctx, ref_scores, emb, q, nn).embedding
+
 The default start is the first n_components columns of the scores scaled to [0, 10] (PCA init); umap-learn's spectral start is
 not offered.  On a sharded context every rank passes its own rows of the scores and of the kNN lists (find_nn(...,
 self_offset=its first cell)) and gets its own rows of the embedding."""
@@ -134,6 +140,68 @@ def umap(ctx, scores, nbr, options: UmapOptions | None = None, init=None) -> Uma
     info = SbUmapInfo()
     L.check(L.lib().sb_umap(ctx._h, L.vp(scores), L.vp(nbr), C.c_uint64(n), C.c_uint32(dim), C.c_uint32(k), C.byref(o),
                             None if init is None else L.vp(init), L.vp(out), C.byref(info)))
+    return _result(out[:n], info)
+
+
+# ---------------------------------------------------------------- UMAP transform (csrc/umap.cu)
+def _ref_inputs(ref, scores, nbr):
+    ref = np.ascontiguousarray(ref, dtype=np.float64)
+    scores, nbr = _inputs(scores, nbr)
+    if ref.ndim != 2 or ref.shape[1] != scores.shape[1]:
+        raise ValueError("ref_scores must be n_ref x dim, with the query scores' dim")
+    return ref, scores, nbr
+
+
+def _ref_embedding(ref_embedding, o: SbUmapOpts):
+    e = np.ascontiguousarray(ref_embedding, dtype=np.float64)
+    if e.ndim != 2 or e.shape[1] != o.n_components:
+        raise ValueError(f"ref_embedding must be n_ref x n_components ({o.n_components})")
+    return e
+
+
+def umap_transform_graph(ctx, ref_scores, scores, nbr, options: UmapOptions | None = None):
+    """The query rows' graph against the reference: scores [n x dim] and nbr [n x k] (reference indices, find_nn(ctx, scores, k,
+    ref_scores, include_self=True); k is umap-learn's n_neighbors) -> weights [n x k] (slot order), sigma [n]."""
+    ref, scores, nbr = _ref_inputs(ref_scores, scores, nbr)
+    (n, dim), k = scores.shape, nbr.shape[1]
+    o = _opts(options)
+    w, sigma = np.zeros((max(n, 1), k)), np.zeros(max(n, 1))
+    L.check(L.lib().sb_umap_transform_graph(ctx._h, L.vp(ref), C.c_uint64(ref.shape[0]), L.vp(scores), L.vp(nbr), C.c_uint64(n),
+                                            C.c_uint32(dim), C.c_uint32(k), C.byref(o), L.vp(w), L.vp(sigma)))
+    return w[:n], sigma[:n]
+
+
+def umap_transform_layout(ctx, ref_embedding, nbr, weights, options: UmapOptions | None = None) -> UmapResult:
+    """The start and the epochs of the query rows against the fixed reference embedding [n_ref x n_components]."""
+    o = _opts(options)
+    e = _ref_embedding(ref_embedding, o)
+    nbr = np.ascontiguousarray(nbr, dtype=np.uint32)
+    weights = np.ascontiguousarray(weights, dtype=np.float64)
+    if nbr.ndim != 2 or weights.shape != nbr.shape:
+        raise ValueError("nbr and weights must both be n x k")
+    n, k = nbr.shape
+    out = np.zeros((max(n, 1), o.n_components))
+    info = SbUmapInfo()
+    L.check(L.lib().sb_umap_transform_layout(ctx._h, L.vp(e), C.c_uint64(e.shape[0]), L.vp(nbr), L.vp(weights), C.c_uint64(n), C.c_uint32(k),
+                                             C.byref(o), L.vp(out), C.byref(info)))
+    return _result(out[:n], info)
+
+
+def umap_transform(ctx, ref_scores, ref_embedding, scores, nbr, options: UmapOptions | None = None) -> UmapResult:
+    """New points placed into a fitted embedding (umap-learn's transform; the reference does not move): the graph and the layout
+    with the weights kept on the device.  options: the fit's (n_components = the embedding's width; init and set_op_mix_ratio are
+    ignored; n_epochs = 0: 100 up to 10,000 query points, else 30, otherwise n_epochs // 3).  On a sharded context every rank
+    passes the whole reference and its own query rows, and gets its own rows back."""
+    ref, scores, nbr = _ref_inputs(ref_scores, scores, nbr)
+    (n, dim), k = scores.shape, nbr.shape[1]
+    o = _opts(options)
+    e = _ref_embedding(ref_embedding, o)
+    if e.shape[0] != ref.shape[0]:
+        raise ValueError("ref_scores and ref_embedding must have the same rows")
+    out = np.zeros((max(n, 1), o.n_components))
+    info = SbUmapInfo()
+    L.check(L.lib().sb_umap_transform(ctx._h, L.vp(ref), L.vp(e), C.c_uint64(ref.shape[0]), L.vp(scores), L.vp(nbr), C.c_uint64(n),
+                                      C.c_uint32(dim), C.c_uint32(k), C.byref(o), L.vp(out), C.byref(info)))
     return _result(out[:n], info)
 
 

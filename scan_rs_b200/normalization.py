@@ -81,6 +81,19 @@ def log_normalize(matrix, umi_count_sum, log_base):  # normalization.rs:119-129
     return log_normalize_with_size_factor(matrix, umi_count_sum, log_base, None)
 
 
+def normalize_like(query: AdaptiveMat, reference: LowRankOffset) -> LowRankOffset:
+    """The reference's normalization applied to the query's cells (sb_normalize_like): column scales target / total_c from the
+    query's own cell totals, the reference's log base, 1/sd row scales and -mean/sd offset.  The reference must be CellRanger,
+    CellRanger8, SeuratLog or log_normalize without size factors; the query must have the reference's genes in the same order
+    (AdaptiveMat.select_rows).  The result borrows the query, so the reference may be freed first.
+
+    Query scores in the reference's PCA space (u, d, v = BkSvd().run_pca(reference, k); the reference's own scores are v * d):
+        normalize_like(query, reference).rdot(u.T).T"""
+    h = C.c_void_p()
+    L.check(L.lib().sb_normalize_like(query._h, reference._h, C.byref(h)))
+    return LowRankOffset(query, h)
+
+
 def log1p_normalize_fixed_point(matrix: AdaptiveMat, log_base: LogBase, base: int, exponent: int) -> LowRankOffset:
     """normalization.rs:191-213 (FixedPointFormat { base, exponent })."""
     h = C.c_void_p()
