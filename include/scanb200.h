@@ -106,18 +106,20 @@ SB_API int sb_multi_size(const sb_multi *mm);
 SB_API int sb_multi_ctx(sb_multi *mm, int rank, sb_ctx **out);
 SB_API int sb_multi_run(sb_multi *mm, sb_rank_fn fn, void *user);
 SB_API void sb_multi_shutdown(sb_multi *mm);
-/* Options: "direct_projection" (0/1, default 0): 1 forces the wide projection pass T = Q^T A of
- * bk_svd.rs:102,131 to run as a sparse product; 0 lets the library use Q^T A = R^-T (K^T A) when R is usable.
+/* Options (a name not listed here is answered with SB_ERR_INVALID_ARG, "unknown option"):
+ * "direct_projection" (0/1, default 0): 1 forces the wide projection pass T = Q^T A of bk_svd.rs:102,131 to run as a sparse
+ * product; 0 lets the library use Q^T A = R^-T (K^T A) when R is usable.  "verify_projection" (default 0): 1 always checks that
+ * identity a posteriori (otherwise only when cond(R) > 1e9).
+ * "own_dense" (default 1): QR / Gram / projections on the library's own kernels; 0 = cuSOLVER / cuBLAS.  "gemm_skinny"
+ * (default 1), "eig_host" (default 1), "eig_jacobi" (default 0): choices of the dense steps (DESIGN.md).
  * "gather" (default 1): 1 = panelled gather kernels for the sparse halves of both products, 0 = the first-generation
- * cell-major / gene-major kernels (A/B and accuracy reference).  "dense_genes" (default 2048) / "dense_min_density"
- * (default 0.12): size of the dense hot-gene panel of matrices uploaded afterwards (0 disables it).
- * "upload_sync" (default 1): drain the build stream after every stage of a pipelined upload.
- * "overlap" / "overlap_t" (default 0): experimental concurrent sparse + panel kernels.
- * "dense_max_count" (default 15, 1..15): largest count kept in the dense panel of matrices uploaded afterwards.
- * "gather_split" (default 0): EXPERIMENTAL separate 4-byte stream for the sparse entries with a count of 1 (gather_split.cu);
- * written without hardware access, off until validated.
- * "panel_i8" (default 0): EXPERIMENTAL tcgen05 int8 contraction of the T-side panel (needs dense_max_count <= 3, a
- * 2,048-gene panel and width <= 20); written without hardware access, off until validated. */
+ * cell-major / gene-major kernels (accuracy reference).  "gather_defer" (default 1), "gather_calibrate" (default 1, 0..8),
+ * "gather_items_per_cta" (default 1, 1..64), "gather_seg_cost" (default 0), "gather_flush_cost" (default 5): the T-side gather.
+ * "plane_cap" (default 12288): most gene ranks the bit planes of matrices built afterwards may cover; below 128 no planes
+ * are built and every entry stays sparse.  "plane_levels" (default 6, 1..6), "plane_min_density" (default 0.01) and
+ * "plane_items_per_cta" (default 48, 1..256): the rest of the plane layout of matrices built afterwards.
+ * "upload_chunks" (default 8, 1..256) / "upload_sync" (default 1): chunks of a pipelined upload, and whether the build
+ * stream is drained after every stage.  "block_cache_gb" (default: half the device memory): the exact-size block cache. */
 SB_API int sb_set_option(sb_ctx *ctx, const char *name, double value);
 
 /* Page-locked host memory for inputs / outputs (optional): copies to and from pinned buffers run at PCIe

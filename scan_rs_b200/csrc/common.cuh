@@ -140,27 +140,12 @@ struct sb_ctx {
     cudaStream_t stream = nullptr;
     cudaMemPool_t pool = nullptr;        // the context's own stream-ordered memory pool (nothing is changed on the device's default pool)
     cudaStream_t copy_stream = nullptr;  // host -> device copies of the pipelined upload
-    cudaStream_t aux_stream = nullptr;   // the dense panel kernels when overlapped with the sparse kernels
-    cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
-    // Experimental (default off, measured slower -- DESIGN.md 3): run the sparse and the DMMA panel kernel of a product on two
-    // streams with CTAs of both resident on every SM.
-    bool overlap = false;    // A.X
-    bool overlap_t = false;  // A^T.Y
     cublasHandle_t cublas = nullptr;
     cusolverDnHandle_t cusolver = nullptr;
     ncclComm_t comm = nullptr;
     int nranks = 1, rank = 0;
-    int dense_cap = 2048;            // max genes in the dense hot panel (0 disables the hybrid layout)
-    double dense_min_density = 0.12; // a gene joins the panel only if nnz/n_global is at least this
-    bool panel_i8 = false;           // EXPERIMENTAL (panel_i8.cu): T-side dense panel on tcgen05 int8 instead of FP64 mma.sync
-    int dense_max_count = 15;        // largest count kept in the dense panel of matrices uploaded afterwards (<= 15)
-    // dense half of the hybrid layout of matrices built afterwards: 0 none, 1 u8 panel on the FP64 mma.sync path (dense_panel.cu),
-    // 2 bit planes on the int8 tensor cores (planes.cu)
-    int panel_mode = 2;
-    int pl_debug = 0;                // timing experiments only (planes.cu): 1 no output reductions, 2 no epilogue arithmetic, 4 no tile expansion
-    int pl_variant = 3;              // kernel generations of planes.cu (A/B): bit 0 T side (warp layout, paired stages), bit 1 N side (bulk-copied digit rows, 12 producers)
     int plane_items_per_cta = 48;    // T-side plane kernel: work items per CTA on its queue (tail length vs boundary cost)
-    int plane_cap = 12288;           // most ranks a plane may cover
+    int plane_cap = 12288;           // most ranks a plane may cover (< 128: no planes, every entry of matrices built afterwards sparse)
     int plane_levels = 6;            // most count levels kept as planes (<= PL_MAX_LEVELS)
     double plane_min_density = 0.01; // a 128-rank block joins level k only if this fraction of the cells has exactly that count
     bool gemm_skinny = true;         // tall products with at most 16 output columns: row-per-thread kernel instead of the 128-column MMA tiles
@@ -275,16 +260,14 @@ struct sb_mat {
     DevBuf<uint2> gm;
     DevBuf<u64> gm_base;
     DevBuf<u64> unit_ptr;
-    bool have_full_gm = false;  // gm / gm_base above cover ALL entries; built lazily when a dense panel exists
-    // Hybrid layout (log-normalization maps only): the `gd` most expressed genes live in a dense u8 panel
-    // D[n x gd] (counts 1..SB_DENSE_MAX_COUNT, 0 elsewhere); every other entry -- cold genes and the rare larger
-    // counts of hot genes -- stays in the sparse `cold_*` pair of layouts (same formats as cm / gm).
+    bool have_full_gm = false;  // gm / gm_base above cover ALL entries; built lazily when planes exist
+    // Hybrid layout (log-normalization maps only): the entries with a count k of the G_k most expressed genes (rank < G_k,
+    // k = 1 .. L) live in the bit planes `pl`; every other entry -- cold genes and the counts above a gene's top plane level --
+    // stays in the sparse `cold_*` pair of layouts (same formats as cm / gm).  gd = G_1, the ranks of level 1 (0: no planes).
     u32 gd = 0;
-    u32 dense_max_count = 15;  // counts 1..dense_max_count live in D
-    DevBuf<unsigned char> D;
-    DevBuf<u32> hot_idx;      // [gd] gene id of panel column j
-    DevBuf<u32> hot_of_gene;  // [m] panel column of a gene or 0xFFFFFFFF
-    PlaneSet pl;  // panel_mode 2: bit planes instead of D (gd = ranks of level 1; hot_idx / hot_of_gene are in rank order)
+    DevBuf<u32> hot_idx;      // [gd] gene id of rank r
+    DevBuf<u32> hot_of_gene;  // [m] rank of a gene or 0xFFFFFFFF
+    PlaneSet pl;
     u64 cold_nnz = 0;
     DevBuf<u64> cold_cm_ptr;
     DevBuf<uint2> cold_cm;
@@ -302,8 +285,6 @@ struct sb_mat {
     DevBuf<u32> cell_tot;
     bool have_cell_tot = false;
 };
-#define SB_DENSE_MAX_COUNT 15u
-#define SB_DENSE_LUT 16
 
 // device view of the per-nonzero map (sqz/src/matrix_map.rs): see MapDev in map.cuh
 struct sb_nmat {

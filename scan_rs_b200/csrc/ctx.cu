@@ -166,9 +166,6 @@ extern "C" int sb_init(int device, sb_ctx **out) {
     SB_CUBLAS(cublasSetStream(ctx->cublas, ctx->stream));
     SB_CUSOLVER(cusolverDnCreate(&ctx->cusolver));
     SB_CUSOLVER(cusolverDnSetStream(ctx->cusolver, ctx->stream));
-    SB_CUDA(cudaStreamCreateWithFlags(&ctx->aux_stream, cudaStreamNonBlocking));
-    SB_CUDA(cudaEventCreateWithFlags(&ctx->ev_fork, cudaEventDisableTiming));
-    SB_CUDA(cudaEventCreateWithFlags(&ctx->ev_join, cudaEventDisableTiming));
     SB_CUDA(cudaEventCreate(&ctx->t0));
     SB_CUDA(cudaEventCreate(&ctx->t1));
     SB_CUDA(cudaMallocHost(&ctx->pinned, 4096));
@@ -201,12 +198,6 @@ extern "C" void sb_shutdown(sb_ctx *ctx) {
     cudaStreamSynchronize(ctx->stream);
 
     if (ctx->copy_stream) cudaStreamDestroy(ctx->copy_stream);
-    if (ctx->aux_stream) {
-        cudaStreamSynchronize(ctx->aux_stream);
-        cudaStreamDestroy(ctx->aux_stream);
-    }
-    if (ctx->ev_fork) cudaEventDestroy(ctx->ev_fork);
-    if (ctx->ev_join) cudaEventDestroy(ctx->ev_join);
     if (ctx->stream) {
         sb_stream_register(ctx->stream, false);
         cudaStreamDestroy(ctx->stream);
@@ -240,43 +231,12 @@ extern "C" int sb_set_option(sb_ctx *ctx, const char *name, double value) {
         ctx->own_dense = value != 0.0;
         return SB_OK;
     }
-    if (!strcmp(name, "overlap")) {  // A.X: run the sparse and the dense-panel kernel concurrently
-        ctx->overlap = value != 0.0;
-        return SB_OK;
-    }
-    if (!strcmp(name, "overlap_t")) {  // same for A^T.Y
-        ctx->overlap_t = value != 0.0;
-        return SB_OK;
-    }
-    if (!strcmp(name, "panel_i8")) {  // experimental, see panel_i8.cu
-        ctx->panel_i8 = value != 0.0;
-        return SB_OK;
-    }
-    if (!strcmp(name, "dense_max_count")) {  // applies to matrices uploaded afterwards
-        if (value < 1 || value > 15) return sb_fail(SB_ERR_INVALID_ARG, "sb_set_option: dense_max_count must be 1..15");
-        ctx->dense_max_count = (int)value;
-        return SB_OK;
-    }
     if (!strcmp(name, "upload_sync")) {
         ctx->upload_sync = value != 0.0;
         return SB_OK;
     }
     if (!strcmp(name, "gather")) {  // 1 (default): panelled gather kernels; 0: first-generation sparse kernels
         ctx->use_gather = value != 0.0;
-        return SB_OK;
-    }
-    if (!strcmp(name, "dense_genes")) {  // applies to matrices uploaded afterwards
-        ctx->dense_cap = value < 0 ? 0 : (int)value;
-        return SB_OK;
-    }
-    if (!strcmp(name, "dense_min_density")) {
-        ctx->dense_min_density = value;
-        return SB_OK;
-    }
-    // dense half of matrices built afterwards: 0 none, 1 u8 panel / FP64 mma.sync (dense_panel.cu), 2 bit planes / int8 tcgen05 (planes.cu)
-    if (!strcmp(name, "panel_mode")) {
-        if (value != 0.0 && value != 1.0 && value != 2.0) return sb_fail(SB_ERR_INVALID_ARG, "sb_set_option: panel_mode must be 0, 1 or 2");
-        ctx->panel_mode = (int)value;
         return SB_OK;
     }
     if (!strcmp(name, "gather_items_per_cta")) {  // applies to matrices built afterwards
@@ -329,15 +289,7 @@ extern "C" int sb_set_option(sb_ctx *ctx, const char *name, double value) {
         ctx->plane_items_per_cta = (int)value;
         return SB_OK;
     }
-    if (!strcmp(name, "pl_variant")) {
-        ctx->pl_variant = (int)value;
-        return SB_OK;
-    }
-    if (!strcmp(name, "pl_debug")) {  // timing experiments: results are wrong on purpose
-        ctx->pl_debug = (int)value;
-        return SB_OK;
-    }
-    if (!strcmp(name, "plane_cap")) {
+    if (!strcmp(name, "plane_cap")) {  // applies to matrices built afterwards; < 128: no planes
         ctx->plane_cap = value < 0 ? 0 : (int)value;
         return SB_OK;
     }

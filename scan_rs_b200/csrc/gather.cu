@@ -1,5 +1,5 @@
 // gather.cu -- the panelled sparse gather behind both products of the Krylov loop (the cold half of the
-// hybrid layout, or every entry when a matrix has no dense panel).
+// hybrid layout, or every entry when a matrix has no planes).
 //
 //   N side (K8)  P[g,:] += sum_c x_gc * X[c,:]      restates low_rank_offset.rs:68-81 -> mat.rs:1074-1090 -> prod.rs:30-51,87-148
 //       stream: cell panels of `rows` cells, inside a panel sorted by (gene, cell); entry {gene | cell_local << 22, count}
@@ -260,7 +260,7 @@ k_gather(const uint2 *__restrict__ ent, const GUnit *__restrict__ units, const u
     }
 }
 
-// out[c, j] = v_c * uy[j] (or 0): the rank-1 offset of A^T.Y; the dense panel kernel and the gather add on top
+// out[c, j] = v_c * uy[j] (or 0): the rank-1 offset of A^T.Y; the plane kernels and the gather add on top
 __global__ void k_t_init(double *__restrict__ out, u64 n, u32 w, u32 ldo, const double *__restrict__ uy, const double *__restrict__ v) {
     const u64 total = n * w;
     for (u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (u64)gridDim.x * blockDim.x) {

@@ -394,112 +394,24 @@ int mat_ensure_full_gm(sb_mat *mt) {
     return SB_OK;
 }
 
-// splits the cell-major stream into the dense panel D and the cold sparse entries (count / fill passes).
-// ptr / D are already offset to the first cell of the range; new_ptr and out are range-local.
-__global__ void k_split_hot(const u64 *__restrict__ ptr, const uint2 *__restrict__ cm, u64 n, const u32 *__restrict__ hot_of_gene, u32 gd,
-                            u32 max_count, const u64 *__restrict__ new_ptr, u32 *__restrict__ counts, uint2 *__restrict__ out,
-                            unsigned char *__restrict__ D) {
-    u64 warp = ((u64)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-    u64 nwarps = ((u64)gridDim.x * blockDim.x) >> 5;
-    int lane = threadIdx.x & 31;
-    for (u64 c = warp; c < n; c += nwarps) {
-        u64 s = ptr[c], e = ptr[c + 1];
-        u64 wpos = new_ptr ? new_ptr[c] : 0;
-        u32 total = 0;
-        for (u64 k0 = s; k0 < e; k0 += 32) {
-            u64 k = k0 + lane;
-            bool valid = k < e;
-            uint2 z = valid ? cm[k] : make_uint2(0, 0);
-            u32 h = valid ? hot_of_gene[z.x] : 0xFFFFFFFFu;
-            bool dense = valid && h != 0xFFFFFFFFu && z.y <= max_count;
-            bool cold = valid && !dense;
-            if (D && dense) D[c * (u64)gd + h] = (unsigned char)z.y;
-            unsigned mask = __ballot_sync(0xffffffffu, cold);
-            if (out && cold) out[wpos + total + __popc(mask & ((1u << lane) - 1u))] = z;
-            total += __popc(mask);
-        }
-        if (counts && lane == 0) counts[c] = total;
-    }
-}
-
 __global__ void k_add_offset(const u64 *__restrict__ src, u64 n, u64 add, u64 *__restrict__ dst) {
     u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x;
     if (i < n) dst[i] = src[i] + add;
 }
 
-// Picks the hot genes from the non-zero counts of local cells [c0, c1) (the whole shard, or the first upload
-// chunk as a sample), summed over ranks: most non-zeros first, at least dense_min_density of the sampled
-// cells, at most dense_cap, whole groups of 64.  Allocates and zeroes the panel.
-static int select_hot_genes(sb_mat *mt, u64 c0, u64 c1) {
-    sb_ctx *ctx = mt->ctx;
-    mt->gd = 0;
-    mt->pl.active = false;
-    if (ctx->panel_mode == 0) return SB_OK;
-    if (ctx->panel_mode == 2) return ctx->dense_cap >= 64 ? planes_select(mt, c0, c1) : SB_OK;  // sets gd = ranks of level 1 when planes are built
-    mt->dense_max_count = (u32)std::min(std::max(ctx->dense_max_count, 1), (int)SB_DENSE_MAX_COUNT);
-    if (ctx->dense_cap < 64 || mt->m < 64 || mt->n_global == 0) return SB_OK;
-    SyncScope tr(ctx, "build: hot gene selection");
-    DevBuf<u64> d_nnz;
-    SB_TRY(d_nnz.alloc((size_t)mt->m + 1));
-    SB_CUDA(cudaMemsetAsync(d_nnz.p, 0, ((size_t)mt->m + 1) * sizeof(u64), ctx->stream));
-    if (c1 > c0) {
-        ProfScope ps(ctx, PH_REDUCE);
-        k_gene_sums<<<grid_for((c1 - c0) * 32, 256, ctx, 16), 256, 0, ctx->stream>>>(mt->cm_ptr.p + c0, mt->cm.p, c1 - c0, 2, nullptr, nullptr,
-                                                                                    (unsigned long long *)d_nnz.p);
-        count_launch(ctx);
-    }
-    u64 sample = c1 - c0;
-    SB_CUDA(cudaMemcpyAsync(d_nnz.p + mt->m, &sample, sizeof(u64), cudaMemcpyHostToDevice, ctx->stream));
-    SB_TRY(comm_allreduce_u64(ctx, d_nnz.p, (size_t)mt->m + 1));
-    std::vector<u64> h((size_t)mt->m + 1);
-    SB_CUDA(cudaMemcpyAsync(h.data(), d_nnz.p, h.size() * sizeof(u64), cudaMemcpyDeviceToHost, ctx->stream));
-    SB_CUDA(cudaStreamSynchronize(ctx->stream));
-    if (h[mt->m] == 0) return SB_OK;
-    std::vector<u32> order(mt->m);
-    std::iota(order.begin(), order.end(), 0u);
-    std::stable_sort(order.begin(), order.end(), [&](u32 a, u32 b) { return h[a] > h[b]; });
-    u32 gd = 0;
-    double thr = ctx->dense_min_density * (double)h[mt->m];
-    while (gd < mt->m && gd < (u32)ctx->dense_cap && (double)h[order[gd]] >= thr && h[order[gd]] > 0) gd++;
-    gd &= ~63u;  // whole 64-gene groups: 16-byte aligned panel rows, full fragment tiles
-    if (gd == 0) return SB_OK;
-    std::vector<u32> hot(order.begin(), order.begin() + gd), hot_of(mt->m, 0xFFFFFFFFu);
-    std::sort(hot.begin(), hot.end());  // panel columns in ascending gene order
-    for (u32 j = 0; j < gd; j++) hot_of[hot[j]] = j;
-    SB_TRY(mt->hot_idx.alloc(gd));
-    SB_TRY(mt->hot_of_gene.alloc(mt->m));
-    SB_CUDA(cudaMemcpyAsync(mt->hot_idx.p, hot.data(), gd * sizeof(u32), cudaMemcpyHostToDevice, ctx->stream));
-    SB_CUDA(cudaMemcpyAsync(mt->hot_of_gene.p, hot_of.data(), (size_t)mt->m * sizeof(u32), cudaMemcpyHostToDevice, ctx->stream));
-    SB_TRY(mt->D.alloc((size_t)mt->n * gd));
-    SB_CUDA(cudaMemsetAsync(mt->D.p, 0, std::max<size_t>(1, (size_t)mt->n * gd), ctx->stream));
-    SB_CUDA(cudaStreamSynchronize(ctx->stream));  // hot / hot_of are host temporaries
-    mt->gd = gd;
-    return SB_OK;
-}
-
-// dense / cold split of local cells [c0, c1): fills their panel rows, returns the range-local cold pair
+// plane / cold split of local cells [c0, c1): sets their plane bits, returns the range-local cold pair
 static int split_range(sb_mat *mt, u64 c0, u64 c1, DevBuf<u64> &ptr_local, DevBuf<uint2> &cold, u64 *cold_nnz) {
     sb_ctx *ctx = mt->ctx;
     const u64 nc = c1 - c0;
     DevBuf<u32> counts;
     SB_TRY(counts.alloc(nc));
     SB_TRY(ptr_local.alloc(nc + 1));
-    int grid = grid_for(nc * 32, 256, ctx, 16);
-    if (mt->pl.active) SB_TRY(planes_split_launch(mt, c0, nc, nullptr, counts.p, nullptr));
-    else if (nc) {
-        k_split_hot<<<grid, 256, 0, ctx->stream>>>(mt->cm_ptr.p + c0, mt->cm.p, nc, mt->hot_of_gene.p, mt->gd, mt->dense_max_count, nullptr, counts.p, nullptr, nullptr);
-        count_launch(ctx);
-    }
+    SB_TRY(planes_split_launch(mt, c0, nc, nullptr, counts.p, nullptr));
     SB_TRY(exclusive_scan_u32_to_u64(ctx, counts.p, nc, ptr_local.p));
     SB_CUDA(cudaMemcpyAsync(cold_nnz, ptr_local.p + nc, sizeof(u64), cudaMemcpyDeviceToHost, ctx->stream));
     SB_CUDA(cudaStreamSynchronize(ctx->stream));
     SB_TRY(cold.alloc(*cold_nnz));
-    if (mt->pl.active) SB_TRY(planes_split_launch(mt, c0, nc, ptr_local.p, nullptr, cold.p));
-    else if (nc) {
-        k_split_hot<<<grid, 256, 0, ctx->stream>>>(mt->cm_ptr.p + c0, mt->cm.p, nc, mt->hot_of_gene.p, mt->gd, mt->dense_max_count, ptr_local.p, nullptr, cold.p,
-                                                   mt->D.p + c0 * (u64)mt->gd);
-        count_launch(ctx);
-    }
+    SB_TRY(planes_split_launch(mt, c0, nc, ptr_local.p, nullptr, cold.p));
     return SB_OK;
 }
 
@@ -507,7 +419,7 @@ static int split_range(sb_mat *mt, u64 c0, u64 c1, DevBuf<u64> &ptr_local, DevBu
 static int build_hybrid(sb_mat *mt) {
     sb_ctx *ctx = mt->ctx;
     SyncScope tr(ctx, "build: hybrid total");
-    SB_TRY(select_hot_genes(mt, 0, mt->n));
+    SB_TRY(planes_select(mt, 0, mt->n));
     if (mt->gd == 0) return SB_OK;
     {
         SyncScope t4(ctx, "build: split hot/cold");
@@ -683,8 +595,8 @@ static int packed_status(sb_ctx *ctx, const HostEntries &he, DevEntries &de) {
 }
 
 // Cell-major upload as a pipeline: the host arrays are copied in chunks of whole cell panels on a second
-// stream while the library stream turns the previous chunk into the device layouts (interleave, dense /
-// cold split, per-chunk panel sort).  The hot genes are chosen from the first chunk (a sample of the cells).
+// stream while the library stream turns the previous chunk into the device layouts (interleave, plane /
+// cold split, per-chunk panel sort).  The planes are chosen from the first chunk (a sample of the cells).
 static int upload_pipelined(sb_mat *mt, const u64 *h_indptr, const HostEntries &he, DevEntries &de, u32 *d_max) {
     sb_ctx *ctx = mt->ctx;
     const u64 n = mt->n;
@@ -739,7 +651,7 @@ static int upload_pipelined(sb_mat *mt, const u64 *h_indptr, const HostEntries &
                 rc = sb_fail(SB_ERR_INVALID_ARG, "sb_upload: index %u out of range %u", hmax, mt->m);
             if (rc == SB_OK) rc = packed_status(ctx, he, de);
         }
-        if (rc == SB_OK && i == 0) rc = select_hot_genes(mt, c0, c1);
+        if (rc == SB_OK && i == 0) rc = planes_select(mt, c0, c1);
         if (rc == SB_OK && mt->gd > 0) {
             {
                 SyncScope t1(ctx, "chunk: split hot/cold");
@@ -854,7 +766,7 @@ static int upload_impl(sb_ctx *ctx, int major, uint32_t m, uint64_t n_local, con
     if (pipelined) {
         SB_CUDA(cudaMemcpyAsync(d_ptr.p, indptr, (nvec + 1) * sizeof(u64), cudaMemcpyHostToDevice, ctx->stream));
         // private flags {pointer check, largest index}: the context scratch is also the staging buffer of the collectives
-        // that set_global_shape / select_hot_genes run on a sharded context
+        // that set_global_shape / planes_select run on a sharded context
         DevBuf<int> flags;
         SB_TRY(flags.alloc(64));
         void *scr0 = flags.p;

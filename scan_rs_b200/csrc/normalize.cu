@@ -10,7 +10,7 @@ int mat_median_total(sb_mat *mat, u32 *median, int *nonempty);
 int mat_gene_sums_dev(sb_mat *mat, int mode, const unsigned char *excl_cells, const unsigned char *excl_genes, u64 *d_out, bool allreduce);
 int spmm_t(sb_nmat *a, const double *Y, u32 ldy, u32 w, double *out, u32 ldo, double *uy_scratch);
 int spmm_n(sb_nmat *a, const double *X, u32 ldx, u32 w, double *P, u32 ldp);
-int dense_moments(sb_nmat *a, double *S1, double *S2);
+int planes_moments(sb_nmat *a, double *S1, double *S2);
 int mat_ensure_full_gm(sb_mat *mt);
 
 #define FULLMASK 0xffffffffu
@@ -132,7 +132,7 @@ int nmat_moments(sb_nmat *a, double *S /* 2m */) {
             k_moments<<<grid, 256, 0, ctx->stream>>>(gm, gm_base, mt->np, mt->pc, a->log_base, a->col_scale.p, S, S + mt->m);
             count_launch(ctx);
         }
-        if (hybrid) SB_TRY(dense_moments(a, S, S + mt->m));
+        if (hybrid) SB_TRY(planes_moments(a, S, S + mt->m));
         SB_CUDA(cudaGetLastError());
     }
     SB_TRY(comm_allreduce_f64(ctx, S, 2 * (size_t)mt->m));

@@ -7,8 +7,8 @@
 // with L_c(k) = log_b(col_scale_c * k + 1) the only cell-dependent factor (map.cuh).  The dense f64 operand is cut per column
 // into 7 balanced base-256 digits of a 54-bit fixed-point number (Ozaki splitting): every M_k . digit-plane product is an
 // EXACT int8 x int8 -> int32 tensor-core product, and the digits are recombined in the epilogue (two int64 halves -> f64,
-// one rounding).  The error is that of one rounding to 54 bits of the column maximum per operand entry -- measured against
-// the oracle at the same level as the f64 DMMA panel it replaces (tests/test_gpu_parity.py).
+// one rounding).  The error is that of one rounding to 54 bits of the column maximum per operand entry (tests/test_spmm_kernels_gpu.py
+// bounds it entry by entry; tests/test_gpu_parity.py checks the products against the oracle).
 //
 // Layout ("bit planes"): genes are ranked by how many cells express them; level k keeps the first G_k ranks (multiples of
 // 128, G_1 >= G_2 >= ...), chosen so that a (gene, level) pair lives here only if at least `plane_min_density` of the cells
@@ -16,13 +16,15 @@
 // cell 128 tile + cell, stored at ((tile * G_k/32) + gw) * 128 + cell -- both products read 128-cell x 32-gene blocks as
 // 512 contiguous bytes.  Every entry not covered by a plane stays in the sparse streams (gather.cu).
 //
-// Kernels (one CTA per SM, warp-specialised: warps 0-3 epilogue, warp 4 MMA issue, warps 5-12 producers):
+// Kernels (one persistent CTA per SM, warp-specialised):
 //   k_planes_t : a CTA keeps the digit planes of 1,024 ranks resident in shared memory as the B operand (K-major, 144 KB),
 //                walks cell tiles; producers expand plane words into 0/1 int8 A tiles (K-major core matrices) through an
 //                8-stage mbarrier ring; up to three levels accumulate into three TMEM accumulators (3 x 144 columns).
+//                Warps 0-7 epilogue, 8 MMA issue, 9 item scheduler, 10-17 producers.
 //   k_planes_n : a CTA owns 384 ranks (three 128-gene accumulators) and a range of cell tiles; per 32-cell K step and level
-//                the producers expand the plane words into an MN-major A tile and copy the digit rows of L_c(k).X[c,:]
-//                (written once per product by k_pl_digits_n) as the MN-major B tile; all levels share the accumulators.
+//                the producers expand the plane words into an MN-major A tile and start a bulk copy of the digit rows of
+//                L_c(k).X[c,:] (written once per product by k_pl_digits_n) as the MN-major B tile; all levels share the
+//                accumulators.  Warps 0-3 epilogue, 4 MMA issue, 5-16 producers.
 #include <numeric>
 
 #include "common.cuh"
@@ -47,10 +49,12 @@ using namespace tc05;
 #define PT_SUB 2u                               // sub-stages per MMA stage: 128 genes, four MMAs per barrier round trip
 #define PT_NSTG (PT_NSTAGES / PT_SUB)
 #define PT_PROD_WARPS PT_NSTAGES
-#define PL_EPI_WARPS 4u
-#define PL_PROD_WARPS 8u
-#define PL_THREADS ((PL_EPI_WARPS + 1 + PL_PROD_WARPS) * 32)  // 416
+#define PT_EPI_WARPS 8u                         // two per TMEM lane quarter, ten columns each
+#define PT_WARPS (PT_EPI_WARPS + 1 + 1 + PT_PROD_WARPS)  // 18: epilogue, MMA issue, item scheduler, producers
 
+#define PL_EPI_WARPS 4u                         // N side
+#define PN_PROD_WARPS 12u
+#define PN_THREADS ((PL_EPI_WARPS + 1 + PN_PROD_WARPS) * 32)  // 544
 #define PN_GROUP 384u                           // ranks per CTA (N side): three M tiles
 #define PN_A_BYTES (3u * 4096u)
 #define PN_B_BYTES (32u * PL_NCOL)              // 4,608
@@ -130,10 +134,12 @@ static void units_round(std::vector<u32> &nctas, const std::vector<double> &cost
 }
 
 // Chooses the planes from the entry counts of local cells [c0, c1) (the whole shard or the first upload chunk), summed
-// over ranks.  Allocates and zeroes the planes, fills hot_idx (rank -> gene), hot_of_gene (gene -> rank) and the unit tables.
+// over ranks.  Allocates and zeroes the planes, fills hot_idx (rank -> gene), hot_of_gene (gene -> rank) and the unit tables,
+// and sets gd = G_1; gd stays 0 (no planes, every entry sparse) when no level clears the density bar or plane_cap < 128.
 int planes_select(sb_mat *mt, u64 c0, u64 c1) {
     sb_ctx *ctx = mt->ctx;
     PlaneSet &pl = mt->pl;
+    mt->gd = 0;
     pl.active = false;
     pl.L = 0;
     const u32 m = mt->m;
@@ -406,10 +412,10 @@ __global__ void k_pl_colmax_t(const double *__restrict__ Y, u32 ldy, const u32 *
     atomic_max_abs(&colmax_bits[c], v);
 }
 
-// Bd[range][k / 16][n / 8][n % 8][k % 16], k = rank % 1024, n = 7 c + s (digit s of column c); with `split` the second ten columns
-// start at accumulator column 72 (a multiple of 8) so that each half of the epilogue warps reads its own aligned 72-column range
+// Bd[range][k / 16][n / 8][n % 8][k % 16], k = rank % 1024, n = 7 c + s (digit s of column c); the second ten columns start at
+// accumulator column 72 (a multiple of 8) so that each half of the epilogue warps reads its own aligned 72-column range
 __global__ void k_pl_digits_t(const double *__restrict__ Y, u32 ldy, const u32 *__restrict__ hot_idx, const double *__restrict__ rs, u32 G1, u32 col0,
-                              u32 wt, const int *__restrict__ ex, signed char *__restrict__ Bd, u32 split) {
+                              u32 wt, const int *__restrict__ ex, signed char *__restrict__ Bd) {
     const u32 i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= G1 * PL_COLS) return;
     const u32 r = i / PL_COLS, c = i - r * PL_COLS;
@@ -423,7 +429,7 @@ __global__ void k_pl_digits_t(const double *__restrict__ Y, u32 ldy, const u32 *
     signed char *base = Bd + (size_t)range * PT_B_BYTES + (size_t)(k >> 4) * PT_KCHUNK_BYTES + (k & 15);
 #pragma unroll
     for (u32 s = 0; s < PL_DIG; s++) {
-        const u32 n = c * PL_DIG + s + ((split && c >= PL_COLS / 2) ? 2u : 0u);
+        const u32 n = c * PL_DIG + s + (c >= PL_COLS / 2 ? 2u : 0u);
         base[(size_t)(n >> 3) * 128 + (n & 7) * 16] = d[s];
     }
 }
@@ -455,30 +461,6 @@ __device__ __forceinline__ void read_acc(u32 taddr, double (&val)[PL_COLS]) {
                 else if (s == 4) hi = d;
                 else hi = fma(d, (double)(1u << (8 * (s - 4))), hi);
                 if (s == PL_DIG - 1) val[c] = fma(hi, 4294967296.0, lo);
-            }
-        }
-    }
-}
-
-// res[c] += lk * value_c, straight from the accumulator (keeps the epilogue's register footprint small)
-__device__ __forceinline__ void read_acc_fma(u32 taddr, double lk, double (&res)[PL_COLS]) {
-    double lo = 0.0, hi = 0.0;
-#pragma unroll
-    for (u32 cb = 0; cb < PL_NCOL; cb += 16) {
-        u32 r[16];
-        tmem_ld16(taddr + cb, r);
-        tmem_ld_wait();
-#pragma unroll
-        for (u32 i = 0; i < 16; i++) {
-            const u32 n = cb + i;  // compile-time after unrolling
-            if (n < PL_COLS * PL_DIG) {
-                const u32 c = n / PL_DIG, s = n - c * PL_DIG;
-                const double d = i32_to_f64(r[i]);
-                if (s == 0) lo = d;
-                else if (s < 4) lo = fma(d, (double)(1u << (8 * s)), lo);
-                else if (s == 4) hi = d;
-                else hi = fma(d, (double)(1u << (8 * (s - 4))), hi);
-                if (s == PL_DIG - 1) res[c] = fma(lk, fma(hi, 4294967296.0, lo), res[c]);
             }
         }
     }
@@ -521,28 +503,18 @@ __device__ __forceinline__ void read_acc_fma_half(u32 taddr, double lk, double (
 }
 
 // ---------------------------------------------------------------- k_planes_t
-// Roles: warps 0-3 epilogue, warp 4 MMA issue, warps 5-20 producers, warp 21 scheduler.  The producers' refill latency
-// (expand one sub-stage after its slot was freed) against the MMA work in flight in the ring decides the throughput: sixteen
-// warps each own a 4 KB sub-slot (one MMA's A operand), four sub-slots make a stage.
-// Two generations of the kernel (A/B through the option pl_variant bit 0; profiles/planes_r02_findings.md).
-//   V = 0: warps 0-3 epilogue, 4 MMA issue, 5-12 producers, 13 item scheduler.
-//   V = 1: what ncu showed of V = 0 at 400k cells -- (1) 17 % of all warp samples sit in the reload of the resident B block at a
-//          unit change (a 21-iteration LDG -> STS loop per thread, one exposed L2 round trip each: ~16 us per change); (2) the four
-//          epilogue warps are busy 70 % of the time: 3,600 cycles per (tile, level) job, a single warp per scheduler working
-//          through nine dependent tcgen05.ld -> convert -> FMA chains, against 576-2,304 cycles of MMAs per job -- the epilogue,
-//          not the tensor pipe (32 % busy), paces the kernel.  So: the B block arrives by bulk asynchronous copies (cp.async.bulk,
-//          one thread, completion on an mbarrier); EIGHT epilogue warps, two per TMEM lane quarter (a warp may only touch lanes
-//          32 (warp % 4) ..), each owning ten of the twenty columns, with the TMEM loads of the next chunk in flight while the
-//          current one is recombined; descriptor low words carry the leading-byte-offset field so an MMA costs 7 issue slots
-//          instead of 11.  Warps: 0-7 epilogue, 8 MMA, 9 item scheduler, 10-17 producers.
-//          (Measured without effect and dropped: isolating the MMA warp on its scheduler, issuing two stages per election.)
-template <int V> struct PtLayout;
-template <> struct PtLayout<0> {
-    static constexpr u32 WARPS = PL_EPI_WARPS + 1 + PT_PROD_WARPS + 1, EPI = PL_EPI_WARPS;
-};
-template <> struct PtLayout<1> {
-    static constexpr u32 WARPS = 8 + 1 + 1 + PT_PROD_WARPS, EPI = 8;
-};
+// Roles: warps 0-7 epilogue, 8 MMA issue, 9 item scheduler, 10-17 producers.  The producers' refill latency (expand one
+// sub-stage after its slot was freed) against the MMA work in flight in the ring decides the throughput.
+// This is the second generation of the kernel (DESIGN.md 3).  What ncu showed of the first at 400k cells: (1) 17 % of all warp
+// samples sat in the reload of the resident B block at a unit change (a 21-iteration LDG -> STS loop per thread, one exposed L2
+// round trip each: ~16 us per change); (2) its four epilogue warps were busy 70 % of the time: 3,600 cycles per (tile, level)
+// job, a single warp per scheduler working through nine dependent tcgen05.ld -> convert -> FMA chains, against 576-2,304 cycles
+// of MMAs per job -- the epilogue, not the tensor pipe (32 % busy), paced the kernel.  So: the B block arrives by bulk
+// asynchronous copies (cp.async.bulk, one thread, completion on an mbarrier); EIGHT epilogue warps, two per TMEM lane quarter (a
+// warp may only touch lanes 32 (warp % 4) ..), each owning ten of the twenty columns, with the TMEM loads of the next chunk in
+// flight while the current one is recombined; descriptor low words carry the leading-byte-offset field so an MMA costs 7 issue
+// slots instead of 11.  (Measured without effect and dropped: isolating the MMA warp on its scheduler, issuing two stages per
+// election.)
 struct PtShared {
     unsigned long long full[PT_NSTG], empty[PT_NSTG], tfull[3], tempty[3], item_full[2], item_empty[2], bload;
     u32 tmem;
@@ -559,22 +531,20 @@ struct PtShared {
 // Output: the CTA's 20 values per (unit, cell) go to part[unit][cell][20] with plain stores -- every (unit, tile) is
 // produced exactly once -- and k_pl_reduce_t adds the units up (f64 reductions into T cost 1.3 cycles per lane on the
 // LSU and were the bottleneck of the first version: 0.43 of 1.5 ms).
-template <int V>
-__global__ void __launch_bounds__(PtLayout<V>::WARPS * 32, 1)
+__global__ void __launch_bounds__(PT_WARPS * 32, 1)
 k_planes_t(PlDev pl, const PlUnitT *__restrict__ units, const PlItem *__restrict__ items, u32 n_items, u32 *__restrict__ counter,
            const signed char *__restrict__ Bd, const double *__restrict__ scale2_g, const double *__restrict__ lk, u32 wt,
-           double *__restrict__ part, u32 dbg) {
+           double *__restrict__ part) {
     extern __shared__ __align__(1024) unsigned char smem[];
     unsigned char *sB = smem;
     unsigned char *sA = sB + PT_B_BYTES;
     PtShared *sh = reinterpret_cast<PtShared *>(sA + PT_NSTAGES * PT_STAGE_BYTES);
-    using LY = PtLayout<V>;
-    constexpr u32 PT_WARPS = LY::WARPS, PT_THREADS = LY::WARPS * 32, EPI = LY::EPI;  // roles: [0, EPI) epilogue, EPI MMA, EPI + 1 .. producers, last (V0) / EPI + 1 (V1) item scheduler
-    constexpr u32 W_MMA = EPI, W_SCHED = V ? EPI + 1 : PT_WARPS - 1, W_PROD0 = V ? EPI + 2 : EPI + 1;
+    constexpr u32 EPI = PT_EPI_WARPS;  // roles: [0, EPI) epilogue, EPI MMA, EPI + 1 item scheduler, EPI + 2 .. producers
+    constexpr u32 W_MMA = EPI, W_SCHED = EPI + 1, W_PROD0 = EPI + 2;
     const u32 tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const u32 full0 = smem_u32(sh->full), empty0 = smem_u32(sh->empty), tfull0 = smem_u32(sh->tfull), tempty0 = smem_u32(sh->tempty);
     const u32 ifull0 = smem_u32(sh->item_full), iempty0 = smem_u32(sh->item_empty), bload0 = smem_u32(&sh->bload);
-    u32 breloads = 0;  // V1: bulk reloads of the B block so far (phase of `bload`)
+    u32 breloads = 0;  // bulk reloads of the B block so far (phase of `bload`)
 
     if (tid == 0) {
         for (u32 i = 0; i < PT_NSTG; i++) {
@@ -600,7 +570,6 @@ k_planes_t(PlDev pl, const PlUnitT *__restrict__ units, const PlItem *__restrict
     const u32 tmem = sh->tmem;
     const u32 sA_addr = smem_u32(sA), sB_addr = smem_u32(sB);
     const u32 idesc = instr_desc_i8(PL_TILE, PL_NCOL, false, false);
-    const uint64_t da_hi = smem_desc(0, PL_TILE * 16, 128), db_hi = smem_desc(0, PT_KCHUNK_BYTES, 128);
     const u64 n_pad = pl.ntiles * PL_TILE;
     const bool scheduler = warp == W_SCHED;
 
@@ -647,29 +616,21 @@ k_planes_t(PlDev pl, const PlUnitT *__restrict__ units, const PlItem *__restrict
             lev1 = nlev > 1 ? un.lev[1] : 0;
             lev2 = nlev > 2 ? un.lev[2] : 0;
             S = (nkb0 + nkb1 + nkb2) / PT_WORDS;  // sub-stages per tile, level-major: [level 0 | level 1 | level 2]
-            if (V == 1) {
-                // one thread starts nine 16 KB bulk copies (the TMA engine's 1-D form); everybody waits on their byte count
-                if (tid == 0) {
-                    mbar_expect_tx(bload0, PT_B_BYTES);
-                    const signed char *src = Bd + (size_t)(g0 / PT_RANGE) * PT_B_BYTES;
+            // one thread starts nine 16 KB bulk copies (the TMA engine's 1-D form); everybody waits on their byte count
+            if (tid == 0) {
+                mbar_expect_tx(bload0, PT_B_BYTES);
+                const signed char *src = Bd + (size_t)(g0 / PT_RANGE) * PT_B_BYTES;
 #pragma unroll 1
-                    for (u32 o = 0; o < PT_B_BYTES; o += 16384u) bulk_g2s(sB_addr + o, src + o, 16384u, bload0);
-                    mbar_arrive(bload0);
-                }
-                mbar_wait(bload0, breloads & 1u);
-                breloads++;
-            } else {
-                const uint4 *src = reinterpret_cast<const uint4 *>(Bd + (size_t)(g0 / PT_RANGE) * PT_B_BYTES);
-                uint4 *dst = reinterpret_cast<uint4 *>(sB);
-                for (u32 i = tid; i < PT_B_BYTES / 16; i += PT_THREADS) dst[i] = src[i];
-                fence_async_smem();
-                __syncthreads();
+                for (u32 o = 0; o < PT_B_BYTES; o += 16384u) bulk_g2s(sB_addr + o, src + o, 16384u, bload0);
+                mbar_arrive(bload0);
             }
+            mbar_wait(bload0, breloads & 1u);
+            breloads++;
         }
         const u64 t0 = item.t0, t1 = item.t1;
 
-        if (V == 1 && warp < EPI) {
-            // ===== epilogue, V1: warp w reads TMEM lanes 32 (w % 4) .. of columns [72 (w / 4), 72 (w / 4) + 72): ten columns of 32 cells
+        if (warp < EPI) {
+            // ===== epilogue: warp w reads TMEM lanes 32 (w % 4) .. of columns [72 (w / 4), 72 (w / 4) + 72): ten columns of 32 cells
             const u32 quarter = warp & 3u, half = warp >> 2;
             const u32 row = quarter * 32 + lane;
             double *pu = part + (size_t)item.unit * n_pad * PL_COLS + half * (PL_COLS / 2);
@@ -689,48 +650,15 @@ k_planes_t(PlDev pl, const PlUnitT *__restrict__ units, const PlItem *__restrict
                     const u32 slot = job % 3u;
                     mbar_wait(tfull0 + 8 * slot, (job / 3u) & 1u);
                     fence_after_sync();
-                    if (!(dbg & 2u)) read_acc_fma_half(tmem + ((quarter * 32u) << 16) + slot * PL_NCOL + half * 72u, a == 0 ? L0 : (a == 1 ? L1 : L2), res);
+                    read_acc_fma_half(tmem + ((quarter * 32u) << 16) + slot * PL_NCOL + half * 72u, a == 0 ? L0 : (a == 1 ? L1 : L2), res);
                     fence_before_sync();
                     __syncwarp();
                     if (lane == 0) mbar_arrive(tempty0 + 8 * slot);
                 }
-                if (!(dbg & 1u)) {
-                    double2 *o = reinterpret_cast<double2 *>(pu + cell * PL_COLS);
+                double2 *o = reinterpret_cast<double2 *>(pu + cell * PL_COLS);
 #pragma unroll
-                    for (u32 j = 0; j < PL_COLS / 2; j += 2)
-                        o[j >> 1] = make_double2(res[j] * sh->scale2[half * (PL_COLS / 2) + j], res[j + 1] * sh->scale2[half * (PL_COLS / 2) + j + 1]);
-                }
-            }
-        } else if (warp < EPI) {
-            // ===== epilogue: TMEM -> registers -> f64 -> partial output (one thread per cell row)
-            const u32 row = warp * 32 + lane;
-            double *pu = part + (size_t)item.unit * n_pad * PL_COLS;
-            for (u64 tile = t0; tile < t1; tile++) {
-                const u64 cell = tile * PL_TILE + row;
-                double res[PL_COLS];
-#pragma unroll
-                for (u32 j = 0; j < PL_COLS; j++) res[j] = 0.0;
-                double L0 = 0.0, L1 = 0.0, L2 = 0.0;
-                if (cell < pl.n) {  // L_c(level) from the per-cell table written by sb_normalize
-                    const double *lc = lk + cell * PL_MAX_LEVELS;
-                    L0 = lc[lev0];
-                    if (nlev > 1) L1 = lc[lev1];
-                    if (nlev > 2) L2 = lc[lev2];
-                }
-                for (u32 a = 0; a < nlev; a++, job++) {
-                    const u32 slot = job % 3u;
-                    mbar_wait(tfull0 + 8 * slot, (job / 3u) & 1u);
-                    fence_after_sync();
-                    if (!(dbg & 2u)) read_acc_fma(tmem + ((warp * 32u) << 16) + slot * PL_NCOL, a == 0 ? L0 : (a == 1 ? L1 : L2), res);
-                    fence_before_sync();
-                    __syncwarp();
-                    if (lane == 0) mbar_arrive(tempty0 + 8 * slot);  // this warp's quarter of the accumulator is free
-                }
-                if (!(dbg & 1u)) {  // rows of a tile are adjacent: a warp writes 32 x 160 contiguous bytes
-                    double2 *o = reinterpret_cast<double2 *>(pu + cell * PL_COLS);
-#pragma unroll
-                    for (u32 j = 0; j < PL_COLS; j += 2) o[j >> 1] = make_double2(res[j] * sh->scale2[j], res[j + 1] * sh->scale2[j + 1]);
-                }
+                for (u32 j = 0; j < PL_COLS / 2; j += 2)
+                    o[j >> 1] = make_double2(res[j] * sh->scale2[half * (PL_COLS / 2) + j], res[j + 1] * sh->scale2[half * (PL_COLS / 2) + j + 1]);
             }
         } else if (warp == W_MMA) {
             // ===== MMA issue.  The warp runs the loops converged, every value warp-uniform, and only the tensor-core instructions
@@ -739,8 +667,8 @@ k_planes_t(PlDev pl, const PlUnitT *__restrict__ units, const PlItem *__restrict
             // 5 x R2UR.BROADCAST / branch loop -- ~90 instructions per 4-MMA stage, more than the 288 cycles the MMAs take.
             {
                 const u32 a16 = sA_addr >> 4, b16 = sB_addr >> 4;
-                // V = 1: the low descriptor words carry the leading-byte-offset field (bits 16-29; the 14-bit address field below
-                // it never carries into it), so a descriptor is one add away from the previous one and the high word is an immediate
+                // the low descriptor words carry the leading-byte-offset field (bits 16-29; the 14-bit address field below it never
+                // carries into it), so a descriptor is one add away from the previous one and the high word is an immediate
                 const u32 a16x = a16 + ((PL_TILE * 16u >> 4) << 16), b16x = b16 + ((PT_KCHUNK_BYTES >> 4) << 16);
                 auto level = [&](u32 nkb) {
                     const u32 slot = job % 3u;
@@ -749,32 +677,15 @@ k_planes_t(PlDev pl, const PlUnitT *__restrict__ units, const PlItem *__restrict
                         fence_after_sync();
                     }
                     const u32 acc = tmem + slot * PL_NCOL;
-                    u32 kb = 0;
-                    if (V == 1) {
-                        for (; kb < nkb; kb += PT_SUB * PT_WORDS) {
-                            const u32 sg = q / PT_SUB, ss = sg & (PT_NSTG - 1);
-                            mbar_spin(full0 + 8 * ss, (sg / PT_NSTG) & 1u);
-                            fence_after_sync();
-                            const u32 alo = a16x + ss * (PT_SUB * PT_STAGE_BYTES >> 4), blo = b16x + kb * (2 * PT_KCHUNK_BYTES >> 4);
-                            if (elect_one()) {
-#pragma unroll
-                                for (u32 t = 0; t < PT_SUB * PT_WORDS; t++)
-                                    mma_i8_lo<0x4008u, 0x4008u>(acc, alo + t * (PL_TILE * 32 >> 4), blo + t * (2 * PT_KCHUNK_BYTES >> 4), idesc, kb | t);
-                                commit(empty0 + 8 * ss);
-                            }
-                            __syncwarp();
-                            q += PT_SUB;
-                        }
-                    }
-                    for (; kb < nkb; kb += PT_SUB * PT_WORDS) {  // kb counts 32-gene blocks (one MMA each)
+                    for (u32 kb = 0; kb < nkb; kb += PT_SUB * PT_WORDS) {  // kb counts 32-gene blocks (one MMA each)
                         const u32 sg = q / PT_SUB, ss = sg & (PT_NSTG - 1);
                         mbar_spin(full0 + 8 * ss, (sg / PT_NSTG) & 1u);
                         fence_after_sync();
-                        const u32 alo = a16 + ss * (PT_SUB * PT_STAGE_BYTES >> 4), blo = b16 + kb * (2 * PT_KCHUNK_BYTES >> 4);
+                        const u32 alo = a16x + ss * (PT_SUB * PT_STAGE_BYTES >> 4), blo = b16x + kb * (2 * PT_KCHUNK_BYTES >> 4);
                         if (elect_one()) {
 #pragma unroll
                             for (u32 t = 0; t < PT_SUB * PT_WORDS; t++)  // K = 32 per MMA = two 16-gene core-matrix columns (4 KB of A)
-                                mma_i8(acc, da_hi | (alo + t * (PL_TILE * 32 >> 4)), db_hi | (blo + t * (2 * PT_KCHUNK_BYTES >> 4)), idesc, kb | t);
+                                mma_i8_lo<0x4008u, 0x4008u>(acc, alo + t * (PL_TILE * 32 >> 4), blo + t * (2 * PT_KCHUNK_BYTES >> 4), idesc, kb | t);
                             commit(empty0 + 8 * ss);  // the stage is reusable once these MMAs have read it
                         }
                         __syncwarp();
@@ -844,45 +755,29 @@ k_planes_t(PlDev pl, const PlUnitT *__restrict__ units, const PlItem *__restrict
                 const bool more = ntile < t1;
                 if (more) load_words(ntile, ni, nxt);
                 if (ntile != tile) prefetch_tile(ntile + 2);
-                if (V == 1) {
-                    // the refill of a freed slot is on the critical path of the ring (microbenchmarks: 190 cycles from the last MMA to
-                    // the `empty` phase, 125-215 per barrier hop, against 1,152 cycles of MMAs in the whole ring): the expansion
-                    // arithmetic happens BEFORE the wait, into registers, and only the sixteen stores follow it
-                    // (the first 32-gene word group only: all sixteen vectors would need 64 registers and spill under the 96 this CTA
-                    // size allows; the second group is expanded after the wait, while the first group's stores drain)
-                    uint4 ex[8];
+                // the refill of a freed slot is on the critical path of the ring (microbenchmarks: 190 cycles from the last MMA to the
+                // `empty` phase, 125-215 per barrier hop, against 1,152 cycles of MMAs in the whole ring): the expansion arithmetic
+                // happens BEFORE the wait, into registers, and only the sixteen stores follow it (the first 32-gene word group only:
+                // all sixteen vectors would need 64 registers and spill under the 96 this CTA size allows; the second group is
+                // expanded after the wait, while the first group's stores drain)
+                uint4 ex[8];
 #pragma unroll
-                    for (u32 c4 = 0; c4 < 4; c4++) expand_bits32(cur[c4], ex[2 * c4], ex[2 * c4 + 1]);
-                    if (fills > 0) mbar_wait(empty0 + 8 * (p / PT_SUB), (fills - 1) & 1u);
-                    if (!(dbg & 4u)) {
-#pragma unroll
-                        for (u32 c4 = 0; c4 < 4; c4++) {
-                            st_shared_v4(st + c4 * 512, ex[2 * c4]);
-                            st_shared_v4(st + (PL_TILE * 16) + c4 * 512, ex[2 * c4 + 1]);
-                        }
-#pragma unroll
-                        for (u32 j = 1; j < PT_WORDS; j++)
-#pragma unroll
-                            for (u32 c4 = 0; c4 < 4; c4++) {
-                                uint4 lo, hi;
-                                expand_bits32(cur[j * 4 + c4], lo, hi);
-                                st_shared_v4(st + (2 * j) * (PL_TILE * 16) + c4 * 512, lo);
-                                st_shared_v4(st + (2 * j + 1) * (PL_TILE * 16) + c4 * 512, hi);
-                            }
-                    }
-                } else {
+                for (u32 c4 = 0; c4 < 4; c4++) expand_bits32(cur[c4], ex[2 * c4], ex[2 * c4 + 1]);
                 if (fills > 0) mbar_wait(empty0 + 8 * (p / PT_SUB), (fills - 1) & 1u);
-                if (!(dbg & 4u))
 #pragma unroll
-                    for (u32 j = 0; j < PT_WORDS; j++)
-#pragma unroll
-                        for (u32 c4 = 0; c4 < 4; c4++) {
-                            uint4 lo, hi;
-                            expand_bits32(cur[j * 4 + c4], lo, hi);
-                            st_shared_v4(st + (2 * j) * (PL_TILE * 16) + c4 * 512, lo);
-                            st_shared_v4(st + (2 * j + 1) * (PL_TILE * 16) + c4 * 512, hi);
-                        }
+                for (u32 c4 = 0; c4 < 4; c4++) {
+                    st_shared_v4(st + c4 * 512, ex[2 * c4]);
+                    st_shared_v4(st + (PL_TILE * 16) + c4 * 512, ex[2 * c4 + 1]);
                 }
+#pragma unroll
+                for (u32 j = 1; j < PT_WORDS; j++)
+#pragma unroll
+                    for (u32 c4 = 0; c4 < 4; c4++) {
+                        uint4 lo, hi;
+                        expand_bits32(cur[j * 4 + c4], lo, hi);
+                        st_shared_v4(st + (2 * j) * (PL_TILE * 16) + c4 * 512, lo);
+                        st_shared_v4(st + (2 * j + 1) * (PL_TILE * 16) + c4 * 512, hi);
+                    }
                 fence_async_smem();
                 __syncwarp();
                 if (lane == 0) mbar_arrive(full0 + 8 * (p / PT_SUB));
@@ -999,11 +894,11 @@ struct PnShared {
 // out[gene * row_stride + (col0 + j) * col_stride] += value
 // Persistent CTAs pull work items {group of 384 ranks, range of cell tiles} from a global queue (about equal cost each); an item
 // ends with its epilogue (the accumulators are reused by the next item), so the CTA-wide barrier between items costs nothing extra.
-// V = 1: twelve producer warps (ncu: the N side waits on its producers -- 114 polls of the `full` barrier per stage by the MMA
-// warp, producers busy 80 % of the time) and the digit rows of a sub-stage (4,608 contiguous bytes) arrive by one bulk
-// asynchronous copy (cp.async.bulk, completion counted on the stage's `full` barrier) instead of 9 LDG.128 + 9 STS.128 per lane.
-template <int V>
-__global__ void __launch_bounds__((PL_EPI_WARPS + 1 + (V ? 12 : 8)) * 32, 1)
+// Second generation (DESIGN.md 3): twelve producer warps instead of eight (ncu: the first generation waited on its producers -- 114
+// polls of the `full` barrier per stage by the MMA warp, producers busy 80 % of the time), and the digit rows of a sub-stage (4,608
+// contiguous bytes) arrive by one bulk asynchronous copy (cp.async.bulk, completion counted on the stage's `full` barrier) instead
+// of 9 LDG.128 + 9 STS.128 per lane.
+__global__ void __launch_bounds__(PN_THREADS, 1)
 k_planes_n(PlDev pl, const PlUnitN *__restrict__ units, const PlItem *__restrict__ items, u32 n_items, u32 *__restrict__ counter,
            const signed char *__restrict__ Bn, u64 n_pad, const double *__restrict__ scale2_g, const u32 *__restrict__ hot_idx, u32 col0, u32 wt,
            double *__restrict__ out, u64 row_stride, u64 col_stride) {
@@ -1012,7 +907,7 @@ k_planes_n(PlDev pl, const PlUnitN *__restrict__ units, const PlItem *__restrict
     PnShared *sh = reinterpret_cast<PnShared *>(sS + PN_NSTAGES * PN_STAGE_BYTES);
     const u32 tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const u32 full0 = smem_u32(sh->full), empty0 = smem_u32(sh->empty), tfull0 = smem_u32(&sh->tfull);
-    constexpr u32 PW = V ? 12u : 8u;  // producer warps
+    constexpr u32 PW = PN_PROD_WARPS;
     if (tid == 0) {
         for (u32 i = 0; i < PN_NSTG; i++) {
             mbar_init(full0 + 8 * i, PN_SUB);  // one arrival per producer warp of the stage
@@ -1030,8 +925,6 @@ k_planes_n(PlDev pl, const PlUnitN *__restrict__ units, const PlItem *__restrict
     const u32 tmem = sh->tmem;
     const u32 sS_addr = smem_u32(sS);
     const u32 idesc = instr_desc_i8(128, PL_NCOL, true, true);
-    const uint64_t da_hi = smem_desc(0, 128, 512);               // MN-major A: lbo = next 8 cells, sbo = next 16 genes
-    const uint64_t db_hi = smem_desc(0, PN_CELLGRP_BYTES, 128);  // MN-major B: lbo = next 8 cells, sbo = next 16 digit columns
 
     u32 sg = 0;  // stages issued (MMA) / sub-stages before this item (producers: Q0)
     u32 Q0 = 0;
@@ -1074,26 +967,16 @@ k_planes_n(PlDev pl, const PlUnitN *__restrict__ units, const PlItem *__restrict
                     mbar_spin(full0 + 8 * slot, (sg / PN_NSTG) & 1u);
                     fence_after_sync();
                     const u32 nmt = mtp & 15u;
-                    if (V == 1) {
-                        if (elect_one()) {
-#pragma unroll
-                            for (u32 ks = 0; ks < PN_SUB; ks++) {
-                                const u32 alo = s16 + (slot * PN_SUB + ks) * (PN_STAGE_BYTES >> 4) + ((128u >> 4) << 16);
-                                const u32 blo = s16 + (slot * PN_SUB + ks) * (PN_STAGE_BYTES >> 4) + (PN_A_BYTES >> 4) + ((PN_CELLGRP_BYTES >> 4) << 16);
-                                mma_i8_lo<0x4020u, 0x4008u>(tmem, alo, blo, idesc, (started & 1u) | ks);
-                                if (nmt > 1) mma_i8_lo<0x4020u, 0x4008u>(tmem + PL_NCOL, alo + 256, blo, idesc, ((started >> 1) & 1u) | ks);
-                                if (nmt > 2) mma_i8_lo<0x4020u, 0x4008u>(tmem + 2 * PL_NCOL, alo + 512, blo, idesc, ((started >> 2) & 1u) | ks);
-                            }
-                            commit(empty0 + 8 * slot);
-                        }
-                    } else if (elect_one()) {
+                    // MN-major descriptors: A lbo = next 8 cells (128 B), sbo = next 16 genes (512 B); B lbo = next 8 cells (1,152 B),
+                    // sbo = next 16 digit columns (128 B).  The low words carry address and lbo, the high words (sbo, version) are immediates.
+                    if (elect_one()) {
 #pragma unroll
                         for (u32 ks = 0; ks < PN_SUB; ks++) {
-                            const u32 alo = s16 + (slot * PN_SUB + ks) * (PN_STAGE_BYTES >> 4);
-                            const uint64_t db = db_hi | (alo + (PN_A_BYTES >> 4));
-                            mma_i8(tmem, da_hi | alo, db, idesc, (started & 1u) | ks);
-                            if (nmt > 1) mma_i8(tmem + PL_NCOL, da_hi | (alo + 256), db, idesc, ((started >> 1) & 1u) | ks);
-                            if (nmt > 2) mma_i8(tmem + 2 * PL_NCOL, da_hi | (alo + 512), db, idesc, ((started >> 2) & 1u) | ks);
+                            const u32 alo = s16 + (slot * PN_SUB + ks) * (PN_STAGE_BYTES >> 4) + ((128u >> 4) << 16);
+                            const u32 blo = s16 + (slot * PN_SUB + ks) * (PN_STAGE_BYTES >> 4) + (PN_A_BYTES >> 4) + ((PN_CELLGRP_BYTES >> 4) << 16);
+                            mma_i8_lo<0x4020u, 0x4008u>(tmem, alo, blo, idesc, (started & 1u) | ks);
+                            if (nmt > 1) mma_i8_lo<0x4020u, 0x4008u>(tmem + PL_NCOL, alo + 256, blo, idesc, ((started >> 1) & 1u) | ks);
+                            if (nmt > 2) mma_i8_lo<0x4020u, 0x4008u>(tmem + 2 * PL_NCOL, alo + 512, blo, idesc, ((started >> 2) & 1u) | ks);
                         }
                         commit(empty0 + 8 * slot);
                     }
@@ -1105,7 +988,7 @@ k_planes_n(PlDev pl, const PlUnitN *__restrict__ units, const PlItem *__restrict
             __syncwarp();
         } else {
             // ===== producers: sub-stage = (32-cell K step, level): A tiles [M tile][16-gene chunk (8)][cell / 8 (4)][cell % 8][16 B] + B
-            // digit rows.  Sub-stage Q of the CTA (tile-major, then level, then K step) goes to ring slot Q % 12, filled by warp Q % 8.
+            // digit rows.  Sub-stage Q of the CTA (tile-major, then level, then K step) goes to ring slot Q % 12, filled by warp Q % 12.
             const u32 p = warp - (PL_EPI_WARPS + 1);
             const u32 per_tile = PN_SUB * nlev;
             u32 cur[12], nxt[12];
@@ -1153,16 +1036,11 @@ k_planes_n(PlDev pl, const PlUnitN *__restrict__ units, const PlItem *__restrict
                 if (ntile != tile) prefetch_tile(ntile + 2);
                 // B rows of these 32 cells at level k (contiguous 4,608 bytes in Bn)
                 const uint4 *bsrc = reinterpret_cast<const uint4 *>(Bn + ((size_t)k * (n_pad / 8) + (tile * PL_TILE + ks * 32) / 8) * PN_CELLGRP_BYTES);
-                uint4 bv[V ? 1 : PN_B_BYTES / 16 / 32];
-                if (V == 0) {
-#pragma unroll
-                    for (u32 t = 0; t < PN_B_BYTES / 16 / 32; t++) bv[V ? 0 : t] = __ldg(bsrc + lane + 32 * t);
-                }
                 const u32 nw = ((mt_pack >> (4 * k)) & 15u) * 4;
                 const u32 sgq = Q / PN_SUB, slot = sgq % PN_NSTG, sub = Q % PN_NSTAGES;  // stage, its ring slot, my sub-slot (= slot * 4 + ks)
                 if (sgq >= PN_NSTG) mbar_wait(empty0 + 8 * slot, (sgq / PN_NSTG - 1) & 1u);
                 const u32 st = sS_addr + sub * PN_STAGE_BYTES;
-                if (V == 1 && lane == 0) {  // the slot is free: start the bulk copy of the digit rows, its bytes complete on the stage's barrier
+                if (lane == 0) {  // the slot is free: start the bulk copy of the digit rows, its bytes complete on the stage's barrier
                     mbar_expect_tx(full0 + 8 * slot, PN_B_BYTES);
                     bulk_g2s(st + PN_A_BYTES, bsrc, PN_B_BYTES, full0 + 8 * slot);
                 }
@@ -1175,10 +1053,6 @@ k_planes_n(PlDev pl, const PlUnitN *__restrict__ units, const PlItem *__restrict
                         st_shared_v4(a0, lo);
                         st_shared_v4(a0 + 512, hi);
                     }
-                }
-                if (V == 0) {
-#pragma unroll
-                    for (u32 t = 0; t < PN_B_BYTES / 16 / 32; t++) st_shared_v4(st + PN_A_BYTES + (lane + 32 * t) * 16, bv[V ? 0 : t]);
                 }
                 fence_async_smem();
                 __syncwarp();
@@ -1239,9 +1113,7 @@ int planes_t(sb_nmat *a, const double *Y, u32 ldy, u32 w, double *out, u32 ldo, 
     double *t1 = gl ? part.p + (size_t)pl.n_units_t * n_pad * PL_COLS : nullptr;
     const double *rs = a->has_row_scale ? a->row_scale.p : nullptr;
     const size_t smem = (size_t)PT_B_BYTES + PT_NSTAGES * PT_STAGE_BYTES + sizeof(PtShared);
-    const bool v1 = ctx->pl_variant & 1;
-    cudaError_t e = v1 ? cudaFuncSetAttribute(k_planes_t<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)
-                       : cudaFuncSetAttribute(k_planes_t<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    cudaError_t e = cudaFuncSetAttribute(k_planes_t, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return sb_fail(SB_ERR_CUDA, "planes_t: %zu B of shared memory: %s", smem, cudaGetErrorString(e));
     const u32 items = G1 * PL_COLS;
     const unsigned rblocks = (unsigned)std::max<u64>(1, std::min<u64>((mt->n * (PL_COLS / 2) + 255) / 256, (u64)ctx->sm_count * 16));
@@ -1251,20 +1123,14 @@ int planes_t(sb_nmat *a, const double *Y, u32 ldy, u32 w, double *out, u32 ldo, 
         if (col0 == 0) SB_CUDA(cudaMemsetAsync(Bd.p, 0, (size_t)nranges * PT_B_BYTES, ctx->stream));  // padding columns / ranks stay zero
         k_pl_colmax_t<<<cdiv(items, 256), 256, 0, ctx->stream>>>(Y, ldy, mt->hot_idx.p, rs, G1, col0, wt, colmax.p);
         SB_TRY(scales_from_colmax(ctx, colmax, scale2, ex));
-        k_pl_digits_t<<<cdiv(items, 256), 256, 0, ctx->stream>>>(Y, ldy, mt->hot_idx.p, rs, G1, col0, wt, ex.p, Bd.p, v1 ? 1u : 0u);
+        k_pl_digits_t<<<cdiv(items, 256), 256, 0, ctx->stream>>>(Y, ldy, mt->hot_idx.p, rs, G1, col0, wt, ex.p, Bd.p);
         SB_CUDA(cudaMemsetAsync(pl.counter.p, 0, sizeof(u32), ctx->stream));
         if (gl) {  // the sparse half of this column pass, in units of L_c(1)
             SB_CUDA(cudaMemsetAsync(t1, 0, (size_t)mt->n * PL_COLS * sizeof(double), ctx->stream));
             SB_TRY(gather_run_tile(ctx, *gl, 2, *mp, mt->n, Y, ldy, w, col0, t1 - col0, PL_COLS, col0 == 0 ? cycles : nullptr));
         }
-        if (v1)
-            k_planes_t<1><<<pl.t_grid, PtLayout<1>::WARPS * 32, smem, ctx->stream>>>(make_pldev(mt), (const PlUnitT *)pl.units_t.p,
-                                                                                     (const PlItem *)pl.items_t.p, pl.n_items_t, pl.counter.p, Bd.p, scale2.p,
-                                                                                     a->lk.p, wt, part.p, (u32)ctx->pl_debug);
-        else
-            k_planes_t<0><<<pl.t_grid, PtLayout<0>::WARPS * 32, smem, ctx->stream>>>(make_pldev(mt), (const PlUnitT *)pl.units_t.p,
-                                                                                     (const PlItem *)pl.items_t.p, pl.n_items_t, pl.counter.p, Bd.p, scale2.p,
-                                                                                     a->lk.p, wt, part.p, (u32)ctx->pl_debug);
+        k_planes_t<<<pl.t_grid, PT_WARPS * 32, smem, ctx->stream>>>(make_pldev(mt), (const PlUnitT *)pl.units_t.p, (const PlItem *)pl.items_t.p,
+                                                                    pl.n_items_t, pl.counter.p, Bd.p, scale2.p, a->lk.p, wt, part.p);
         k_pl_reduce_t<<<rblocks, 256, 0, ctx->stream>>>(part.p, pl.n_units_t, mt->n, n_pad, col0, wt, out, ldo, t1, gl ? a->l1c.p : nullptr);
         count_launch(ctx); count_launch(ctx); count_launch(ctx); count_launch(ctx);
     }
@@ -1285,9 +1151,7 @@ static int planes_n_impl(sb_nmat *a, const double *X, u32 ldx, u32 w, int mode, 
     SB_TRY(colmax.ensure(PL_COLS));
     SB_TRY(Bn.ensure((size_t)pl.L * (n_pad / 8) * PN_CELLGRP_BYTES));
     const size_t smem = (size_t)PN_NSTAGES * PN_STAGE_BYTES + sizeof(PnShared);
-    const bool v1 = ctx->pl_variant & 2;
-    cudaError_t e = v1 ? cudaFuncSetAttribute(k_planes_n<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)
-                       : cudaFuncSetAttribute(k_planes_n<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    cudaError_t e = cudaFuncSetAttribute(k_planes_n, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return sb_fail(SB_ERR_CUDA, "planes_n: %zu B of shared memory: %s", smem, cudaGetErrorString(e));
     const int cm_blocks = (int)std::max<u64>(1, std::min<u64>((mt->n + 255) / 256, (u64)ctx->sm_count * 4));
     for (u32 col0 = 0; col0 < w; col0 += PL_COLS) {
@@ -1297,14 +1161,9 @@ static int planes_n_impl(sb_nmat *a, const double *X, u32 ldx, u32 w, int mode, 
         SB_TRY(scales_from_colmax(ctx, colmax, scale2, ex));
         k_pl_digits_n<<<cdiv(n_pad * pl.L, 128), 128, 0, ctx->stream>>>(X, ldx, mt->n, n_pad, a->lk.p, pl.L, col0, wt, mode, ex.p, Bn.p);
         SB_CUDA(cudaMemsetAsync(pl.counter.p, 0, sizeof(u32), ctx->stream));
-        if (v1)
-            k_planes_n<1><<<pl.n_grid, (PL_EPI_WARPS + 1 + 12) * 32, smem, ctx->stream>>>(make_pldev(mt), (const PlUnitN *)pl.units_n.p,
-                                                                                          (const PlItem *)pl.items_n.p, pl.n_items_n, pl.counter.p, Bn.p, n_pad,
-                                                                                          scale2.p, mt->hot_idx.p, col0, wt, out, row_stride, col_stride);
-        else
-            k_planes_n<0><<<pl.n_grid, PL_THREADS, smem, ctx->stream>>>(make_pldev(mt), (const PlUnitN *)pl.units_n.p, (const PlItem *)pl.items_n.p,
-                                                                        pl.n_items_n, pl.counter.p, Bn.p, n_pad, scale2.p, mt->hot_idx.p, col0, wt, out,
-                                                                        row_stride, col_stride);
+        k_planes_n<<<pl.n_grid, PN_THREADS, smem, ctx->stream>>>(make_pldev(mt), (const PlUnitN *)pl.units_n.p, (const PlItem *)pl.items_n.p,
+                                                                 pl.n_items_n, pl.counter.p, Bn.p, n_pad, scale2.p, mt->hot_idx.p, col0, wt, out,
+                                                                 row_stride, col_stride);
         count_launch(ctx); count_launch(ctx); count_launch(ctx);
     }
     SB_CUDA(cudaGetLastError());

@@ -95,7 +95,7 @@ template <int LPR_T>
 __global__ void __launch_bounds__(256) k_spmm_t(const u64 *__restrict__ cm_ptr, const uint2 *__restrict__ cm, u64 n, MapDev mp,
                                                 const double *__restrict__ Y, u32 ldy, u32 col0, u32 wt, u32 w,
                                                 const double *__restrict__ uy, const double *__restrict__ v,
-                                                double *__restrict__ out, u32 ldo, int lpr_rt, int accumulate) {
+                                                double *__restrict__ out, u32 ldo, int lpr_rt) {
     __shared__ StageEnt stage_all[8][32];
     const int LPR = LPR_T > 0 ? LPR_T : lpr_rt;
     const int G = 32 / LPR;
@@ -178,10 +178,7 @@ __global__ void __launch_bounds__(256) k_spmm_t(const u64 *__restrict__ cm_ptr, 
             }
             double *dst = out + (size_t)c * ldo + c_lo;
             const bool two = c_lo + 1 < col0 + wt && c_lo + 1 < w;
-            if (accumulate) {  // the dense panel kernel adds into the same (zeroed) block concurrently
-                atomicAdd(dst, o0);
-                if (two) atomicAdd(dst + 1, o1);
-            } else if (two) {
+            if (two) {
                 *reinterpret_cast<double2 *>(dst) = make_double2(o0, o1);
             } else {
                 dst[0] = o0;
@@ -206,8 +203,8 @@ struct __align__(16) StageN {
     u32 gene;
 };
 
-template <int LPR_T, int THREADS>
-__global__ void __launch_bounds__(THREADS, 1024 / THREADS)  // <= 64 registers: two 512-thread CTAs' worth of room
+template <int LPR_T>
+__global__ void __launch_bounds__(1024, 1)  // <= 64 registers
 k_spmm_n(const uint2 *__restrict__ gm, const u64 *__restrict__ gm_base, u32 np, u32 ur, u32 pc, u64 n, MapDev mp,
          const double *__restrict__ X, u32 ldx, u32 col0, u32 wt, u32 w, double *__restrict__ P, u32 ldp, int lpr_rt) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -385,23 +382,22 @@ static void account(sb_ctx *ctx, const sb_mat *mt, u32 w, bool is_t) {
     }
 }
 
-// K7 driver: out[n x w] (ld ldo) = A^T . Y[m x w] (ld ldy) + v (u^T Y).  uy_scratch: device vector of >= w doubles.
-int dense_t(sb_nmat *a, const double *Y, u32 ldy, u32 w, double *out, u32 ldo, cudaStream_t stream, bool overlap);
-int dense_n(sb_nmat *a, const double *X, u32 ldx, u32 w, double *P, u32 ldp, cudaStream_t stream, bool overlap);
 int mat_ensure_full_gm(sb_mat *mt);
 // planes.cu
 int planes_t(sb_nmat *a, const double *Y, u32 ldy, u32 w, double *out, u32 ldo, const GatherLayout *gl, const MapDev *mp, long long *cycles);
+int planes_n(sb_nmat *a, const double *X, u32 ldx, u32 w, double *P, u32 ldp);
 // gather.cu
 int gather_run(sb_ctx *ctx, const GatherLayout &L, int mode, const MapDev &mp, u64 n_cells, const double *B, u32 ldb, u32 w, double *out, u32 ldo,
                long long *cycles = nullptr);
 int gather_recalibrate_t(sb_mat *mt, const long long *cycles_dev);
 int gather_t_init(sb_ctx *ctx, double *out, u64 n, u32 w, u32 ldo, const double *uy, const double *v);
-// the panelled gather layouts cover the cold entries of a hybrid matrix, or every entry of a matrix without a dense panel
+// the panelled gather layouts cover the cold entries of a hybrid matrix, or every entry of a matrix without planes
 static bool gather_usable(const sb_nmat *a, const GatherLayout &L) {
     const sb_mat *mt = a->mat;
     return mt->ctx->use_gather && L.ready && ((a->kind == 1 && mt->gd > 0) || mt->gd == 0);
 }
 
+// K7 driver: out[n x w] (ld ldo) = A^T . Y[m x w] (ld ldy) + v (u^T Y).  uy_scratch: device vector of >= w doubles.
 int spmm_t(sb_nmat *a, const double *Y, u32 ldy, u32 w, double *out, u32 ldo, double *uy_scratch) {
     sb_mat *mt = a->mat;
     sb_ctx *ctx = mt->ctx;
@@ -414,10 +410,10 @@ int spmm_t(sb_nmat *a, const double *Y, u32 ldy, u32 w, double *out, u32 ldo, do
     if (mt->n == 0 || w == 0) return SB_OK;
     MapDev mp = make_map(a);
     ProfScope ps(ctx, PH_SPMM_T);
-    // hybrid layout: the sparse kernel sees the cold entries only, the dense panel kernel adds the rest
+    // hybrid layout: the sparse kernel sees the cold entries only, the plane kernels add the rest
     const bool hybrid = a->kind == 1 && mt->gd > 0;
     if (gather_usable(a, mt->gt)) {
-        // T = v (u^T Y)  ->  += dense panel (DMMA)  ->  += panelled gather of the sparse set (f64 reductions)
+        // T = v (u^T Y)  ->  += planes (int8 tensor cores)  ->  += panelled gather of the sparse set (f64 reductions)
         SB_TRY(gather_t_init(ctx, out, mt->n, w, ldo, uy, a->v_ones ? nullptr : a->v.p));
         // first full-width product of this matrix: time every CTA of the gather, then re-cut its static shares (gather.cu)
         const bool calibrate = mt->t_calibrated < ctx->gather_calibrate && mt->gt.n_items == mt->gt.grid && w >= 8;
@@ -428,11 +424,11 @@ int spmm_t(sb_nmat *a, const double *Y, u32 ldy, u32 w, double *out, u32 ldo, do
         }
         // plane kernels + log chain: the gather runs inside planes_t, per column pass, with its run factor L_c(1) deferred to the
         // reduction of the per-unit partial rows (planes.cu)
-        const bool fused = hybrid && mt->pl.active && ctx->gather_defer && mp.kind == 1 && a->l1c.p;
+        const bool fused = hybrid && ctx->gather_defer && mp.kind == 1 && a->l1c.p;
         if (fused) {
             SB_TRY(planes_t(a, Y, ldy, w, out, ldo, &mt->gt, &mp, calibrate ? cyc.p : nullptr));
         } else {
-            if (hybrid) SB_TRY(dense_t(a, Y, ldy, w, out, ldo, ctx->stream, false));
+            if (hybrid) SB_TRY(planes_t(a, Y, ldy, w, out, ldo, nullptr, nullptr, nullptr));
             SB_TRY(gather_run(ctx, mt->gt, 1, mp, mt->n, Y, ldy, w, out, ldo, calibrate ? cyc.p : nullptr));
         }
         if (calibrate) SB_TRY(gather_recalibrate_t(mt, cyc.p));
@@ -448,30 +444,17 @@ int spmm_t(sb_nmat *a, const double *Y, u32 ldy, u32 w, double *out, u32 ldo, do
     int blocks = ctx->sm_count * 8;
     u64 need = (mt->n + 7) / 8;
     if ((u64)blocks > need) blocks = (int)need;
-    // Overlap: the sparse gather is bound by the L1 / shared-memory pipe, the panel kernel by the FP64 tensor pipe.
-    // Run them on two streams with CTAs of both resident on every SM; both add into the zeroed output block
-    // (0 + a + b is the same in either order, so the result stays deterministic).
-    const bool overlap = hybrid && !mt->pl.active && ctx->overlap_t && ctx->aux_stream != nullptr;
-    if (overlap) {
-        const u32 wpad = (w + 1) & ~1u;
-        SB_CUDA(cudaMemset2DAsync(out, (size_t)ldo * sizeof(double), 0, (size_t)wpad * sizeof(double), (size_t)mt->n, ctx->stream));
-        SB_CUDA(cudaEventRecord(ctx->ev_fork, ctx->stream));
-        SB_CUDA(cudaStreamWaitEvent(ctx->aux_stream, ctx->ev_fork, 0));
-        SB_TRY(dense_t(a, Y, ldy, w, out, ldo, ctx->aux_stream, true));
-        SB_CUDA(cudaEventRecord(ctx->ev_join, ctx->aux_stream));
-    }
     for (u32 col0 = 0; col0 < w; col0 += tw) {
         u32 wt = min(tw, w - col0);
         int lpr = (int)((wt + 1) / 2);
         dispatch_lpr(lpr, [&](auto tag) {
             constexpr int L = decltype(tag)::value;
             k_spmm_t<L><<<blocks, 256, 0, ctx->stream>>>(cm_ptr, cm, mt->n, mp, Y, ldy, col0, wt, w, uy,
-                                                         a->v_ones ? nullptr : a->v.p, out, ldo, lpr, overlap ? 1 : 0);
+                                                         a->v_ones ? nullptr : a->v.p, out, ldo, lpr);
         });
         count_launch(ctx);
     }
-    if (overlap) SB_CUDA(cudaStreamWaitEvent(ctx->stream, ctx->ev_join, 0));
-    else if (hybrid) SB_TRY(dense_t(a, Y, ldy, w, out, ldo, ctx->stream, false));
+    if (hybrid) SB_TRY(planes_t(a, Y, ldy, w, out, ldo, nullptr, nullptr, nullptr));
     account(ctx, mt, w, true);
     SB_CUDA(cudaGetLastError());
     return SB_OK;
@@ -497,62 +480,48 @@ int spmm_n(sb_nmat *a, const double *X, u32 ldx, u32 w, double *P, u32 ldp) {
     const u64 sparse_nnz = hybrid ? mt->cold_nnz : mt->nnz;
     if (mt->nnz && w) {
         ProfScope ps(ctx, PH_SPMM_N);
-        // tile width: the X panel (pc x wt doubles) must fit in shared memory next to the staging buffers
-        // Overlap: this kernel is bound by the shared-memory pipe, the panel kernel by the FP64 tensor pipe and it needs
-        // little shared memory; with 512-thread CTAs here and 256-thread CTAs there both are resident on every SM.
         if (gather_usable(a, mt->gn)) {
             SB_TRY(gather_run(ctx, mt->gn, 0, mp, mt->n, X, ldx, w, P, ldp));
-            if (hybrid) SB_TRY(dense_n(a, X, ldx, w, P, ldp, ctx->stream, false));
+            if (hybrid) SB_TRY(planes_n(a, X, ldx, w, P, ldp));
             account(ctx, mt, w, false);
             SB_CUDA(cudaGetLastError());
         } else {
-        const bool overlap = hybrid && !mt->pl.active && ctx->overlap && ctx->aux_stream != nullptr && sparse_nnz > 0;
-        if (overlap) {
-            SB_CUDA(cudaEventRecord(ctx->ev_fork, ctx->stream));
-            SB_CUDA(cudaStreamWaitEvent(ctx->aux_stream, ctx->ev_fork, 0));
-            SB_TRY(dense_n(a, X, ldx, w, P, ldp, ctx->aux_stream, true));
-            SB_CUDA(cudaEventRecord(ctx->ev_join, ctx->aux_stream));
-        }
-        const size_t smem_budget = 200 * 1024;
-        const int threads = overlap ? 512 : 1024;
-        size_t fixed = (size_t)mt->pc * 8 + 128 * sizeof(LogEnt) + (threads / 32) * 32 * sizeof(StageN);
-        u32 tile_max = (u32)((smem_budget - fixed) / ((size_t)mt->pc * 8));
-        tile_max &= ~1u;
-        if (tile_max > 64) tile_max = 64;
-        if (tile_max < 2) return sb_fail(SB_ERR_UNSUPPORTED, "spmm_n: panel does not fit in shared memory");
-        u32 ntiles = (w + tile_max - 1) / tile_max;
-        u32 tw = (w + ntiles - 1) / ntiles;
-        tw = (tw + 1) & ~1u;
-        u64 total_units = (u64)mt->np * mt->ur;
-        for (u32 col0 = 0; col0 < w && sparse_nnz; col0 += tw) {
-            u32 wt = min(tw, w - col0);
-            int lpr = (int)((wt + 1) / 2);
-            size_t smem = (size_t)mt->pc * (2 * lpr) * 8 + fixed;
-            int ctas_per_sm = (int)std::min<size_t>(2, (220 * 1024) / smem);
-            if (ctas_per_sm < 1) ctas_per_sm = 1;
-            int blocks = ctx->sm_count * ctas_per_sm;
-            if ((u64)blocks > total_units) blocks = (int)total_units;
-            int rc = SB_OK;
-            dispatch_lpr(lpr, [&](auto tag) {
-                constexpr int L = decltype(tag)::value;
-                cudaError_t e = overlap ? cudaFuncSetAttribute(k_spmm_n<L, 512>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)
-                                        : cudaFuncSetAttribute(k_spmm_n<L, 1024>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-                if (e != cudaSuccess) {
-                    rc = sb_fail(SB_ERR_CUDA, "cudaFuncSetAttribute(%zu B smem): %s", smem, cudaGetErrorString(e));
-                    return;
-                }
-                if (overlap)
-                    k_spmm_n<L, 512><<<blocks, 512, smem, ctx->stream>>>(gm, gm_base, mt->np, mt->ur, mt->pc, mt->n, mp, X, ldx, col0, wt, w, P, ldp, lpr);
-                else
-                    k_spmm_n<L, 1024><<<blocks, 1024, smem, ctx->stream>>>(gm, gm_base, mt->np, mt->ur, mt->pc, mt->n, mp, X, ldx, col0, wt, w, P, ldp, lpr);
-            });
-            SB_TRY(rc);
-            count_launch(ctx);
-        }
-        if (overlap) SB_CUDA(cudaStreamWaitEvent(ctx->stream, ctx->ev_join, 0));
-        else if (hybrid) SB_TRY(dense_n(a, X, ldx, w, P, ldp, ctx->stream, false));
-        account(ctx, mt, w, false);
-        SB_CUDA(cudaGetLastError());
+            // tile width: the X panel (pc x wt doubles) must fit in shared memory next to the staging buffers
+            const size_t smem_budget = 200 * 1024;
+            const int threads = 1024;
+            size_t fixed = (size_t)mt->pc * 8 + 128 * sizeof(LogEnt) + (threads / 32) * 32 * sizeof(StageN);
+            u32 tile_max = (u32)((smem_budget - fixed) / ((size_t)mt->pc * 8));
+            tile_max &= ~1u;
+            if (tile_max > 64) tile_max = 64;
+            if (tile_max < 2) return sb_fail(SB_ERR_UNSUPPORTED, "spmm_n: panel does not fit in shared memory");
+            u32 ntiles = (w + tile_max - 1) / tile_max;
+            u32 tw = (w + ntiles - 1) / ntiles;
+            tw = (tw + 1) & ~1u;
+            u64 total_units = (u64)mt->np * mt->ur;
+            for (u32 col0 = 0; col0 < w && sparse_nnz; col0 += tw) {
+                u32 wt = min(tw, w - col0);
+                int lpr = (int)((wt + 1) / 2);
+                size_t smem = (size_t)mt->pc * (2 * lpr) * 8 + fixed;
+                int ctas_per_sm = (int)std::min<size_t>(2, (220 * 1024) / smem);
+                if (ctas_per_sm < 1) ctas_per_sm = 1;
+                int blocks = ctx->sm_count * ctas_per_sm;
+                if ((u64)blocks > total_units) blocks = (int)total_units;
+                int rc = SB_OK;
+                dispatch_lpr(lpr, [&](auto tag) {
+                    constexpr int L = decltype(tag)::value;
+                    cudaError_t e = cudaFuncSetAttribute(k_spmm_n<L>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+                    if (e != cudaSuccess) {
+                        rc = sb_fail(SB_ERR_CUDA, "cudaFuncSetAttribute(%zu B smem): %s", smem, cudaGetErrorString(e));
+                        return;
+                    }
+                    k_spmm_n<L><<<blocks, threads, smem, ctx->stream>>>(gm, gm_base, mt->np, mt->ur, mt->pc, mt->n, mp, X, ldx, col0, wt, w, P, ldp, lpr);
+                });
+                SB_TRY(rc);
+                count_launch(ctx);
+            }
+            if (hybrid) SB_TRY(planes_n(a, X, ldx, w, P, ldp));
+            account(ctx, mt, w, false);
+            SB_CUDA(cudaGetLastError());
         }
     }
     SB_TRY(comm_allreduce_f64(ctx, P, ((size_t)mt->m + 1) * ldp));

@@ -1,6 +1,6 @@
 // tc05.cuh -- thin PTX wrappers for the sm_100a tensor-core path (tcgen05.mma kind::i8, TMEM, mbarriers) used by the
-// bit-plane panel kernels (planes.cu).  Encodings follow cute/arch/mma_sm100_desc.hpp (UMMA::SmemDescriptor,
-// UMMA::InstrDescriptor); the K-major / no-swizzle form was validated on hardware by panel_i8.cu in round 2.
+// bit-plane kernels (planes.cu) and the microbenchmarks under profiles/microbench.  Encodings follow
+// cute/arch/mma_sm100_desc.hpp (UMMA::SmemDescriptor, UMMA::InstrDescriptor).
 #pragma once
 #include <cstdint>
 
@@ -107,16 +107,6 @@ __device__ __forceinline__ void bulk_g2s(uint32_t dst_saddr, const void *src, ui
     asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst_saddr), "l"(src), "r"(bytes),
                  "r"(mbar)
                  : "memory");
-}
-
-// one non-blocking look at a barrier phase
-__device__ __forceinline__ bool mbar_test(uint32_t mbar, uint32_t parity) {
-    uint32_t done = 0;
-    asm volatile("{\n\t.reg .pred p;\n\tmbarrier.test_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}\n"
-                 : "=r"(done)
-                 : "r"(mbar), "r"(parity)
-                 : "memory");
-    return done != 0;
 }
 
 // long waits (an epilogue waiting for a whole CTA's worth of MMAs): back off so the spinning warps leave the issue slots alone

@@ -49,16 +49,3 @@ for g in (0, 1):
     sig[g] = s.copy()
     print(f"gather={g}: pca {ms:.1f} ms, spmm_t {p['spmm_t_ms']/p['spmm_t_launches']:.2f} ms/pass, spmm_n {p['spmm_n_ms']/p['spmm_n_launches']:.2f} ms/pass", flush=True)
 print("sigma rel diff", np.abs(sig[0] - sig[1]).max() / sig[0].max())
-# hot-panel size sweep with the panelled gather: (max genes in the dense panel, min density)
-del a, dm
-for cap, dens in ((2048, 0.12), (1536, 0.16), (1280, 0.20), (1024, 0.25)):
-    ctx.set_option("dense_genes", cap); ctx.set_option("dense_min_density", dens); ctx.set_option("gather", 1)
-    dm = generate_device(ctx, SynthConfig(n_cells=n, n_genes=33538, seed=3))
-    a = sb.normalize(dm, sb.Normalization.CellRanger)
-    a.dot(x); a.rdot(y)
-    ctx.profile_enable(True); ctx.profile_reset()
-    for _ in range(5):
-        a.dot(x); a.rdot(y)
-    p = ctx.profile(); ctx.profile_enable(False)
-    print(f"panel cap {cap} density>={dens}: spmm_t {p['spmm_t_ms']/p['spmm_t_launches']:.3f} ms/pass, spmm_n {p['spmm_n_ms']/p['spmm_n_launches']:.3f} ms/pass", flush=True)
-    del a, dm

@@ -1,4 +1,4 @@
-"""A few A.X / A^T.Y passes at n_cells for an ncu launch list.  usage: python scripts/prof_passes.py [n_cells] [panel_mode] [passes]"""
+"""A few A.X / A^T.Y passes at n_cells for an ncu launch list.  usage: python scripts/prof_passes.py [n_cells] [passes]"""
 import sys
 sys.path.insert(0, "/root/repo")
 import numpy as np
@@ -6,10 +6,8 @@ import scan_rs_b200 as sb
 from scan_rs_b200.synth import SynthConfig, generate_device
 
 n = int(sys.argv[1]) if len(sys.argv) > 1 else 400_000
-mode = int(sys.argv[2]) if len(sys.argv) > 2 else 2
-passes = int(sys.argv[3]) if len(sys.argv) > 3 else 2
+passes = int(sys.argv[2]) if len(sys.argv) > 2 else 2
 ctx = sb.Context(0)
-ctx.set_option("panel_mode", mode)
 dm = generate_device(ctx, SynthConfig(n_cells=n, n_genes=33538, seed=3))
 a = sb.normalize(dm, sb.Normalization.CellRanger)
 x = np.random.default_rng(0).standard_normal((n, 20))

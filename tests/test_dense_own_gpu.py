@@ -12,7 +12,6 @@ directly through tests/cuda/dense_harness.cu, linked against the library's objec
 - the PCA itself must take no fallback on well-conditioned inputs, and the two dense back ends must agree on sigma.
 """
 import ctypes as C
-import glob
 import os
 import shutil
 import subprocess
@@ -22,7 +21,7 @@ import pytest
 
 import scan_rs_b200 as sb
 from scan_rs_b200 import _lib as L
-from tests.util import synth_pair
+from tests.util import library_objects, synth_pair
 
 pytestmark = pytest.mark.gpu
 
@@ -111,8 +110,7 @@ def dh(tmp_path_factory):
     nvcc = _nvcc()
     cuda_lib = os.path.join(os.path.dirname(os.path.dirname(os.path.realpath(nvcc))), "lib64")
     out = str(tmp_path_factory.mktemp("dense_harness") / "libdense_harness.so")
-    objs = sorted(glob.glob(os.path.join(csrc, "_build", "*.o")))
-    assert objs, "no object files under scan_rs_b200/csrc/_build"
+    objs = library_objects(csrc)
     subprocess.check_call([nvcc, "-shared", "-O2", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a", "-Xcompiler", "-fPIC",
                            "-o", out, os.path.join(ROOT, "tests", "cuda", "dense_harness.cu"), *objs, "-L" + cuda_lib,
                            "-lcublas", "-lcusolver", "-ldl", "-Xlinker", "-Bsymbolic", "-Xlinker", "-rpath," + cuda_lib])

@@ -297,15 +297,15 @@ def test_projection_shortcut_and_direct_pass_agree(ctx, n_cells, n_genes):
     check_pca_parity(res_fast, res_direct)
 
 
-def test_hybrid_dense_panel_matches_pure_sparse(ctx):
-    """The dense hot-gene panel (csrc/dense_panel.cu) and the pure sparse layout give the same products and
-    moments to rounding, and both match the oracle; counts above 15 in hot genes stay on the sparse side."""
+def test_hybrid_planes_match_pure_sparse(ctx):
+    """The bit planes of the hot genes (csrc/planes.cu) and the pure sparse layout give the same products and
+    moments to rounding, and both match the oracle; counts above a gene's top plane level stay on the sparse side."""
     cfg, cm, dm_h, (ip, g, c) = synth_pair(ctx, 3000, 2500, seed=37, n_dense=40, dense_mean=40.0)
     try:
-        ctx.set_option("dense_genes", 0)
+        ctx.set_option("plane_cap", 0)
         dm_s = sb.AdaptiveMat.from_csc(ctx, 2500, 3000, ip, g, c)
     finally:
-        ctx.set_option("dense_genes", 2048)
+        ctx.set_option("plane_cap", 12288)
     a_o = orc.normalize(cm, orc.CELLRANGER)
     a_h, a_s = sb.normalize(dm_h, sb.Normalization.CellRanger), sb.normalize(dm_s, sb.Normalization.CellRanger)
     for p_h, p_s, p_o in zip(a_h.params(), a_s.params(), (a_o.mat.spec.col_scale, a_o.mat.spec.row_scale, a_o.u.ravel(), a_o.v.ravel())):
@@ -326,20 +326,23 @@ def test_hybrid_dense_panel_matches_pure_sparse(ctx):
     check_pca_parity(sb.BkSvd().run_pca(a_s, 10), res_o)
 
 
-@pytest.mark.parametrize("n_cells,n_genes,norm", [(3000, 2500, "log"), (40000, 1500, "log"), (2000, 1300, "deviance"), (600, 90, "log")])
-def test_panelled_gather_matches_first_generation_kernels(ctx, n_cells, n_genes, norm):
+# the binomial maps take the panelled gather only on a matrix without planes: their case is built with plane_cap 0
+@pytest.mark.parametrize("n_cells,n_genes,norm,plane_cap", [(3000, 2500, "log", 12288), (40000, 1500, "log", 12288), (2000, 1300, "deviance", 0),
+                                                            (600, 90, "log", 12288)])
+def test_panelled_gather_matches_first_generation_kernels(ctx, n_cells, n_genes, norm, plane_cap):
     """The panelled gather kernels (csrc/gather.cu; default) against the first-generation cell-major / gene-major
     kernels (csrc/spmm.cu; option gather=0) and the oracle, on both products: several cell blocks and gene panels,
     ragged panels, widths that need 1-3 column passes with and without the 4-column tail."""
     cfg, cm, dm, (ip, g, c) = synth_pair(ctx, n_cells, n_genes, seed=41, depth=600.0)
-    if norm == "log":
-        a_o, a_g = orc.normalize(cm, orc.CELLRANGER), sb.normalize(dm, sb.Normalization.CellRanger)
-    else:  # the binomial maps take the panelled gather only on a matrix without a dense panel
+    if plane_cap != 12288:
         try:
-            ctx.set_option("dense_genes", 0)
+            ctx.set_option("plane_cap", plane_cap)
             dm = sb.AdaptiveMat.from_csc(ctx, n_genes, n_cells, ip, g, c)
         finally:
-            ctx.set_option("dense_genes", 2048)
+            ctx.set_option("plane_cap", 12288)
+    if norm == "log":
+        a_o, a_g = orc.normalize(cm, orc.CELLRANGER), sb.normalize(dm, sb.Normalization.CellRanger)
+    else:
         a_o, a_g = orc.binom_deviance_resid(cm), sb.binom_deviance_resid(dm)
     rng = np.random.default_rng(6)
     for w in (20, 16, 9, 45):
@@ -359,42 +362,12 @@ def test_panelled_gather_matches_first_generation_kernels(ctx, n_cells, n_genes,
         assert np.abs(got[0][1] - got[1][1]).max() <= 1e-11 * np.abs(ref_t).max()
 
 
-def test_int8_draft_panel_matches_fp64_panel(ctx):
-    """Round 1's draft of the T-side panel on the integer tensor cores (csrc/panel_i8.cu, option panel_i8 over the u8 panel of
-    panel_mode 1 restricted to counts 1..3): first run on hardware in round 2, agrees with the FP64 mma.sync panel and the
-    oracle.  Superseded by the bit-plane kernels (csrc/planes.cu, panel_mode 2, the default); kept as the validated reference point."""
-    n_cells, n_genes = 6000, 33538
-    try:
-        ctx.set_option("panel_mode", 1)
-        ctx.set_option("dense_max_count", 3)
-        cfg, cm, _, (ip, g, c) = synth_pair(ctx, n_cells, n_genes, seed=44)
-        dm = sb.AdaptiveMat.from_csc(ctx, n_genes, n_cells, ip, g, c)
-    finally:
-        ctx.set_option("dense_max_count", 15)
-        ctx.set_option("panel_mode", 2)
-    a_o, a_g = orc.normalize(cm, orc.CELLRANGER), sb.normalize(dm, sb.Normalization.CellRanger)
-    rng = np.random.default_rng(8)
-    for w in (20, 7):
-        y = rng.standard_normal((w, n_genes))
-        ref = a_o.rdot(y)
-        got = {}
-        for on in (0, 1):
-            try:
-                ctx.set_option("panel_i8", on)
-                got[on] = a_g.rdot(y)
-            finally:
-                ctx.set_option("panel_i8", 0)
-            assert np.abs(got[on] - ref).max() <= 1e-10 * np.abs(ref).max(), (on, w)
-        assert np.abs(got[0] - got[1]).max() <= 1e-11 * np.abs(ref).max()
-        assert np.abs(got[0] - got[1]).max() > 0.0  # the two paths really are different kernels
-
-
 @pytest.mark.parametrize("n_cells,n_genes,kw", [(3000, 2500, dict(n_dense=40, dense_mean=40.0)), (6000, 33538, {}), (1000, 200, {}),
                                                  (130, 400, {}), (20000, 9000, dict(depth=6000.0))])
-def test_plane_kernels_match_oracle_and_other_layouts(ctx, n_cells, n_genes, kw):
-    """The three layouts of the dense half -- none (pure sparse gather), u8 panel on the FP64 mma.sync path, bit planes on the
-    tcgen05 int8 path (default) -- give the same normalization parameters and products, and all match the oracle: widths with
-    one, partial and several column passes; a ragged last cell tile; matrices with one to six count levels."""
+def test_plane_kernels_match_oracle_and_pure_sparse(ctx, n_cells, n_genes, kw):
+    """Both layouts of the dense half -- none (pure sparse gather, plane_cap 0) and bit planes on the tcgen05 int8 path
+    (default) -- give the same normalization parameters and products, and both match the oracle: widths with one, partial and
+    several column passes; a ragged last cell tile; matrices with one to six count levels."""
     cfg, cm, _, (ip, g, c) = synth_pair(ctx, n_cells, n_genes, seed=37, **kw)
     a_o = orc.normalize(cm, orc.CELLRANGER)
     ref_p = (a_o.mat.spec.col_scale, a_o.mat.spec.row_scale, a_o.u.ravel(), a_o.v.ravel())
@@ -404,22 +377,22 @@ def test_plane_kernels_match_oracle_and_other_layouts(ctx, n_cells, n_genes, kw)
     ref_n = {w: a_o.dot(xs[w]) for w in xs}
     ref_t = {w: a_o.rdot(ys[w]) for w in ys}
     got = {}
-    for mode in (0, 1, 2):
+    for cap in (0, 12288):
         try:
-            ctx.set_option("panel_mode", mode)
+            ctx.set_option("plane_cap", cap)
             dm = sb.AdaptiveMat.from_csc(ctx, n_genes, n_cells, ip, g, c)
         finally:
-            ctx.set_option("panel_mode", 2)
+            ctx.set_option("plane_cap", 12288)
         a = sb.normalize(dm, sb.Normalization.CellRanger)
         for p_g, p_o in zip(a.params(), ref_p):
             np.testing.assert_allclose(p_g, p_o, rtol=1e-9, atol=1e-12)
-        got[mode] = a.params()
+        got[cap] = a.params()
         for w in xs:
-            assert np.abs(a.dot(xs[w]) - ref_n[w]).max() <= 1e-10 * np.abs(ref_n[w]).max(), (mode, w)
-            assert np.abs(a.rdot(ys[w]) - ref_t[w]).max() <= 1e-10 * np.abs(ref_t[w]).max(), (mode, w)
+            assert np.abs(a.dot(xs[w]) - ref_n[w]).max() <= 1e-10 * np.abs(ref_n[w]).max(), (cap, w)
+            assert np.abs(a.rdot(ys[w]) - ref_t[w]).max() <= 1e-10 * np.abs(ref_t[w]).max(), (cap, w)
         a.free()
         dm.free()
-    for p2, p0 in zip(got[2], got[0]):
+    for p2, p0 in zip(got[12288], got[0]):
         np.testing.assert_allclose(p2, p0, rtol=1e-11, atol=1e-13)
 
 

@@ -32,7 +32,6 @@ Non-finite operands: where the reference is NaN or +-inf the device must not be 
 operand column j makes the whole of output column j NaN (include/scanb200.h, sb_nmat_dot).
 """
 import ctypes as C
-import glob
 import os
 import shutil
 import subprocess
@@ -44,6 +43,7 @@ import scipy.sparse as sp
 from oracle import oracle as orc
 from scan_rs_b200 import _lib as L
 from scan_rs_b200.synth import SynthConfig, generate_host
+from tests.util import library_objects
 
 pytestmark = pytest.mark.gpu
 
@@ -54,8 +54,8 @@ C_PL = 1.0
 NAN = float("nan")
 LD = np.longdouble
 # library defaults of the options the tests change (csrc/common.cuh)
-DEFAULTS = {"plane_levels": 6, "plane_cap": 12288, "plane_min_density": 0.01, "plane_items_per_cta": 48, "pl_variant": 3,
-            "gather_defer": 1, "gather_calibrate": 1, "gather": 1}
+DEFAULTS = {"plane_levels": 6, "plane_cap": 12288, "plane_min_density": 0.01, "plane_items_per_cta": 48, "gather_defer": 1,
+            "gather_calibrate": 1, "gather": 1}
 
 
 def even_up(w):
@@ -115,8 +115,7 @@ def sh(tmp_path_factory):
     nvcc = _nvcc()
     cuda_lib = os.path.join(os.path.dirname(os.path.dirname(os.path.realpath(nvcc))), "lib64")
     out = str(tmp_path_factory.mktemp("spmm_harness") / "libspmm_harness.so")
-    objs = sorted(glob.glob(os.path.join(csrc, "_build", "*.o")))
-    assert objs, "no object files under scan_rs_b200/csrc/_build"
+    objs = library_objects(csrc)
     subprocess.check_call([nvcc, "-shared", "-O2", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a", "-Xcompiler", "-fPIC",
                            "-o", out, os.path.join(ROOT, "tests", "cuda", "spmm_harness.cu"), *objs, "-L" + cuda_lib,
                            "-lcublas", "-lcusolver", "-ldl", "-Xlinker", "-Bsymbolic", "-Xlinker", "-rpath," + cuda_lib])
@@ -428,21 +427,18 @@ def test_plane_items_per_cta(sh, per_cta):
     check_dot(M, rng.standard_normal((M.n, 41)), f"items={per_cta}")
 
 
-@pytest.mark.parametrize("variant", [0, 1, 2, 3])
-def test_plane_kernel_variants(sh, variant):
-    """Both generations of each plane kernel (pl_variant bit 0: T side, bit 1: N side), on one layout with two T ranges."""
-    M = mat(sh, "variants", plane_min_density=0.0, plane_cap=1152, plane_levels=4)
+def test_plane_kernels_two_t_ranges(sh):
+    """Both plane kernels on a layout with two T ranges (1,152 ranks) and four full levels, at the default items per CTA."""
+    M = mat(sh, "two_ranges", plane_min_density=0.0, plane_cap=1152, plane_levels=4)
     assert_planes(M, L=4, G=[1152] * 4)
-    rng = np.random.default_rng(variant)
-    X, Y = rng.standard_normal((M.n, 41)), rng.standard_normal((M.m, 41))
-    with Options(sh, pl_variant=variant):
-        check_dot(M, X, f"variant={variant}")
-        check_rdot(M, Y, f"variant={variant}")
+    rng = np.random.default_rng(3)
+    check_dot(M, rng.standard_normal((M.n, 41)), "two T ranges")
+    check_rdot(M, rng.standard_normal((M.m, 41)), "two T ranges")
 
 
 @pytest.mark.parametrize("defer", [0, 1])
 def test_gather_defer(sh, defer):
-    """gather_defer 0: the T side runs dense_t -> planes_t without the fused gather, then the gather applies L_c(1) itself."""
+    """gather_defer 0: the T side runs planes_t without the fused gather, then the gather applies L_c(1) itself."""
     M = mat(sh, "base")
     assert_planes(M)
     rng = np.random.default_rng(defer)

@@ -1,4 +1,7 @@
 """Shared helpers of the parity tests."""
+import glob
+import os
+
 import numpy as np
 
 from oracle import oracle as orc
@@ -29,3 +32,14 @@ def check_pca_parity(res_gpu, res_orc, sigma_tol=1e-6, angle_tol=1e-5):
     au, av = sin_theta(uo, ug), sin_theta(vo, vg)
     assert au < angle_tol and av < angle_tol, (au, av)
     return rel.max(), au, av
+
+
+def library_objects(csrc):
+    """The library's object files for linking a test harness: _build/<stem>.o for every csrc/*.cu, as the Makefile builds them.
+    An object whose source is gone (left in _build by an earlier tree) is not linked; a missing object is an error."""
+    srcs = sorted(glob.glob(os.path.join(csrc, "*.cu")))
+    assert srcs, f"no CUDA sources under {csrc}"
+    objs = [os.path.join(csrc, "_build", os.path.splitext(os.path.basename(s))[0] + ".o") for s in srcs]
+    missing = [o for o in objs if not os.path.isfile(o)]
+    assert not missing, f"object files missing (build the library first): {missing}"
+    return objs
